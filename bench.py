@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the L-TAE + TemporalAggregator hot path (BASELINE.json metric: patches/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the U-TAE temporal bottleneck over a batch of B synthetic patches
 (BASELINE.json configs[1]: bf16, B=64, T=61 with irregular lengths 27..61 and pad masks):
@@ -34,6 +34,7 @@ T_FRAMES = 61
 LEVELS = ((64, 32), (64, 64), (64, 128))  # (channels, resolution) of the three skip feature maps
 LTAE_C, LTAE_RES = 128, 16
 N_HEAD = 16
+DUMP_PATCHES = 8  # 6.6 MB of float32 outputs per patch: 8 patches keep a dump under 64 MB at any batch size
 FALLBACK_HBM_GBS = 6650.0  # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
 
 
@@ -51,7 +52,14 @@ def parse_args():
     ap.add_argument("--cpu-patches", type=int, default=2, help="patches in the CPU-baseline sample")
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-records (placements, training, tile, sustained)")
     ap.add_argument("--sub-seconds", type=float, default=1.0, help="minimum timed seconds of every sub-record")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the last timed step's outputs to DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path; it does not apply to --impl reference")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -94,6 +102,24 @@ def agg128_bytes(lengths, elem):
     n_valid = int(sum(lengths))
     b = len(lengths)
     return elem * n_valid * c * r * r + elem * b * c * r * r + 4 * N_HEAD * n_valid * LTAE_RES ** 2
+
+
+def dump_outputs(dump_dir, out, att, skips):
+    """Write what one step returned -- the encoder's output and attention and the three aggregations -- for a fixed,
+    seeded sample of the batch's patches as float32 ``dump_dir/<name>.npy``, so that two builds of the project can be
+    compared output for output.  Returns a description of the files for the result line."""
+    import numpy as np
+    import torch
+    batch = out.shape[0]
+    patches = np.sort(np.random.RandomState(0).choice(batch, min(batch, DUMP_PATCHES), replace=False))
+    idx = torch.from_numpy(patches).to(out.device)
+    arrays = {"ltae_out": out.index_select(0, idx), "ltae_attn": att.index_select(1, idx)}
+    for (_, r), s in zip(LEVELS, skips):
+        arrays[f"agg_{r}"] = s.index_select(0, idx)
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dump_dir, name + ".npy"), t.float().cpu().numpy())
+    return {"dir": dump_dir, "patches": patches.tolist(), "arrays": {n: list(t.shape) for n, t in arrays.items()}}
 
 
 class ClockSampler:
@@ -306,7 +332,7 @@ def run_b200(args):
             for x in xs_:
                 skips.append(agg(x, pad_mask=pad, attn_mask=att))
                 mark()
-        return out, skips
+        return out, att, skips
 
     def barrier():
         if world > 1:
@@ -322,11 +348,14 @@ def run_b200(args):
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local_rank) as clocks:
         start.record()
-        for _ in range(args.steps):
+        for _ in range(args.steps - 1):
             step(x4, xs, timers)
+        last = step(x4, xs, timers)  # kept for --dump-outputs; no step runs while it is held
         stop.record()
         barrier()
     launches = _lib.launch_count()
+    dumped = dump_outputs(args.dump_outputs, *last) if args.dump_outputs and rank == 0 else None
+    del last
     elapsed_ms = start.elapsed_time(stop)
     t = torch.tensor([elapsed_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -488,6 +517,8 @@ def run_b200(args):
             "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "parity": parity, "gpu_launches": int(launches),
             "clocks": clocks.summary(),
         }
+        if dumped is not None:
+            line["dump"] = dumped
         line.update(sub)
         print(json.dumps(line), flush=True)
     if world > 1:

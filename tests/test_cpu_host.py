@@ -158,13 +158,33 @@ def test_install_swaps_reference_bindings():
                 sys.modules[n] = m
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/backbones"), reason="needs the reference checkout")
-def test_install_imports_then_uninstall_restores_the_reference_classes():
+# A stand-in for the reference's src/backbones with the same import-time bindings: the model files take the hot-path
+# classes by name from tae.py / temporal_aggregator.py (utae.py:8-9, wtae.py:9-10, timeunet.py:4-5).
+STAND_IN_REFERENCE = {
+    "src/__init__.py": "",
+    "src/backbones/__init__.py": "",
+    "src/backbones/tae.py": "class LTAE:\n    pass\n\n\nclass LTAE4WTAE:\n    pass\n",
+    "src/backbones/temporal_aggregator.py": "class TemporalAggregator:\n    pass\n",
+    "src/backbones/utae.py": ("from src.backbones.tae import LTAE\n"
+                              "from src.backbones.temporal_aggregator import TemporalAggregator\n"),
+    "src/backbones/wtae.py": ("from src.backbones.tae import LTAE4WTAE\n"
+                              "from src.backbones.temporal_aggregator import TemporalAggregator\n"),
+    "src/backbones/timeunet.py": ("from src.backbones.tae import LTAE\n"
+                                  "from src.backbones.temporal_aggregator import TemporalAggregator\n\n\n"
+                                  "class TimeUNet_v1:\n    def forward(self, input, batch_positions=None, return_att=False):\n"
+                                  "        return input\n"),
+}
+
+
+def test_install_imports_then_uninstall_restores_the_reference_classes(tmp_path):
     """install() doing the importing itself must still remember the reference classes (the model files import
     src.backbones.tae, so saving while importing would record the fused class as the original)."""
     import subprocess
+    for rel, text in STAND_IN_REFERENCE.items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(text)
     code = (
-        "import sys; sys.path.insert(0, '/root/reference'); sys.path.insert(0, %r)\n"
+        "import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
         "import crop2seg_b200 as c2s\n"
         "swapped = c2s.install(assume_zero_padded=True)\n"
         "import src.backbones.utae as u, src.backbones.tae as t, src.backbones.timeunet as tu\n"
@@ -175,7 +195,7 @@ def test_install_imports_then_uninstall_restores_the_reference_classes():
         "assert t.LTAE.__module__ == 'src.backbones.tae' and u.LTAE is t.LTAE and tu.LTAE is t.LTAE\n"
         "assert u.TemporalAggregator.__module__ == 'src.backbones.temporal_aggregator'\n"
         "assert tu.TimeUNet_v1.forward is not wrapped and c2s.LTAE().assume_zero_padded is False\n"
-        "print('ok')\n") % ROOT
+        "print('ok')\n") % (str(tmp_path), ROOT)
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert res.returncode == 0 and "ok" in res.stdout, res.stderr[-2000:]
 
