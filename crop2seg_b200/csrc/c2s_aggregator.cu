@@ -17,9 +17,7 @@
 #include <cstdlib>
 #include <type_traits>
 
-#include <cuda.h>
-
-#include "c2s_common.cuh"
+#include "c2s_sm100.cuh"
 
 namespace c2s {
 namespace {
@@ -42,17 +40,6 @@ struct AggArgs {
   int pv_per_plane;  // hw / VEC
   int items_per_b;   // (C / CPT) * pv_per_plane
 };
-
-// ATen area_pixel_compute_source_index(scale, dst, align_corners=false) + the i0/i1/lambda split
-// of upsample_bilinear2d (called through nn.Upsample at temporal_aggregator.py:17-19).
-__device__ __forceinline__ void source_index(float scale, int dst, int in_size, int& i0, int& i1, float& l1) {
-  float src = scale * (static_cast<float>(dst) + 0.5f) - 0.5f;
-  src = src < 0.f ? 0.f : src;
-  i0 = static_cast<int>(src);
-  i0 = i0 < in_size - 1 ? i0 : in_size - 1;
-  i1 = i0 + (i0 < in_size - 1 ? 1 : 0);
-  l1 = src - static_cast<float>(i0);
-}
 
 template <typename T, int VEC>
 struct PixelVec;  // VEC pixels of one channel
@@ -286,38 +273,6 @@ __global__ void avg_pool_kernel(const float* __restrict__ in, float* __restrict_
 constexpr int kPipeCPT = 4;
 constexpr int kPipeMaxConsumers = 256;
 
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-// 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (TMA engine, UBLKCP in SASS)
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ uint4 lds_v4(uint32_t addr) {
-  uint4 r;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
-  return r;
-}
-
 // The CTAs of a sample do work proportional to its number of valid frames (27 .. 61 in the benchmark) and the hardware
 // hands CTAs out in grid order, so the kernel's tail is whatever the last samples happen to be.  One small CTA sorts the
 // samples by decreasing length (rank by counting, stable) and the pipelined kernel walks the grid's y dimension through
@@ -390,16 +345,16 @@ __global__ void __launch_bounds__(kPipeMaxConsumers + 32, (S >= 4 && sizeof(T) =
     if (threadIdx.x == 0) {
       n_frames_s = count;
       for (int s = 0; s < n_stages; ++s) {
-        mbar_init(smem_addr(&bars[s]), 1);
-        mbar_init(smem_addr(&bars[16 + s]), n_cwarps);
+        mbar_init(s32(&bars[s]), 1);
+        mbar_init(s32(&bars[16 + s]), n_cwarps);
       }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+      fence_mbarrier_init();
     }
   }
   __syncthreads();
   const int n_frames = n_frames_s;
   const size_t frame_stride = static_cast<size_t>(a.C) * a.hw;
-  const uint32_t stage0 = smem_addr(pipe_smem);
+  const uint32_t stage0 = s32(pipe_smem);
 
   if (warp == n_cwarps) {  // ---- producer -------------------------------------------------------------
     if (lane == 0) {
@@ -410,8 +365,8 @@ __global__ void __launch_bounds__(kPipeMaxConsumers + 32, (S >= 4 && sizeof(T) =
       const uint32_t tap_bytes = TAPS ? static_cast<uint32_t>(n_rows_att * a.wa) * 4u : 0u;
       for (int i = 0; i < n_frames; ++i) {
         const int s = i % n_stages, round = i / n_stages;
-        if (round > 0) mbar_wait(smem_addr(&bars[16 + s]), (round - 1) & 1);
-        const uint32_t full = smem_addr(&bars[s]);
+        if (round > 0) mbar_wait(s32(&bars[16 + s]), (round - 1) & 1);
+        const uint32_t full = s32(&bars[s]);
         mbar_expect_tx(full, stage_bytes + tap_bytes);
         const T* fp = src + static_cast<size_t>(frames[i]) * frame_stride;
 #pragma unroll
@@ -478,7 +433,7 @@ __global__ void __launch_bounds__(kPipeMaxConsumers + 32, (S >= 4 && sizeof(T) =
       }
     }
     const int s = i % n_stages;
-    mbar_wait(smem_addr(&bars[s]), (i / n_stages) & 1);
+    mbar_wait(s32(&bars[s]), (i / n_stages) & 1);
     uint4 xv[kPipeCPT];
     const uint32_t base = stage0 + s * stage_stride + my_off;
 #pragma unroll
@@ -489,7 +444,7 @@ __global__ void __launch_bounds__(kPipeMaxConsumers + 32, (S >= 4 && sizeof(T) =
       for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
     }
     __syncwarp();
-    if (lane == 0) mbar_arrive(smem_addr(&bars[16 + s]));  // the stage's data now lives in registers
+    if (lane == 0) mbar_arrive(s32(&bars[16 + s]));  // the stage's data now lives in registers
 
     float w[VEC];
 #pragma unroll
@@ -645,13 +600,6 @@ __global__ void skipconv_prep_kernel(const float* __restrict__ w, uint4* __restr
   frag[4 * 4 * 32 + idx] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
 }
 
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-      "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-
 template <int S, bool TAPS>
 __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(const __grid_constant__ CUtensorMap map_x,
                                                                              const __grid_constant__ CUtensorMap map_att,
@@ -693,15 +641,15 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
     if (threadIdx.x == 0) {
       n_frames_s = count;
       for (int s = 0; s < n_stages; ++s) {
-        mbar_init(smem_addr(&bars[s]), 1);
-        mbar_init(smem_addr(&bars[16 + s]), n_cwarps);
+        mbar_init(s32(&bars[s]), 1);
+        mbar_init(s32(&bars[16 + s]), n_cwarps);
       }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+      fence_mbarrier_init();
     }
   }
   __syncthreads();
   const int n_frames = n_frames_s;
-  const uint32_t stage0 = smem_addr(pipe_smem);
+  const uint32_t stage0 = s32(pipe_smem);
 
   if (warp == n_cwarps) {  // ---- producer: one box {128 pixels, 64 channels, 1 frame} per valid frame and, with staged
     // taps, one box {tap_floats of the map from row r_lo, 1 frame, 16 heads} of the attention (16 separate bulk copies
@@ -710,8 +658,8 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
       const uint32_t tap_bytes = taps ? 16u * k.tap_floats * 4u : 0u;
       for (int i = 0; i < n_frames; ++i) {
         const int s = i % n_stages, round = i / n_stages;
-        if (round > 0) mbar_wait(smem_addr(&bars[16 + s]), (round - 1) & 1);
-        const uint32_t full = smem_addr(&bars[s]);
+        if (round > 0) mbar_wait(s32(&bars[16 + s]), (round - 1) & 1);
+        const uint32_t full = s32(&bars[s]);
         mbar_expect_tx(full, kScStageBytes + tap_bytes);
         tma_load_3d(stage0 + s * stage_stride, &map_x, pblk * kScPB, 0, b * a.T + frames[i], full);
         if (taps) tma_load_3d(stage0 + s * stage_stride + kScStageBytes, &map_att, r_lo * a.wa, b * a.T + frames[i], 0, full);
@@ -776,7 +724,7 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
       }
     }
     const int s = i % n_stages;
-    mbar_wait(smem_addr(&bars[s]), (i / n_stages) & 1);
+    mbar_wait(s32(&bars[s]), (i / n_stages) & 1);
     uint4 xv[4];
     const uint32_t base = stage0 + s * stage_stride + my_off;
 #pragma unroll
@@ -787,7 +735,7 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
       for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
     }
     __syncwarp();
-    if (lane == 0) mbar_arrive(smem_addr(&bars[16 + s]));
+    if (lane == 0) mbar_arrive(s32(&bars[16 + s]));
 
     float w[VEC];
 #pragma unroll
@@ -828,23 +776,17 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
     // B fragments: ldmatrix.x4.trans of the four 8x8 blocks (k 0-7 | 8-15) x (n 0-7 | 8-15) of this k-step
     const int mrow = ks * 16 + (lane & 7) + ((lane >> 3) & 1) * 8;  // channel row this lane addresses
     const int ncol = warp * 16 + (lane >> 4) * 8;                   // first pixel of the 8x8 block
-    uint32_t b0, b1, b2, b3;
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(b0), "=r"(b1), "=r"(b2), "=r"(b3)
-                 : "r"(tile + mrow * kScTileStride + ncol * 2));
+    uint32_t bf[4];
+    ldsm_x4_trans(bf, tile + mrow * kScTileStride + ncol * 2);
 #pragma unroll
     for (int mt = 0; mt < 4; ++mt) {
-      const uint4 ah = __ldg(k.wfrag + (mt * 4 + ks) * 32 + lane);
-      const uint4 al = __ldg(k.wfrag + 4 * 4 * 32 + (mt * 4 + ks) * 32 + lane);
+      const uint4 h4 = __ldg(k.wfrag + (mt * 4 + ks) * 32 + lane);
+      const uint4 l4 = __ldg(k.wfrag + 4 * 4 * 32 + (mt * 4 + ks) * 32 + lane);
+      const uint32_t ah[4] = {h4.x, h4.y, h4.z, h4.w}, al[4] = {l4.x, l4.y, l4.z, l4.w};
 #pragma unroll
       for (int nt = 0; nt < 2; ++nt) {
-        const uint32_t bb0 = nt ? b2 : b0, bb1 = nt ? b3 : b1;
-        asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                     : "+f"(d[mt][nt][0]), "+f"(d[mt][nt][1]), "+f"(d[mt][nt][2]), "+f"(d[mt][nt][3])
-                     : "r"(ah.x), "r"(ah.y), "r"(ah.z), "r"(ah.w), "r"(bb0), "r"(bb1));
-        asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                     : "+f"(d[mt][nt][0]), "+f"(d[mt][nt][1]), "+f"(d[mt][nt][2]), "+f"(d[mt][nt][3])
-                     : "r"(al.x), "r"(al.y), "r"(al.z), "r"(al.w), "r"(bb0), "r"(bb1));
+        mma_bf16(d[mt][nt], ah, bf[2 * nt], bf[2 * nt + 1]);
+        mma_bf16(d[mt][nt], al, bf[2 * nt], bf[2 * nt + 1]);
       }
     }
   }
@@ -862,21 +804,6 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
         *reinterpret_cast<uint32_t*>(op + static_cast<size_t>(o) * a.hw + nt * 8) = Elem<T>::pack2(v0, v1);
       }
     }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn agg_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
 }
 
 template <int S, bool TAPS>
@@ -1082,35 +1009,22 @@ int c2s_agg_skipconv_forward(const c2s_agg_desc* d, const void* x, const float* 
                       tap_floats <= 256 && scale_class >= 4;
     k.tap_floats = taps ? tap_floats : 0;
   }
-  EncodeTiledFn fn = agg_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return C2S_ERR_CUDA;
-  }
   CUtensorMap map_x;  // x as [B*T][C][H*W] bf16; box = 128 pixels x 64 channels x 1 frame, dense in shared memory
   const cuuint64_t dims[3] = {static_cast<cuuint64_t>(hw), static_cast<cuuint64_t>(kScC), static_cast<cuuint64_t>(d->B) * d->T};
   const cuuint64_t strides[2] = {static_cast<cuuint64_t>(hw) * 2, static_cast<cuuint64_t>(kScC) * hw * 2};
-  const cuuint32_t box[3] = {kScPB, kScC, 1}, estr[3] = {1, 1, 1};
-  const CUresult r = fn(&map_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (skip features) failed with CUresult %d", static_cast<int>(r));
-    return C2S_ERR_CUDA;
-  }
+  const cuuint32_t box[3] = {kScPB, kScC, 1};
+  status = encode_tensor_map(&map_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                             CU_TENSOR_MAP_L2_PROMOTION_NONE, "skip features");
+  if (status != C2S_OK) return status;
   CUtensorMap map_att = map_x;  // attention as [16 heads][B*T][ha*wa] fp32; box = tap_floats of one map x 1 frame x 16 heads
   if (k.tap_floats > 0) {
     const cuuint64_t amap = static_cast<cuuint64_t>(d->ha) * d->wa;
     const cuuint64_t adims[3] = {amap, static_cast<cuuint64_t>(d->B) * d->T, 16};
     const cuuint64_t astrides[2] = {amap * 4, static_cast<cuuint64_t>(d->B) * d->T * amap * 4};
     const cuuint32_t abox[3] = {static_cast<cuuint32_t>(k.tap_floats), 1, 16};
-    const CUresult ra = fn(&map_att, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(attn), adims, astrides, abox, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (ra != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled (attention) failed with CUresult %d", static_cast<int>(ra));
-      return C2S_ERR_CUDA;
-    }
+    status = encode_tensor_map(&map_att, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, attn, adims, astrides, abox,
+                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, "attention");
+    if (status != C2S_OK) return status;
   }
   switch (scale_class) {
     case 2: return launch_skipconv<2>(map_x, map_att, k, stream, "agg_skipconv<x2>");

@@ -13,7 +13,7 @@
 
 #include <cstdlib>
 
-#include "c2s_common.cuh"
+#include "c2s_sm100.cuh"
 
 namespace c2s {
 namespace {
@@ -34,15 +34,6 @@ struct AggBwdArgs {
   int hw, vecs_per_plane;
   int t_chunks, t_per_chunk;  // the frame loop is split over blockIdx.z (set by launch_bwd)
 };
-
-__device__ __forceinline__ void bwd_source_index(float scale, int dst, int in_size, int& i0, int& i1, float& l1) {
-  float src = scale * (static_cast<float>(dst) + 0.5f) - 0.5f;
-  src = src < 0.f ? 0.f : src;
-  i0 = static_cast<int>(src);
-  i0 = i0 < in_size - 1 ? i0 : in_size - 1;
-  i1 = i0 + (i0 < in_size - 1 ? 1 : 0);
-  l1 = src - static_cast<float>(i0);
-}
 
 template <typename T, int VEC>
 struct BVec {
@@ -101,12 +92,12 @@ __global__ void __launch_bounds__(kBwdThreads) agg_backward_kernel(const AggBwdA
   int gcol0[(S == 0) ? VEC : 1], gcol1[(S == 0) ? VEC : 1];
   if constexpr (S >= 0) {
     int iy0, iy1;
-    bwd_source_index(a.sy, y, a.ha, iy0, iy1, ly1);
+    source_index(a.sy, y, a.ha, iy0, iy1, ly1);
     row0 = iy0 * a.wa, row1 = iy1 * a.wa;
 #pragma unroll
     for (int j = 0; j < VEC; ++j) {
       int i0, i1;
-      bwd_source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
+      source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
       if constexpr (S == 0) gcol0[j] = i0, gcol1[j] = i1;
     }
     if constexpr (S > 0) cmin = x0 / S - 1;
@@ -269,37 +260,6 @@ __global__ void __launch_bounds__(kBwdThreads) agg_backward_kernel(const AggBwdA
 constexpr int kBwdPipeCPT = 4;
 constexpr int kBwdPipeMaxConsumers = 256;
 
-__device__ __forceinline__ uint32_t bsmem_addr(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void bmbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void bmbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bmbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void bmbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void bbulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-               "l"(src), "r"(bytes), "r"(bar)
-               : "memory");
-}
-__device__ __forceinline__ uint4 blds_v4(uint32_t addr) {
-  uint4 r;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
-  return r;
-}
-
 // TAPS: as in the forward (c2s_aggregator.cu), the attention rows of the pixel block ride in the stage as one more bulk
 // copy and the consumers read their taps from shared memory instead of 2 * NCOL global loads per thread and frame.
 template <typename T, int S, bool TAPS>
@@ -329,23 +289,23 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
     const int pb = n_consumers * VEC;
     int i0, i1;
     float l1;
-    bwd_source_index(a.sy, (pblk * pb) / a.W, a.ha, i0, i1, l1);
+    source_index(a.sy, (pblk * pb) / a.W, a.ha, i0, i1, l1);
     r_lo = i0;
-    bwd_source_index(a.sy, (pblk * pb + pb - 1) / a.W, a.ha, i0, i1, l1);
+    source_index(a.sy, (pblk * pb + pb - 1) / a.W, a.ha, i0, i1, l1);
     n_rows_att = i1 - r_lo + 1;
   }
 
   for (int t = threadIdx.x; t < a.T; t += blockDim.x) s_pad[t] = a.pad != nullptr && a.pad[b * a.T + t] != 0;
   if (threadIdx.x == 0) {
     for (int s = 0; s < n_stages; ++s) {
-      bmbar_init(bsmem_addr(&bars[s]), 1);
-      bmbar_init(bsmem_addr(&bars[16 + s]), n_cwarps);
+      mbar_init(s32(&bars[s]), 1);
+      mbar_init(s32(&bars[16 + s]), n_cwarps);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   __syncthreads();
   const size_t frame_stride = static_cast<size_t>(a.C) * a.hw;
-  const uint32_t stage0 = bsmem_addr(bpipe_smem);
+  const uint32_t stage0 = s32(bpipe_smem);
   const size_t plane0 = static_cast<size_t>(c0) * a.hw + static_cast<size_t>(pblk) * n_consumers * VEC;
 
   if (warp == n_cwarps) {  // ---- producer: the valid frames of the chunk, in order ------------------------
@@ -358,14 +318,14 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
       for (int t = t_begin; t < t_end; ++t) {
         if (s_pad[t]) continue;
         const int s = i % n_stages, round = i / n_stages;
-        if (round > 0) bmbar_wait(bsmem_addr(&bars[16 + s]), (round - 1) & 1);
-        const uint32_t full = bsmem_addr(&bars[s]);
-        bmbar_expect_tx(full, stage_bytes + tap_bytes);
+        if (round > 0) mbar_wait(s32(&bars[16 + s]), (round - 1) & 1);
+        const uint32_t full = s32(&bars[s]);
+        mbar_expect_tx(full, stage_bytes + tap_bytes);
         const T* fp = src + static_cast<size_t>(t) * frame_stride;
 #pragma unroll
         for (int k = 0; k < CPT; ++k)
-          bbulk_g2s(stage0 + s * stage_stride + k * row_bytes, fp + static_cast<size_t>(k) * a.hw, row_bytes, full);
-        if (TAPS) bbulk_g2s(stage0 + s * stage_stride + stage_bytes, att_src + static_cast<size_t>(t) * amap_p, tap_bytes, full);
+          bulk_g2s(stage0 + s * stage_stride + k * row_bytes, fp + static_cast<size_t>(k) * a.hw, row_bytes, full);
+        if (TAPS) bulk_g2s(stage0 + s * stage_stride + stage_bytes, att_src + static_cast<size_t>(t) * amap_p, tap_bytes, full);
         ++i;
       }
     }
@@ -378,14 +338,14 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
   const int y = p0 / a.W, x0 = p0 - y * a.W;
   int iy0, iy1;
   float ly1;
-  bwd_source_index(a.sy, y, a.ha, iy0, iy1, ly1);
+  source_index(a.sy, y, a.ha, iy0, iy1, ly1);
   const int row0 = iy0 * a.wa, row1 = iy1 * a.wa;
   const float ly0 = 1.f - ly1;
   float lx1[VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) {
     int i0, i1;
-    bwd_source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
+    source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
   }
   const int cmin = x0 / S - 1;
   auto clampc = [&](int c) { return c < 0 ? 0 : (c > a.wa - 1 ? a.wa - 1 : c); };
@@ -426,11 +386,11 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
       }
     }
     const int s = i % n_stages;
-    bmbar_wait(bsmem_addr(&bars[s]), (i / n_stages) & 1);
+    mbar_wait(s32(&bars[s]), (i / n_stages) & 1);
     uint4 xv[CPT];
     const uint32_t base = stage0 + s * stage_stride + my_off;
 #pragma unroll
-    for (int k = 0; k < CPT; ++k) xv[k] = blds_v4(base + k * row_bytes);
+    for (int k = 0; k < CPT; ++k) xv[k] = lds_v4(base + k * row_bytes);
     if (TAPS) {
       const float* tp = reinterpret_cast<const float*>(bpipe_smem + s * stage_stride + stage_bytes);
       const int trow0 = row0 - r_lo * a.wa, trow1 = row1 - r_lo * a.wa;
@@ -441,7 +401,7 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
       }
     }
     __syncwarp();
-    if (lane == 0) bmbar_arrive(bsmem_addr(&bars[16 + s]));  // the stage's data now lives in registers
+    if (lane == 0) mbar_arrive(s32(&bars[16 + s]));  // the stage's data now lives in registers
     ++i;
 
     float g[VEC];  // sum_c x * grad_out of this thread's pixels

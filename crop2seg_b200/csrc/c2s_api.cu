@@ -1,8 +1,9 @@
-// Library services of the crop2seg_b200 C ABI: error text, launch accounting, ABI version.
+// Library services of the crop2seg_b200 C ABI: error text, launch accounting, ABI version; tensor maps and SM counts for the
+// kernels.
 #include <atomic>
 #include <cstring>
 
-#include "c2s_common.cuh"
+#include "c2s_sm100.cuh"
 
 namespace c2s {
 
@@ -29,6 +30,42 @@ int set_max_dynamic_smem(const void* func, int bytes, std::atomic<unsigned long 
   C2S_CUDA(cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes < room ? bytes : room));
   done->fetch_or(bit, std::memory_order_release);
   return C2S_OK;
+}
+
+int encode_tensor_map(CUtensorMap* map, CUtensorMapDataType dtype, cuuint32_t rank, const void* base, const cuuint64_t* dims,
+                      const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle,
+                      CUtensorMapL2promotion l2_promotion, const char* what) {
+  using EncodeTiledFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  // the driver entry point, looked up once (the library does not link libcuda); static initialisation is thread-safe
+  static const EncodeTiledFn fn = []() -> EncodeTiledFn {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+        q == cudaDriverEntryPointSuccess)
+      return reinterpret_cast<EncodeTiledFn>(p);
+    return nullptr;
+  }();
+  if (fn == nullptr) {
+    set_error("cuTensorMapEncodeTiled is not available from the driver");
+    return C2S_ERR_CUDA;
+  }
+  const cuuint32_t elem_strides[5] = {1, 1, 1, 1, 1};
+  const CUresult r = fn(map, dtype, rank, const_cast<void*>(base), dims, strides, box, elem_strides,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2_promotion, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled (%s) failed with CUresult %d", what, static_cast<int>(r));
+    return C2S_ERR_CUDA;
+  }
+  return C2S_OK;
+}
+
+int sm_count() {
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+    sms = 148;
+  return sms;
 }
 
 void set_error(const char* fmt, ...) {

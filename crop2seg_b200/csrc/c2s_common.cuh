@@ -140,6 +140,18 @@ __device__ __forceinline__ float warp_max(float v) {
   return v;
 }
 
+// ATen area_pixel_compute_source_index(scale, dst, align_corners=false) + the i0/i1/lambda split of upsample_bilinear2d
+// (nn.Upsample of the attention masks, reference temporal_aggregator.py:17-19).  The aggregator's forward and backward
+// must agree on it.
+__device__ __forceinline__ void source_index(float scale, int dst, int in_size, int& i0, int& i1, float& l1) {
+  float src = scale * (static_cast<float>(dst) + 0.5f) - 0.5f;
+  src = src < 0.f ? 0.f : src;
+  i0 = static_cast<int>(src);
+  i0 = i0 < in_size - 1 ? i0 : in_size - 1;
+  i1 = i0 + (i0 < in_size - 1 ? 1 : 0);
+  l1 = src - static_cast<float>(i0);
+}
+
 inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 
 }  // namespace c2s

@@ -17,15 +17,15 @@
 //       descriptor accepts any 128-byte-aligned start when the swizzle follows the absolute address), so shared memory is
 //       filled at 1x the input bytes instead of 9x;
 //     * the prepared weights [64][9 * C_in] (bf16, K-major, 64-wide swizzled chunks) stay resident in shared memory;
-//     * one elected thread issues tcgen05.mma (M 128, N 64, K 16) into one of two TMEM accumulators; tcgen05.commit frees
-//       ring slots and hands the accumulator to eight epilogue warps (tcgen05.ld), which add the bias, store the raw
-//       (pre-normalisation) row as bf16 NCHW and keep the GroupNorm sums of their frame in registers (one atomic per warp
-//       and quarter of the channels per unit).
+//     * one elected thread issues the tcgen05 products (umma_bf16: M 128, N 64, K 16) into one of two TMEM accumulators;
+//       umma_commit frees ring slots and hands the accumulator to eight epilogue warps (tmem_ld32), which add the bias,
+//       store the raw (pre-normalisation) row as bf16 NCHW and keep the GroupNorm sums of their frame in registers (one
+//       atomic per warp and quarter of the channels per unit).
 //   c2s_group_stats      per-(frame, group) sum / sum of squares of a raw NCHW tensor (layers whose convolution ran elsewhere)
 //   c2s_group_norm_relu  y = relu((x - mean) * rstd * gamma + beta) [+ residual]: the second, element-wise pass
 //                        (GroupNorm needs the statistics of the whole frame before the first output element).
 // Forward only (inference).  bf16 features; the statistics and the normalisation are fp32.
-#include "c2s_common.cuh"
+#include "c2s_sm100.cuh"
 
 namespace c2s {
 namespace {
@@ -54,63 +54,8 @@ struct ConvArgs {
   float in_eps;
 };
 
-__device__ __forceinline__ uint32_t s32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-// K-major operand, 128-byte swizzle: rows of 128 B, 8-row groups 1024 B apart; any 128-byte aligned start
-__device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3fff);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(1024 >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(2) << 61;
-  return d;
-}
-// the same descriptor from its low word ((address >> 4) | leading byte offset 1 << 16); the high word is constant
-__device__ __forceinline__ uint64_t desc_from(uint32_t lo) {
-  constexpr uint32_t hi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO 1024 B, descriptor version 1, SWIZZLE_128B
-  return (static_cast<uint64_t>(hi) << 32) | lo;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// one lane of a converged warp (the compiler then knows that exactly one thread issues the tcgen05 instructions)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n .reg .pred p;\n elect.sync _|p, 0xffffffff;\n selp.u32 %0, 1, 0, p;\n}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
+// the low-word shortcut of umma_desc_k_sw128: ((address >> 4) | leading byte offset 1 << 16) with the constant high word
+__device__ __forceinline__ uint64_t desc_from(uint32_t lo) { return (static_cast<uint64_t>(kUmmaDescHiSw128) << 32) | lo; }
 
 // the unit -> (frame, rows) arithmetic shared by the three roles
 struct Unit {
@@ -159,11 +104,11 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
     constexpr int kRowWarps = (kRowBlocks < 128 && kRowBlocks % 32 == 0) ? kRowBlocks / 32 : 4;
     for (int s = 0; s < kRing; ++s) mbar_init(full(s), kRowWarps), mbar_init(empty(s), 1);   // one arrival per warp serving the row
     for (int b = 0; b < kAccBufs; ++b) mbar_init(tfull(b), 1), mbar_init(tempty(b), 8);       // one arrival per epilogue warp
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(s32(&tmem_s)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(s32(&tmem_s), 256);
+    tmem_relinquish();
   }
   if (tid < kCN) s_bias[tid] = a.bias != nullptr ? a.bias[tid] : 0.f;
   // resident weights: [chunk][64 rows n][128 B], 16-byte pieces at chunk position c16 ^ (n & 7)
@@ -172,25 +117,20 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
     const uint4 v = *reinterpret_cast<const uint4*>(a.wp + static_cast<size_t>(n) * (NCHUNK * 64) + j * 64 + c16 * 8);
     *reinterpret_cast<uint4*>(sm + j * 8192 + n * 128 + ((c16 ^ (n & 7)) << 4)) = v;
   }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  fence_proxy_async();
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tacc = tmem_s;
 
   if (warp == 0) {
     // ---- MMA issuer ----------------------------------------------------------------------------------------------
-    // The issuing thread is the pipeline's clock: tcgen05.mma blocks it while the (shallow) queue is full, so every scalar
+    // The issuing thread is the pipeline's clock: umma_bf16 blocks it while the (shallow) queue is full, so every scalar
     // instruction between the last product of a row and the first one of the next row is tensor-pipe idle time.  The
     // bookkeeping is therefore incremental (no divisions, one barrier wait and one release per row in the steady state)
     // and the tap loops stay rolled: the descriptor arithmetic of a tap sits between the products, not in front of them.
     if (elect_one()) {
-      uint32_t idesc = 0;
-      idesc |= 1u << 4;                                  // D = fp32
-      idesc |= 1u << 7;                                  // A = bf16
-      idesc |= 1u << 10;                                 // B = bf16
-      idesc |= static_cast<uint32_t>(kCN >> 3) << 17;    // N
-      idesc |= static_cast<uint32_t>(kM >> 4) << 24;     // M
+      static constexpr uint32_t idesc = umma_idesc_bf16(kM, kCN);
       const uint32_t b_lo0 = ((base >> 4) & 0x3fffu) | (1u << 16);
       uint32_t in_slot = 0, in_phase = 0;      // ring slot of the next input row to wait for; bit s = parity of slot s
       uint32_t free_slot = 0;                  // ring slot of the next input row to release
@@ -239,7 +179,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
           const long long dbg_t1 = clock64();
           dbg_tempty += dbg_t1 - dbg_t0;
 #endif
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t d_tmem = tacc + buf * kCN;
           uint32_t b_lo = b_lo0;
 #pragma unroll 1
@@ -394,7 +334,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
               if (pb == kCW / 8 - 1 && j == 6) *reinterpret_cast<uint4*>(sl + (kCW + 1) * 128 + ((cb ^ ((kCW + 1) & 7)) << 4)) = w;  // pixel W = pixel W - 2
             }
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic stores -> tensor-core (async proxy) reads
+          fence_proxy_async();  // generic stores -> tensor-core (async proxy) reads
           __syncwarp();
           if (lane == 0) mbar_arrive(full(slot));  // hundreds of per-thread arrivals on one mbarrier cost ~1000 cycles per row
         }
@@ -504,7 +444,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
             if (pb == kCW / 8 - 1 && j == 6) *reinterpret_cast<uint4*>(sl + (kCW + 1) * 128 + ((cb ^ ((kCW + 1) & 7)) << 4)) = w;  // pixel W = pixel W - 2
           }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic stores -> tensor-core (async proxy) reads
+        fence_proxy_async();  // generic stores -> tensor-core (async proxy) reads
         __syncwarp();
         if (lane == 0) mbar_arrive(full(slot));  // hundreds of per-thread arrivals on one mbarrier cost ~1000 cycles per row
       }
@@ -524,11 +464,11 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
       for (int y = t.y0; y < t.y1; ++y, ++o) {
         const unsigned buf = o & (kAccBufs - 1);
         mbar_wait(tfull(buf), (o / kAccBufs) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         uint32_t r0[32];
         tmem_ld32(tacc + (static_cast<uint32_t>(q * 32) << 16) + buf * kCN + half * 32, r0);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tmem_wait_ld();
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(tempty(buf));  // the accumulator is in registers: the next row but one may overwrite it
         // 2-byte stores, 64 contiguous bytes per warp instruction.  (Staging the tile in shared memory for 16-byte stores was
@@ -556,9 +496,9 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv3x3_tc_kernel(const ConvA
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tacc) : "memory");
+  if (warp == 0) tmem_dealloc(tacc, 256);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -615,11 +555,11 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
   if (tid == 0) {
     for (int s = 0; s < kDRing; ++s) mbar_init(full(s), 4), mbar_init(empty(s), 1);
     for (int b = 0; b < kAccBufs; ++b) mbar_init(tfull(b), 1), mbar_init(tempty(b), 8);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(s32(&tmem_s)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(s32(&tmem_s), 256);
+    tmem_relinquish();
   }
   if (tid < kCN) s_bias[tid] = a.bias != nullptr ? a.bias[tid] : 0.f;
   for (int i = tid; i < kCN * kDChunks * 8; i += kConvThreads) {  // resident weights, as in conv3x3_tc_kernel
@@ -627,19 +567,16 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
     const uint4 v = *reinterpret_cast<const uint4*>(a.wp + static_cast<size_t>(n) * (kDChunks * 64) + j * 64 + c16 * 8);
     *reinterpret_cast<uint4*>(sm + j * 8192 + n * 128 + ((c16 ^ (n & 7)) << 4)) = v;
   }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  fence_proxy_async();
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tacc = tmem_s;
 
   if (warp == 0) {
     // ---- MMA issuer ----------------------------------------------------------------------------------------------
     if (elect_one()) {
-      uint32_t idesc = 0;
-      idesc |= 1u << 4, idesc |= 1u << 7, idesc |= 1u << 10;  // D = fp32, A = B = bf16
-      idesc |= static_cast<uint32_t>(kCN >> 3) << 17;          // N = 64
-      idesc |= static_cast<uint32_t>(64 >> 4) << 24;           // M = 64 (kDWo live rows)
+      static constexpr uint32_t idesc = umma_idesc_bf16(64, kCN);  // M = 64 (kDWo live rows)
       const uint32_t b_lo0 = ((base >> 4) & 0x3fffu) | (1u << 16);
       uint32_t in_slot = 0, in_phase = 0;
       uint32_t o = 0;  // output rows handed out so far (accumulator = o & 3)
@@ -659,7 +596,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
 #ifdef C2S_CONV_TIMING
           dbg_full += clock64() - dbg_t, ++dbg_rows;
 #endif
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t row_lo = (((ring + in_slot * kDSlot) >> 4) & 0x3fffu) | (1u << 16);
           // the output rows fed by input row v (v = r, or the row r stands in for at a reflected frame edge)
           auto contribute = [&](int v) {
@@ -681,7 +618,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
 #ifdef C2S_CONV_TIMING
                 dbg_tempty += clock64() - dbg_t2;
 #endif
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
               }
               const uint32_t d_tmem = tacc + buf * kCN;
               // 16 products with compile-time offsets from three bases (even half, odd half, the tap row of the weights):
@@ -784,7 +721,7 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
               *reinterpret_cast<uint4*>(sl + kDWo * 128 + ((cb ^ (kDWo & 7)) << 4)) = w;
           }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(full(slot));
       }
@@ -804,11 +741,11 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
       for (int y = t.y0; y < t.y1; ++y, ++o) {
         const unsigned buf = o & (kAccBufs - 1);
         mbar_wait(tfull(buf), (o / kAccBufs) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         uint32_t r0[32];
         tmem_ld32(tacc + (static_cast<uint32_t>(q * 32) << 16) + buf * kCN + half * 32, r0);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tmem_wait_ld();
+        tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(tempty(buf));
         const size_t cstride = static_cast<size_t>(Ho) * kDWo;
@@ -832,9 +769,9 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tacc) : "memory");
+  if (warp == 0) tmem_dealloc(tacc, 256);
 }
 
 // weight[c_out][c_in][3][3] fp32 -> wp[c_out][chunks * 64] bf16 with k = tap * CK + c (zero for c >= c_in and behind 9 CK)
@@ -1000,8 +937,7 @@ int c2s_conv2d_forward(const c2s_conv_desc* desc, const void* x, const c2s_conv_
   conv_weight_prep_kernel<<<ceil_div(kCN * k_total, 256), 256, 0, stream>>>(weight, wp, kCN, d.c_in, ck, k_total, down ? 16 : 9);
   C2S_LAUNCH_CHECK("conv_weight_prep");
   if (stats != nullptr) C2S_CUDA(cudaMemsetAsync(stats, 0, static_cast<size_t>(d.frames) * kStatQuarters * 2 * sizeof(float), stream));
-  int sms = 148, dev = 0;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   ConvArgs a{};
   a.x = static_cast<const __nv_bfloat16*>(x), a.y = static_cast<__nv_bfloat16*>(y), a.bias = bias, a.stats = stats, a.wp = wp;
   a.frames = d.frames, a.c_in = d.c_in, a.H = d.H;

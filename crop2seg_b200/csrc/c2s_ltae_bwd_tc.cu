@@ -57,18 +57,6 @@ struct BtSmem {
   static_assert(kTotal <= 232448, "shared memory budget");
 };
 
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, int c0, int c1, int c2, int c3, uint32_t src) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
 __device__ __forceinline__ uint32_t mul_bf16x2(uint32_t a, uint32_t b) {
   uint32_t r;
   asm("mul.rn.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
@@ -135,7 +123,7 @@ ltae_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
   // ---- set-up ------------------------------------------------------------------------------------------------------
   if (tid == 0) {
     for (int i = 0; i < 4; ++i) mbar_init(bars + 8 * i, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   for (int i = tid; i < S::kSlab / 16; i += 256) reinterpret_cast<uint4*>(slab_ptr)[i] = make_uint4(0, 0, 0, 0);  // never NaN
   for (int i = tid; i < kTP * S::kPeRowB / 4; i += 256) reinterpret_cast<uint32_t*>(s_pe)[i] = 0u;
@@ -165,7 +153,7 @@ ltae_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
   }
   const float inv_n_all = 1.f / (static_cast<float>(a.T) * CPG);
   const unsigned long long beyond = (a.T >= 64) ? 0ull : (~0ull << a.T);  // frames t >= T
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic zero fill above, bulk-copy writes below
+  fence_proxy_async();  // generic zero fill above, bulk-copy writes below
   __syncthreads();
 
   int cur_b = -1;
@@ -181,7 +169,7 @@ ltae_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
 
     // ---- the tile's boxes (the previous tile's stores have finished reading the slab) ----------------------------------
     if (tid == 0) {
-      asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+      tma_store_wait_read();
 #pragma unroll
       for (int grp = 0; grp < 4; ++grp)
         if (16 * grp < a.T) {
@@ -707,14 +695,14 @@ ltae_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         atomicAdd(a.g_cpos + (static_cast<size_t>(b) * a.T + t) * kMaxHeads + h, s_gc[t * GP + h]);
       }
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic stores above, bulk-copy reads below
+    fence_proxy_async();  // generic stores above, bulk-copy reads below
     __syncthreads();
     for (int i = tid; i < kTP * GP; i += 256) s_gc[i] = 0.f;  // next adds are behind the next tile's first barrier
     if (tid == 0) {
 #pragma unroll
       for (int grp = 0; grp < 4; ++grp)
         if (16 * grp < a.T) tma_store_4d(&map_gx, pix0, 0, 16 * grp, b, slab + 16 * grp * FB);
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+      tma_store_commit();
     }
   }
 
@@ -729,31 +717,14 @@ ltae_bwd_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
       atomicAdd(a.g_gamma + i, s_ggb[i]);
       atomicAdd(a.g_beta + i, s_ggb[C + i]);
     }
-  if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // the last stores have left shared memory
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn bt_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
+  if (tid == 0) tma_store_wait();  // the last stores have left shared memory
 }
 
 template <int C, bool FULL>
 int bt_launch(const CUtensorMap& map_x, const CUtensorMap& map_gx, const BwdTcArgs& a, cudaStream_t stream, const char* name) {
   using S = BtSmem<C>;
   C2S_SMEM_ATTR((ltae_bwd_tc_kernel<C, FULL>), S::kTotal);
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-    sms = 148;
+  const int sms = sm_count();
   const int grid = a.n_tiles < sms ? a.n_tiles : sms;
   ltae_bwd_tc_kernel<C, FULL><<<static_cast<unsigned>(grid), 256, S::kTotal, stream>>>(map_x, map_gx, a);
   C2S_LAUNCH_CHECK(name);
@@ -776,30 +747,21 @@ bool ltae_bwd_tc_eligible(const c2s_ltae_desc& d, const void* x, const c2s_ltae_
 }
 
 int ltae_bwd_tc_launch(const c2s_ltae_desc& d, const BwdTcArgs& a0, void* grad_x, cudaStream_t stream) {
-  EncodeTiledFn fn = bt_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return C2S_ERR_CUDA;
-  }
   const int C = d.C, hw = d.H * d.W;
   // x / grad_x as [B][T][C][hw] bf16; box = 8 pixels x C channels x 16 frames of one sample: frames t >= T are zero-filled
   // by the loads and clipped by the stores
   CUtensorMap maps[2];
-  void* bases[2] = {const_cast<__nv_bfloat16*>(a0.x), grad_x};
+  const void* bases[2] = {a0.x, grad_x};
+  const char* what[2] = {"backward features", "backward feature gradients"};
   const cuuint64_t dims[4] = {static_cast<cuuint64_t>(hw), static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(d.T),
                               static_cast<cuuint64_t>(d.B)};
   const cuuint64_t strides[3] = {static_cast<cuuint64_t>(hw) * 2, static_cast<cuuint64_t>(C) * hw * 2,
                                  static_cast<cuuint64_t>(d.T) * C * hw * 2};
   const cuuint32_t box[4] = {kPix, static_cast<cuuint32_t>(C), 16, 1};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
   for (int i = 0; i < 2; ++i) {
-    const CUresult r = fn(&maps[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, bases[i], dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled (backward features, map %d) failed with CUresult %d", i, static_cast<int>(r));
-      return C2S_ERR_CUDA;
-    }
+    const int status = encode_tensor_map(&maps[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, bases[i], dims, strides, box,
+                                         CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, what[i]);
+    if (status != C2S_OK) return status;
   }
   BwdTcArgs a = a0;
   a.tiles_per_b = hw / kPix;

@@ -128,7 +128,7 @@ ltae_fa_kernel(const __grid_constant__ CUtensorMap map16, const __grid_constant_
   // ---- set-up: barriers, resident weights ----------------------------------------------------------------
   if (tid == 0) {
     for (int i = 0; i < NBUF * 4; ++i) mbar_init(bars + 8 * i, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   {
     uint4* wc = reinterpret_cast<uint4*>(smem + S::oWc);
@@ -744,7 +744,7 @@ ltae_fa_kernel(const __grid_constant__ CUtensorMap map16, const __grid_constant_
 
     FA_DBG(17);
     // ---- the slab is free: bring the tile after next (NBUF = 2) / the next tile (NBUF = 1) -------------------
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic writes above, bulk-copy writes below
+    fence_proxy_async();  // generic writes above, bulk-copy writes below
     if (tid == 0) cp_async_wait_all();  // the masks of the slab's next tile have landed long ago
     __syncthreads();
     FA_DBG(18);
@@ -827,37 +827,12 @@ __global__ void fa_build_w16_kernel(const float* __restrict__ w, const float* __
   wf[n + i] = lo;
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn fa_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
-int fa_sm_count() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
-      n = 148;
-  }
-  return n;
-}
-
 template <int C, int WPP>
 int fa_launch(const CUtensorMap& map16, const CUtensorMap& map4, const CUtensorMap& map1, const FaArgs& a,
               cudaStream_t stream, const char* name) {
   using S = FaSmem<C, WPP>;
   C2S_SMEM_ATTR((ltae_fa_kernel<C, WPP>), S::kTotal);
-  const int slots = fa_sm_count() * (WPP == 1 ? 2 : 1);  // persistent CTAs: one per SM, two for the single-warp tiles
+  const int slots = sm_count() * (WPP == 1 ? 2 : 1);  // persistent CTAs: one per SM, two for the single-warp tiles
   const int grid = a.n_tiles < slots ? a.n_tiles : slots;
   ltae_fa_kernel<C, WPP><<<static_cast<unsigned>(grid), 256 * WPP, S::kTotal, stream>>>(map16, map4, map1, a);
   C2S_LAUNCH_CHECK(name);
@@ -907,26 +882,17 @@ int ltae_fa_forward(const c2s_ltae_desc& d, const c2s_ltae_params& p, const void
     C2S_LAUNCH_CHECK("ltae_fa_build_wc16");
   }
 
-  EncodeTiledFn fn = fa_encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return C2S_ERR_CUDA;
-  }
   CUtensorMap map16, map4, map1;
   const cuuint64_t dims[3] = {static_cast<cuuint64_t>(hw), static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(d.B) * d.T};
   const cuuint64_t strides[2] = {static_cast<cuuint64_t>(hw) * 2, static_cast<cuuint64_t>(C) * hw * 2};
-  const cuuint32_t estr[3] = {1, 1, 1};
   CUtensorMap* maps[3] = {&map16, &map4, &map1};
   const cuuint32_t frames[3] = {16, 4, 1};
+  const char* what[3] = {"features, 16 frames per box", "features, 4 frames per box", "features, 1 frame per box"};
   for (int i = 0; i < 3; ++i) {
     const cuuint32_t box[3] = {kPix, static_cast<cuuint32_t>(C), frames[i]};
-    const CUresult r = fn(maps[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(x), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled (features, %u frames per box) failed with CUresult %d", frames[i], static_cast<int>(r));
-      return C2S_ERR_CUDA;
-    }
+    const int status = encode_tensor_map(maps[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, x, dims, strides, box,
+                                         CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, what[i]);
+    if (status != C2S_OK) return status;
   }
 
   FaArgs a{};

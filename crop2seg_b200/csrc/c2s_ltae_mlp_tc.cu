@@ -5,12 +5,11 @@
 //                                                                                              tae.py:444-448, 488
 // One CTA = 128 rows.  o (bf16 hi + lo, written by ltae_mma_kernel) and mlp.0.weight (bf16 hi + lo) are K-major;
 // TMA (cp.async.bulk.tensor, 128-byte swizzle) brings 64-wide K chunks into a 2-stage ring, one elected thread
-// issues tcgen05.mma (M = 128, N = c_out, K = 16 per instruction) for the three products hi*hi + lo*hi + hi*lo into
-// one fp32 accumulator in tensor memory, tcgen05.commit signals an mbarrier, and the four warps read their 32 TMEM
-// lanes (= 32 pixel rows) back with tcgen05.ld for the epilogue, which needs every channel of a pixel in one thread.
-#include <cuda.h>
-
+// issues the tcgen05 products (umma_bf16: M = 128, N = c_out, K = 16 per instruction) for hi*hi + lo*hi + hi*lo into
+// one fp32 accumulator in tensor memory, umma_commit signals an mbarrier, and the four warps read their 32 TMEM
+// lanes (= 32 pixel rows) back with tmem_ld32 for the epilogue, which needs every channel of a pixel in one thread.
 #include "c2s_ltae_prep.cuh"
+#include "c2s_sm100.cuh"
 
 namespace c2s {
 namespace {
@@ -34,74 +33,6 @@ struct MlpArgs {
   int n_rows, hw, c_out, tmem_cols;
 };
 
-__device__ __forceinline__ uint32_t s32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-// K-major operand tile in shared memory, 128-byte swizzle: rows of 128 B, 8-row atoms of 1024 B (SBO), LBO = 1
-__device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3fff);   // start address, 16-byte units
-  d |= static_cast<uint64_t>(1) << 16;                      // leading byte offset (unused for swizzled K-major)
-  d |= static_cast<uint64_t>(1024 >> 4) << 32;              // stride byte offset between 8-row groups
-  d |= static_cast<uint64_t>(1) << 46;                      // descriptor version (Blackwell)
-  d |= static_cast<uint64_t>(2) << 61;                      // SWIZZLE_128B
-  return d;
-}
-// kind::f16 instruction descriptor: bf16 x bf16 -> fp32, both operands K-major, M = 128
-__device__ __forceinline__ uint32_t umma_idesc_bf16(int n) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                   // c_format = F32
-  d |= 1u << 7;                                   // a_format = BF16
-  d |= 1u << 10;                                  // b_format = BF16
-  d |= static_cast<uint32_t>(n >> 3) << 17;       // n_dim
-  d |= static_cast<uint32_t>(kRows >> 4) << 24;   // m_dim
-  return d;
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 __global__ void __launch_bounds__(kTcThreads, 1)
 ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_constant__ CUtensorMap map_o_lo,
                    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
@@ -119,16 +50,15 @@ ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_co
 
   if (tid == 0) {
     for (int i = 0; i < 5; ++i) mbar_init(s32(&bars[i]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == 0) {  // one warp allocates the accumulator columns in tensor memory
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&tmem_base_s)), "r"(a.tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(s32(&tmem_base_s), a.tmem_cols);
+    tmem_relinquish();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_acc = tmem_base_s;
 
   if (tid == 0) {  // ---- TMA producer + MMA issuer (one thread) ----------------------------------------------
@@ -142,13 +72,13 @@ ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_co
       tma_load_2d(base + 2 * a_tile, &map_w_hi, kc * kChunk, 0, full);
       tma_load_2d(base + 2 * a_tile + b_tile, &map_w_lo, kc * kChunk, 0, full);
     };
-    const uint32_t idesc = umma_idesc_bf16(a.c_out);
+    const uint32_t idesc = umma_idesc_bf16(kRows, a.c_out);
     load_chunk(0);
     load_chunk(1);
     for (int kc = 0; kc < kNumChunks; ++kc) {
       const int s = kc & 1;
       mbar_wait(s32(&bars[s]), (kc >> 1) & 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const uint32_t base = smem0 + s * stage_bytes;
       const uint64_t d_ohi = umma_desc_k_sw128(base), d_olo = umma_desc_k_sw128(base + a_tile);
       const uint64_t d_whi = umma_desc_k_sw128(base + 2 * a_tile), d_wlo = umma_desc_k_sw128(base + 2 * a_tile + b_tile);
@@ -170,7 +100,7 @@ ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_co
 
   // ---- epilogue: every warp owns 32 accumulator lanes = 32 pixel rows ------------------------------------
   mbar_wait(s32(&bars[4]), 0);
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   float* ys = reinterpret_cast<float*>(smem_al);  // the operand ring is free now: [128 rows][c_out + 1]
   const int pitch = a.c_out + 1;
   const int row = row0 + tid;
@@ -178,8 +108,12 @@ ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_co
   const int b = live ? row / a.hw : 0, pix = live ? row - b * a.hw : 0;
   float* yrow = ys + tid * pitch;
   for (int c0 = 0; c0 < a.c_out; c0 += 32) {
+    uint32_t r[32];
+    tmem_ld32(tmem_acc + (static_cast<uint32_t>(warp * 32) << 16) + c0, r);
+    tmem_wait_ld();
     float v[32];
-    tmem_ld32(tmem_acc + (static_cast<uint32_t>(warp * 32) << 16) + c0, v);
+#pragma unroll
+    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
     const int n = min(32, a.c_out - c0);
     for (int i = 0; i < n; ++i) {
       const int j = c0 + i;
@@ -216,18 +150,17 @@ ltae_mlp_tc_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_co
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 0)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(a.tmem_cols) : "memory");
+  if (warp == 0) tmem_dealloc(tmem_acc, a.tmem_cols);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Persistent, warp-specialised version for c_out = 64 / 128 (the shipped MLPs): one CTA per SM walks over the 128-row tiles.
 //   warp 0 (one thread)  TMA producer: the weights (hi + lo, all four K chunks) once, then the o chunks of tile after tile
 //                        into a ring of 4 (c_out = 64) or 2 (c_out = 128) stages (hi + lo, 32 KB each);
-//   warp 1 (one thread)  issues the 48 tcgen05.mma of a tile into one of TWO accumulators in tensor memory, frees ring
-//                        stages and hands accumulators over with tcgen05.commit;
+//   warp 1 (one thread)  issues the 48 products (umma_bf16) of a tile into one of TWO accumulators in tensor memory, frees
+//                        ring stages and hands accumulators over with umma_commit;
 //   warps 2-5            epilogue: 32 TMEM lanes (= pixel rows) each, 32 channels at a time entirely in registers (the
 //                        GroupNorm groups of 4 / 8 channels never straddle such a chunk): bias, BatchNorm fold, ReLU, dropout
 //                        mask, output GroupNorm, bf16 stores -- while the next tile's loads and products are under way.
@@ -263,11 +196,11 @@ ltae_mlp_tc2_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_c
     mbar_init(bar0, 1);
     for (int s = 0; s < kStages2; ++s) mbar_init(full(s), 1), mbar_init(empty(s), 1);
     for (int b = 0; b < 2; ++b) mbar_init(tfull(b), 1), mbar_init(tempty(b), 4);  // one arrival per epilogue warp
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&tmem_base_s)), "r"(2 * CO) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc(s32(&tmem_base_s), 2 * CO);
+    tmem_relinquish();
   }
   for (int i = tid; i < CO; i += kTc2Threads) {
     s_par[i] = a.bm[i];
@@ -276,9 +209,9 @@ ltae_mlp_tc2_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_c
     s_par[3 * CO + i] = a.on_w != nullptr ? a.on_w[i] : 1.f;
     s_par[4 * CO + i] = a.on_b != nullptr ? a.on_b[i] : 0.f;
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_acc = tmem_base_s;
 
   if (warp == 0) {
@@ -304,19 +237,19 @@ ltae_mlp_tc2_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_c
   } else if (warp == 1) {
     // ---- MMA issuer ---------------------------------------------------------------------------------------------------
     if (lane == 0) {
-      const uint32_t idesc = umma_idesc_bf16(CO);
+      const uint32_t idesc = umma_idesc_bf16(kRows, CO);
       mbar_wait(bar0, 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       uint32_t g = 0, it = 0;
       for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
         const uint32_t buf = it & 1u;
         if (it >= 2) mbar_wait(tempty(buf), ((it >> 1) - 1u) & 1u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const uint32_t d_tmem = tmem_acc + buf * CO;
         for (int kc = 0; kc < kNumChunks; ++kc, ++g) {
           const uint32_t s = g % kStages2;
           mbar_wait(full(s), (g / kStages2) & 1u);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const uint32_t base = ring + s * 2 * A_TILE;
           const uint64_t d_ohi = umma_desc_k_sw128(base), d_olo = umma_desc_k_sw128(base + A_TILE);
           const uint64_t d_whi = umma_desc_k_sw128(w_base + (2 * kc) * B_TILE), d_wlo = umma_desc_k_sw128(w_base + (2 * kc + 1) * B_TILE);
@@ -342,15 +275,19 @@ ltae_mlp_tc2_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_c
       const bool live = row < a.n_rows;
       const int b = live ? row / a.hw : 0, pix = live ? row - b * a.hw : 0;
       mbar_wait(tfull(buf), (it >> 1) & 1u);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
 #pragma unroll 1
       for (int c0 = 0; c0 < CO; c0 += 32) {
+        uint32_t r[32];
+        tmem_ld32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + buf * CO + c0, r);
+        tmem_wait_ld();
         float v[32];
-        tmem_ld32(tmem_acc + (static_cast<uint32_t>(q * 32) << 16) + buf * CO + c0, v);
+#pragma unroll
+        for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
         if (c0 + 32 >= CO) {  // the accumulator is in registers: the tile after next may overwrite it
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          tc_fence_before();
           __syncwarp();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty(buf)) : "memory");
+          if (lane == 0) mbar_arrive(tempty(buf));
         }
 #pragma unroll
         for (int i = 0; i < 32; ++i) v[i] += s_par[c0 + i];
@@ -392,10 +329,9 @@ ltae_mlp_tc2_kernel(const __grid_constant__ CUtensorMap map_o_hi, const __grid_c
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 0)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(2 * CO) : "memory");
+  if (warp == 0) tmem_dealloc(tmem_acc, 2 * CO);
 }
 
 // W[rows][cols] fp32 -> bf16 hi and lo planes, same row-major layout
@@ -409,41 +345,13 @@ __global__ void split_rows_kernel(const float* __restrict__ w, __nv_bfloat16* __
   lo[i] = __float2bfloat16_rn(v - __bfloat162float(h));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn == nullptr) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 // [rows][256] bf16 row-major -> boxes of box_rows x 64 elements, 128-byte swizzle, out-of-range rows read as zero
-int make_map(CUtensorMap* map, const void* base, uint64_t rows, uint32_t box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  if (fn == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return C2S_ERR_CUDA;
-  }
+int make_map(CUtensorMap* map, const void* base, uint64_t rows, uint32_t box_rows, const char* what) {
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(kK), rows};
   const cuuint64_t strides[1] = {static_cast<cuuint64_t>(kK) * 2};
   const cuuint32_t box[2] = {static_cast<cuuint32_t>(kChunk), box_rows};
-  const cuuint32_t estr[2] = {1, 1};
-  const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d", static_cast<int>(r));
-    return C2S_ERR_CUDA;
-  }
-  return C2S_OK;
+  return encode_tensor_map(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, what);
 }
 
 }  // namespace
@@ -477,10 +385,10 @@ int ltae_mlp_tc_forward(const c2s_ltae_desc& d, const c2s_ltae_params& p, float*
     C2S_LAUNCH_CHECK("ltae_split_mlp_weight");
   }
   CUtensorMap m_ohi, m_olo, m_whi, m_wlo;
-  int status = make_map(&m_ohi, o_hi, rows, kRows);
-  if (status == C2S_OK) status = make_map(&m_olo, o_lo, rows, kRows);
-  if (status == C2S_OK) status = make_map(&m_whi, w_hi, d.c_out, d.c_out);
-  if (status == C2S_OK) status = make_map(&m_wlo, w_lo, d.c_out, d.c_out);
+  int status = make_map(&m_ohi, o_hi, rows, kRows, "MLP rows hi");
+  if (status == C2S_OK) status = make_map(&m_olo, o_lo, rows, kRows, "MLP rows lo");
+  if (status == C2S_OK) status = make_map(&m_whi, w_hi, d.c_out, d.c_out, "MLP weight hi");
+  if (status == C2S_OK) status = make_map(&m_wlo, w_lo, d.c_out, d.c_out, "MLP weight lo");
   if (status != C2S_OK) return status;
   MlpArgs a{};
   a.bm = p.mlp_bias, a.bnf = bnf, a.on_w = p.out_norm_weight, a.on_b = p.out_norm_bias;
@@ -490,8 +398,7 @@ int ltae_mlp_tc_forward(const c2s_ltae_desc& d, const c2s_ltae_params& p, float*
   a.tmem_cols = d.c_out <= 32 ? 32 : (d.c_out <= 64 ? 64 : (d.c_out <= 128 ? 128 : 256));
   if (d.c_out == 64 || d.c_out == 128) {  // persistent, warp-specialised kernel
     const int n_tiles = ceil_div(rows, kRows);
-    int sms = 148, dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
     const int grid = n_tiles < sms ? n_tiles : sms;
     const size_t smem2 = static_cast<size_t>(kNumChunks) * 2 * d.c_out * kChunk * 2 + static_cast<size_t>(tc2_stages(d.c_out)) * 2 * kRows * kChunk * 2 + 1024;
     if (d.c_out == 64) {

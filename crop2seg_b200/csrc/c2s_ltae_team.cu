@@ -153,7 +153,7 @@ ltae_team_kernel(const __grid_constant__ CUtensorMap map16, const __grid_constan
   if (ttid == 0) {
     for (int i = 0; i < 4; ++i) mbar_init(bars + 8 * i, 1);
     *s_cnt = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   for (int i = ttid; i < S::kSlab / 16; i += TT) reinterpret_cast<uint4*>(slab_ptr)[i] = make_uint4(0, 0, 0, 0);  // never NaN
   for (int i = ttid; i < 2 * 16 * kPeRow / 2; i += TT) reinterpret_cast<uint32_t*>(s_pe_hi)[i] = 0u;  // hi and lo tables
@@ -170,7 +170,7 @@ ltae_team_kernel(const __grid_constant__ CUtensorMap map16, const __grid_constan
   }
   const float inv_sc = __ldg(a.wscale + 1);
   const float inv_n_all = 1.f / (static_cast<float>(a.T) * CPG);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic zero fill above, bulk-copy writes below
+  fence_proxy_async();  // generic zero fill above, bulk-copy writes below
   __syncthreads();
 
   // one warp issues the boxes of a tile: lanes 0..15 = quads of frames, boxes of 16 / 4 / 1 frames by the live mask
@@ -607,7 +607,7 @@ ltae_team_kernel(const __grid_constant__ CUtensorMap map16, const __grid_constan
       old = __shfl_sync(0xffffffffu, old, 0);
       if (old == TW - 1) {
         if (lane == 0) *s_cnt = 0;
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         if (nxt < a.n_tiles) issue_tile(nxt, nlive);
       }
     }
@@ -760,8 +760,7 @@ int team_launch(const CUtensorMap& map16, const CUtensorMap& map4, const CUtenso
                 cudaStream_t stream, const char* name) {
   using S = TeamSmem<C>;
   C2S_SMEM_ATTR((ltae_team_kernel<C, DROP>), S::kTotal);
-  int sms = 148, dev = 0;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int sms = sm_count();
   const int teams = (a.n_tiles + S::TEAMS - 1) / S::TEAMS;
   const int grid = teams < sms ? teams : sms;
   ltae_team_kernel<C, DROP><<<static_cast<unsigned>(grid), 512, S::kTotal, stream>>>(map16, map4, map1, a);
