@@ -19,7 +19,7 @@
 """
 from __future__ import annotations
 
-from typing import Dict, Optional
+from typing import Dict
 
 import torch
 import torch.nn.functional as F
@@ -31,44 +31,39 @@ class AggregateFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, attn, pad_mask, mode):
         ctx.mode = mode
-        ctx.save_for_backward(x, attn if attn is not None else torch.empty(0, device=x.device),
-                              pad_mask if pad_mask is not None else torch.empty(0, device=x.device))
-        ctx.has_attn, ctx.has_pad = attn is not None, pad_mask is not None
+        ctx.save_for_backward(x, attn, pad_mask)
         return ops.temporal_aggregate_forward(x, pad_mask, attn, mode)
 
     @staticmethod
     def backward(ctx, grad_out):
         x, attn, pad = ctx.saved_tensors
-        attn = attn if ctx.has_attn else None
-        pad = pad if ctx.has_pad else None
-        need_x = ctx.needs_input_grad[0]
-        need_attn = ctx.has_attn and ctx.needs_input_grad[1]
-        gx, gattn = ops.temporal_aggregate_backward(x, pad, attn, grad_out, ctx.mode, need_x=need_x, need_attn=need_attn)
+        gx, gattn = ops.temporal_aggregate_backward(x, pad, attn, grad_out, ctx.mode, need_x=ctx.needs_input_grad[0],
+                                                    need_attn=ctx.needs_input_grad[1])
         return gx, gattn, None, None
 
 
 # ------------------------------------------------------------------------------------------------------------
 # positional table [B,T,D] on the device: stage F needs it (and its autograd graph for learnable tables)
 # ------------------------------------------------------------------------------------------------------------
-def _positional(cfg: Dict, P: Dict[str, torch.Tensor], positions: torch.Tensor, n_rows_per_sample: int):
+def _positional(spec: ops.LtaeSpec, P: Dict[str, torch.Tensor], positions: torch.Tensor):
     """[B,T,D] positional table (identical for every pixel of a sample; positional_encoding.py:25-73)."""
-    h, d = cfg["n_head"], cfg["d_model"] // cfg["n_head"]
+    h, d = spec.n_head, spec.d_model // spec.n_head
 
     def doy(pos, w, b):
         idx = pos.to(torch.int64).clamp(0, 364)
         return (w.t()[idx] + b).repeat(1, 1, h)
 
     def primary(pos):
-        if cfg["pe_mode"] == _lib.PE_DOY_TABLE:
+        if spec.pe_mode == _lib.PE_DOY_TABLE:
             return doy(pos, P["pe_fc_weight"], P["pe_fc_bias"])
         table = pos.to(torch.float32)[:, :, None] / P["pe_denom"][None, None, :]
         enc = torch.where((torch.arange(d, device=table.device) % 2 == 0)[None, None, :], torch.sin(table), torch.cos(table))
         enc = enc.repeat(1, 1, h)
-        if cfg["pe_mode"] == _lib.PE_SINUSOID_LINEAR:
+        if spec.pe_mode == _lib.PE_SINUSOID_LINEAR:
             enc = F.linear(enc, P["pe_fc_weight"], P["pe_fc_bias"])
         return enc
 
-    if cfg["pe_abs"]:
+    if spec.pe_abs:
         return primary(positions[..., 0]) + doy(positions[..., 1], P["pe_abs_fc_weight"], P["pe_abs_fc_bias"])
     return primary(positions)
 
@@ -76,30 +71,12 @@ def _positional(cfg: Dict, P: Dict[str, torch.Tensor], positions: torch.Tensor, 
 _GRAD_PARAM_ORDER = tuple(_lib.LTAE_PARAM_FIELDS)
 
 
-def _folded(cfg: Dict, P: Dict[str, Optional[torch.Tensor]], positions, b: int, t: int):
-    """Differentiable restatement of the weight folding of ``csrc/c2s_ltae_prep.cu`` (stage F of the backward):
-    returns ``U[C,h]``, ``cpos[B,T,h]`` and the positional table ``pe[B,T,D] | None``."""
-    h, dk, D = cfg["n_head"], cfg["d_k"], cfg["d_model"]
-    wc = P["inconv_weight"].reshape(D, -1)
-    qk = torch.einsum("hj,hjd->hd", P["query"].reshape(h, dk), P["key_weight"].reshape(h, dk, D)) / (dk ** 0.5)
-    U = (qk @ wc).t() * P["in_norm_weight"][:, None]
-    wb = P["inconv_bias"] + wc @ P["in_norm_bias"]
-    ub = qk @ wb + (P["query"].reshape(h, dk) * P["key_bias"].reshape(h, dk)).sum(1) / (dk ** 0.5)
-    pe = None
-    cpos = ub[None, None, :].expand(b, t, h)
-    if cfg["pe_mode"] != _lib.PE_NONE:
-        pe = _positional(cfg, P, positions, 0)
-        cpos = cpos + pe @ qk.t()
-    return U, cpos, pe
-
-
-def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params, g_out, g_attn):
+def _cuda_backward(ctx, spec, x, positions, pad_mask, attn_keep, mlp_keep, params, g_out, g_attn):
     b, t, c, hh, ww = x.shape
-    n, h, D = b * hh * ww, cfg["n_head"], cfg["d_model"]
-    dh = D // h
+    n, h, D = b * hh * ww, spec.n_head, spec.d_model
     need = dict(zip(_GRAD_PARAM_ORDER, ctx.needs_input_grad[6:]))
     raw = dict(zip(_GRAD_PARAM_ORDER, params))
-    attn_only = cfg["attn_only"]
+    attn_only = spec.attn_only
     grads: Dict[str, torch.Tensor] = {}
 
     # ---- stage M: rows after the attention (c2s_ltae_mlp_backward) ---------------------------------------------
@@ -108,17 +85,15 @@ def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params
         if g_out is None:
             g_o = torch.zeros((n, D), dtype=torch.float32, device=x.device)
         else:
-            if cfg["c_out"] // h > 16:
+            if spec.c_out // h > 16:
                 raise _lib.C2SError(f"crop2seg_b200: L-TAE backward supports out_norm groups of at most 16 channels "
-                                    f"(mlp[-1]={cfg['c_out']}, n_head={h}); there is no torch fallback")
-            if cfg["bn_batch_stats"]:
+                                    f"(mlp[-1]={spec.c_out}, n_head={h}); there is no torch fallback")
+            if spec.bn_batch_stats:
                 mean, var = ctx.bn_stats
             else:
                 mean, var = raw["bn_running_mean"], raw["bn_running_var"]
-            m_res = ops.ltae_mlp_backward(
-                ctx.o_rows, g_out.to(x.dtype), raw, mean, var, n_head=h, d_model=D, c_out=cfg["c_out"],
-                bn_batch_stats=cfg["bn_batch_stats"], gn_eps=cfg["gn_eps"], bn_eps=cfg["bn_eps"], mlp_keep=mlp_keep,
-                mlp_drop_p=1.0 - 1.0 / cfg["mlp_keep_scale"], y_rows=ctx.y_rows)
+            m_res = ops.ltae_mlp_backward(ctx.o_rows, g_out.to(x.dtype), raw, mean, var, spec, mlp_keep=mlp_keep,
+                                          y_rows=ctx.y_rows)
             g_o = m_res["grad_o"]
             for k in ("mlp_weight", "mlp_bias", "bn_weight", "bn_bias", "out_norm_weight", "out_norm_bias"):
                 if need[k]:
@@ -130,11 +105,8 @@ def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params
         gparams = [torch.zeros_like(p) if (p is not None and need[k]) else None for k, p in zip(_GRAD_PARAM_ORDER, params)]
         return (gx, None, None, None, None, None, *gparams)
     pe_learnable = any(need.get(k) for k in ("pe_fc_weight", "pe_fc_bias", "pe_abs_fc_weight", "pe_abs_fc_bias"))
-    res = ops.ltae_backward(
-        x, positions, pad_mask, raw, g_o, g_attn, n_head=h, d_k=cfg["d_k"], d_model=D, has_inconv=True,
-        c_out=cfg["c_out"], pe_mode=cfg["pe_mode"], pe_abs=cfg["pe_abs"], attn_only=attn_only,
-        zero_padded=cfg["zero_padded"], gn_eps=cfg["gn_eps"], attn_keep=attn_keep,
-        attn_drop_p=1.0 - 1.0 / cfg["attn_keep_scale"], need_grad_pe=pe_learnable)
+    res = ops.ltae_backward(x, positions, pad_mask, raw, g_o, g_attn, spec, attn_keep=attn_keep,
+                            need_grad_pe=pe_learnable)
 
     # ---- stage F: folded quantities -> state_dict tensors (the adjoint of csrc/c2s_ltae_prep.cu, written out) -----
     front = ("in_norm_weight", "in_norm_bias", "inconv_weight", "inconv_bias", "query", "key_weight", "key_bias",
@@ -145,7 +117,7 @@ def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params
             # c2s_ltae_inconv_grad (one launch over the rows)
             want = {k: bool(need.get(k)) for k in front[:7]}
             shapes = {k: tuple(raw[k].shape) for k in front[:7] if raw.get(k) is not None}
-            pe_learnable_now = pe_learnable and cfg["pe_mode"] != _lib.PE_NONE
+            pe_learnable_now = pe_learnable and spec.pe_mode != _lib.PE_NONE
             if pe_learnable_now and res["grad_pe"] is None:  # attention-only encoders: the table acts through the scores only
                 res["grad_pe"] = torch.zeros((b, t, D), dtype=torch.float32, device=x.device)
             folded = ops.ltae_fold_backward(res, want, shapes, grad_pe_through_scores=pe_learnable_now)
@@ -162,7 +134,7 @@ def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params
             with torch.enable_grad():
                 L = {k: (v.detach().float().requires_grad_(k in pe_names) if v is not None and v.is_floating_point() else v)
                      for k, v in raw.items()}
-                got = torch.autograd.grad(_positional(cfg, L, positions, 0), [L[k] for k in pe_names], g_pe,
+                got = torch.autograd.grad(_positional(spec, L, positions), [L[k] for k in pe_names], g_pe,
                                           allow_unused=True)
             for k, gk in zip(pe_names, got):
                 if gk is not None:
@@ -176,31 +148,23 @@ def _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params
 
 
 class LtaeFunction(torch.autograd.Function):
-    """apply(x, positions, pad_mask, attn_keep, mlp_keep, cfg, *params in LTAE_PARAM_FIELDS order)
+    """apply(x, positions, pad_mask, attn_keep, mlp_keep, spec, *params in LTAE_PARAM_FIELDS order)
     -> (out | None, attn, bn_batch_mean | None, bn_batch_var | None)"""
 
     @staticmethod
-    def forward(ctx, x, positions, pad_mask, attn_keep, mlp_keep, cfg, *params):
+    def forward(ctx, x, positions, pad_mask, attn_keep, mlp_keep, spec, *params):
         P = dict(zip(_GRAD_PARAM_ORDER, params))
         # d_model=None (tae.py:398-403: no inconv) is served in the forward only; the reference's shipped models always
         # build the in-projection (utae.py:179-189, wtae.py:196-207, timeunet.py:155-164).  backward() raises for it.
-        ctx.cuda_backward = bool(cfg["has_inconv"])
-        res = ops.ltae_forward(
-            x, positions, pad_mask, P, n_head=cfg["n_head"], d_k=cfg["d_k"], d_model=cfg["d_model"],
-            has_inconv=cfg["has_inconv"], c_out=cfg["c_out"], pe_mode=cfg["pe_mode"], pe_abs=cfg["pe_abs"],
-            attn_only=cfg["attn_only"], need_attn=True, zero_padded=cfg["zero_padded"],
-            bn_batch_stats=cfg["bn_batch_stats"], gn_eps=cfg["gn_eps"], bn_eps=cfg["bn_eps"],
-            attn_keep=attn_keep, attn_drop_p=1.0 - 1.0 / cfg["attn_keep_scale"],
-            mlp_keep=mlp_keep, mlp_drop_p=1.0 - 1.0 / cfg["mlp_keep_scale"],
-            save_o=ctx.cuda_backward and not cfg["attn_only"],
-            save_y=ctx.cuda_backward and not cfg["attn_only"] and cfg["bn_batch_stats"])
-        out, attn, stats = res[:3]
-        ctx.o_rows = res[3] if len(res) > 3 else None
-        ctx.y_rows = res[4] if len(res) > 4 else None  # pre-BatchNorm rows (training mode): the backward does not recompute them
-        ctx.cfg = cfg
+        ctx.cuda_backward = bool(spec.has_inconv)
+        # with save_y the pre-BatchNorm rows of a training-mode forward are kept: the backward does not recompute them
+        out, attn, stats, ctx.o_rows, ctx.y_rows = ops.ltae_forward(
+            x, positions, pad_mask, P, spec, attn_keep=attn_keep, mlp_keep=mlp_keep, save_o=ctx.cuda_backward,
+            save_y=ctx.cuda_backward)
+        ctx.spec = spec
         # the running statistics are updated in place right after a training-mode forward and are not needed by
         # its backward (batch statistics are recomputed), so they are not saved in that case
-        skip = ("bn_running_mean", "bn_running_var") if cfg["bn_batch_stats"] else ()
+        skip = ("bn_running_mean", "bn_running_var") if spec.bn_batch_stats else ()
         params = [None if name in skip else p for name, p in zip(_GRAD_PARAM_ORDER, params)]
         ctx.present = [p is not None for p in params]
         ctx.opt = (positions, pad_mask, attn_keep, mlp_keep)
@@ -213,7 +177,6 @@ class LtaeFunction(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, *grads):
-        cfg = ctx.cfg
         saved = ctx.saved_tensors
         x, rest = saved[0], list(saved[1:])
         positions, pad_mask, attn_keep, mlp_keep = ctx.opt
@@ -222,4 +185,4 @@ class LtaeFunction(torch.autograd.Function):
         if not ctx.cuda_backward:
             raise _lib.C2SError("crop2seg_b200: the L-TAE backward needs the in-projection (d_model is not None); "
                                 "there is no torch fallback for encoders without inconv")
-        return _cuda_backward(ctx, cfg, x, positions, pad_mask, attn_keep, mlp_keep, params, g_out, g_attn)
+        return _cuda_backward(ctx, ctx.spec, x, positions, pad_mask, attn_keep, mlp_keep, params, g_out, g_attn)

@@ -15,6 +15,7 @@ All arithmetic runs in the CUDA library (``ops.py``); there is no fallback.
 from __future__ import annotations
 
 import copy
+import dataclasses
 from typing import List, Optional
 
 import numpy as np
@@ -149,7 +150,7 @@ class _LTAEBase(nn.Module):
         #: False and ``forward`` then skips the [n_head,B,T,H,W] store and returns ``(out, None)``
         self.return_attention = _DEFAULTS["return_attention"]
         #: eval mode keeps the folded weights between calls while no parameter changes (``Tensor._version`` and
-        #: ``data_ptr`` of every parameter / buffer); writes through ``.data`` bypass the version counters -- call
+        #: ``data_ptr`` of every tensor the kernels read); writes through ``.data`` bypass the version counters -- call
         #: ``invalidate_folded_weights()`` after those, or set this to False
         self.cache_folded_weights = True
         self._folded_cache = {}
@@ -167,12 +168,12 @@ class _LTAEBase(nn.Module):
         self._folded_cache.clear()
         return super()._load_from_state_dict(*args, **kwargs)
 
-    def _folded_args(self):
-        """kwargs for ops.ltae_forward: reuse of the weight-only preparation in eval mode."""
+    def _folded_args(self, params):
+        """kwargs for ops.ltae_forward: reuse of the weight-only preparation in eval mode, keyed on the tensors of
+        ``params`` (the ones the kernels read)."""
         if self.training or not self.cache_folded_weights:
             return {}
-        tensors = list(self.parameters()) + list(self.buffers())
-        key = tuple((t._version, t.data_ptr()) for t in tensors)
+        key = tuple((t._version, t.data_ptr()) for t in params.values() if t is not None)
         return {"folded_cache": self._folded_cache, "folded_key": key}
 
     # -- helpers ---------------------------------------------------------------------------------
@@ -184,7 +185,23 @@ class _LTAEBase(nn.Module):
             return _lib.PE_DOY_TABLE
         return _lib.PE_SINUSOID_LINEAR if pe.add_linear else _lib.PE_SINUSOID
 
-    def _front_params(self, device):
+    def _needs_grad(self, x) -> bool:
+        return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters()))
+
+    def _spec(self) -> ops.LtaeSpec:
+        """The encoder's configuration for one forward; training mode selects BatchNorm batch statistics and dropout."""
+        mlp = {}
+        if isinstance(self, LTAE):
+            bn = self.mlp[2]
+            mlp = dict(c_out=self._widths[-1], bn_batch_stats=self.training or not bn.track_running_stats,
+                       bn_eps=bn.eps, mlp_drop_p=float(self.mlp[5].p) if self.training else 0.0)
+        return ops.LtaeSpec(n_head=self.n_head, d_k=self.d_k, d_model=self.d_model, has_inconv=self.inconv is not None,
+                            pe_mode=self._pe_mode(), pe_abs=bool(self.use_abs_rel_enc),
+                            attn_only=not isinstance(self, LTAE), zero_padded=bool(self.assume_zero_padded),
+                            gn_eps=self.in_norm.eps, attn_drop_p=ATTENTION_DROPOUT if self.training else 0.0, **mlp)
+
+    def _params(self, device):
+        """The tensors of ``c2s_ltae_params``, keyed by its field names (the MLP, BatchNorm and out_norm ones for LTAE)."""
         p = {
             "in_norm_weight": self.in_norm.weight, "in_norm_bias": self.in_norm.bias,
             "query": self.attention_head.Q, "key_weight": self.attention_head.fc1_k.weight,
@@ -206,14 +223,14 @@ class _LTAEBase(nn.Module):
             if self.use_abs_rel_enc:
                 p["pe_abs_fc_weight"] = self.positional_encoder_abs.fc.weight
                 p["pe_abs_fc_bias"] = self.positional_encoder_abs.fc.bias
+        if isinstance(self, LTAE):
+            lin, bn = self.mlp[0], self.mlp[2]
+            p.update({
+                "mlp_weight": lin.weight, "mlp_bias": lin.bias, "bn_weight": bn.weight, "bn_bias": bn.bias,
+                "bn_running_mean": bn.running_mean, "bn_running_var": bn.running_var,
+                "out_norm_weight": self.out_norm.weight, "out_norm_bias": self.out_norm.bias,
+            })
         return p
-
-    def _cfg(self, c_out, attn_only, bn_batch_stats, attn_p, mlp_p, bn_eps=1e-5):
-        return {"n_head": self.n_head, "d_k": self.d_k, "d_model": self.d_model, "has_inconv": self.inconv is not None,
-                "c_out": c_out, "pe_mode": self._pe_mode(), "pe_abs": bool(self.use_abs_rel_enc), "attn_only": attn_only,
-                "zero_padded": bool(self.assume_zero_padded), "bn_batch_stats": bool(bn_batch_stats),
-                "gn_eps": self.in_norm.eps, "bn_eps": bn_eps, "attn_keep_scale": 1.0 / (1.0 - attn_p),
-                "mlp_keep_scale": 1.0 / (1.0 - mlp_p)}
 
     def _check_inputs(self, x, batch_positions):
         if self.num_queries != 1 and (self.training or not isinstance(self, LTAE)):
@@ -290,60 +307,35 @@ class LTAE(_LTAEBase):
         if not bn.track_running_stats:
             raise NotImplementedError("crop2seg_b200: num_queries > 1 needs BatchNorm running statistics")
         b, t, _, h, w = x.shape
-        c_out = self._widths[-1]
-        params = self._front_params(x.device)
-        params.update({
-            "mlp_weight": self.mlp[0].weight, "mlp_bias": self.mlp[0].bias, "bn_weight": bn.weight, "bn_bias": bn.bias,
-            "bn_running_mean": bn.running_mean, "bn_running_var": bn.running_var,
-            "out_norm_weight": self.out_norm.weight, "out_norm_bias": self.out_norm.bias,
-        })
+        spec = self._spec()
+        params = self._params(x.device)
         rows, attns = [], []
         for i in range(self.num_queries):
             params["query"] = self.attention_head.Q[:, i:i + 1, :]  # Q[n_head, n, d_k] -> the rows of one query
-            _, attn, _, o_rows = ops.ltae_forward(
-                x, batch_positions, pad_mask, params, n_head=self.n_head, d_k=self.d_k, d_model=self.d_model,
-                has_inconv=self.inconv is not None, c_out=c_out, pe_mode=self._pe_mode(), pe_abs=self.use_abs_rel_enc,
-                need_attn=return_att, zero_padded=self.assume_zero_padded, bn_batch_stats=False,
-                gn_eps=self.in_norm.eps, bn_eps=bn.eps, save_o=True)
-            rows.append(o_rows)
-            attns.append(attn)
-        out = ops.ltae_rows_forward(torch.stack(rows), params, batch=b, height=h, width=w, n_head=self.n_head,
-                                    d_model=self.d_model, c_out=c_out, dtype=x.dtype, gn_eps=self.out_norm.eps, bn_eps=bn.eps)
+            res = ops.ltae_forward(x, batch_positions, pad_mask, params, spec, need_attn=return_att, save_o=True)
+            rows.append(res.o_rows)
+            attns.append(res.attn)
+        # the row kernel applies out_norm alone, with out_norm's own eps
+        out = ops.ltae_rows_forward(torch.stack(rows), params, dataclasses.replace(spec, gn_eps=self.out_norm.eps),
+                                    batch=b, height=h, width=w, dtype=x.dtype)
         return out, (torch.stack(attns, dim=2) if return_att else None)
 
     def _forward_one(self, x, batch_positions, pad_mask, return_att):
-        bn = self.mlp[2]
-        train_bn = self.training or not bn.track_running_stats
-        params = self._front_params(x.device)
-        params.update({
-            "mlp_weight": self.mlp[0].weight, "mlp_bias": self.mlp[0].bias,
-            "bn_weight": bn.weight, "bn_bias": bn.bias,
-            "bn_running_mean": bn.running_mean, "bn_running_var": bn.running_var,
-            "out_norm_weight": self.out_norm.weight, "out_norm_bias": self.out_norm.bias,
-        })
+        spec = self._spec()
+        params = self._params(x.device)
         b, t, _, h, w = x.shape
-        c_out = self._widths[-1]
-        attn_p = ATTENTION_DROPOUT if self.training else 0.0
-        mlp_p = float(self.mlp[5].p) if self.training else 0.0
-        attn_keep = _draw_keep((self.n_head, b, t, h, w), attn_p, x.device, 0)
-        mlp_keep = _draw_keep((b, c_out, h, w), mlp_p, x.device, 1)
-        needs_grad = torch.is_grad_enabled() and (
-            x.requires_grad or any(p.requires_grad for p in self.parameters()))
-        if needs_grad:
+        attn_keep = _draw_keep((self.n_head, b, t, h, w), spec.attn_drop_p, x.device, 0)
+        mlp_keep = _draw_keep((b, spec.c_out, h, w), spec.mlp_drop_p, x.device, 1)
+        if self._needs_grad(x):
             from .autograd import LtaeFunction
-            cfg = self._cfg(c_out, attn_only=False, bn_batch_stats=train_bn, attn_p=attn_p, mlp_p=mlp_p, bn_eps=bn.eps)
-            out, attn, mean, var = LtaeFunction.apply(x, batch_positions, pad_mask, attn_keep, mlp_keep, cfg,
+            out, attn, mean, var = LtaeFunction.apply(x, batch_positions, pad_mask, attn_keep, mlp_keep, spec,
                                                       *[params.get(k) for k in _lib.LTAE_PARAM_FIELDS])
             stats = (mean, var) if mean is not None else None
         else:
-            out, attn, stats = ops.ltae_forward(
-                x, batch_positions, pad_mask, params, n_head=self.n_head, d_k=self.d_k, d_model=self.d_model,
-                has_inconv=self.inconv is not None, c_out=c_out, pe_mode=self._pe_mode(),
-                pe_abs=self.use_abs_rel_enc, need_attn=return_att, zero_padded=self.assume_zero_padded,
-                bn_batch_stats=train_bn, gn_eps=self.in_norm.eps, bn_eps=bn.eps, attn_keep=attn_keep,
-                attn_drop_p=attn_p, mlp_keep=mlp_keep, mlp_drop_p=mlp_p, **self._folded_args())
-        if stats is not None and self.training and bn.track_running_stats:
-            self._update_running_stats(bn, stats, b * h * w)
+            out, attn, stats = ops.ltae_forward(x, batch_positions, pad_mask, params, spec, need_attn=return_att,
+                                                attn_keep=attn_keep, mlp_keep=mlp_keep, **self._folded_args(params))[:3]
+        if stats is not None and self.training and self.mlp[2].track_running_stats:
+            self._update_running_stats(self.mlp[2], stats, b * h * w)
         return out, (attn if return_att else None)
 
     @staticmethod
@@ -370,24 +362,16 @@ class LTAE4WTAE(_LTAEBase):
     def forward(self, x, batch_positions=None, pad_mask=None, return_comp=False):
         """x[B,T,C,H,W] -> attn[n_head,B,T,H,W] (tae.py:589-635); dropout on the attention in training mode."""
         self._check_inputs(x, batch_positions)
+        spec = self._spec()
         b, t, _, h, w = x.shape
-        attn_p = ATTENTION_DROPOUT if self.training else 0.0
-        attn_keep = _draw_keep((self.n_head, b, t, h, w), attn_p, x.device, 0)
-        params = self._front_params(x.device)
-        needs_grad = torch.is_grad_enabled() and (
-            x.requires_grad or any(p.requires_grad for p in self.parameters()))
-        if needs_grad:
+        attn_keep = _draw_keep((self.n_head, b, t, h, w), spec.attn_drop_p, x.device, 0)
+        params = self._params(x.device)
+        if self._needs_grad(x):
             from .autograd import LtaeFunction
-            cfg = self._cfg(0, attn_only=True, bn_batch_stats=False, attn_p=attn_p, mlp_p=0.0)
-            _, attn, _, _ = LtaeFunction.apply(x, batch_positions, pad_mask, attn_keep, None, cfg,
-                                               *[params.get(k) for k in _lib.LTAE_PARAM_FIELDS])
-            return attn
-        _, attn, _ = ops.ltae_forward(
-            x, batch_positions, pad_mask, params, n_head=self.n_head, d_k=self.d_k,
-            d_model=self.d_model, has_inconv=self.inconv is not None, c_out=0, pe_mode=self._pe_mode(),
-            pe_abs=self.use_abs_rel_enc, attn_only=True, zero_padded=self.assume_zero_padded,
-            gn_eps=self.in_norm.eps, attn_keep=attn_keep, attn_drop_p=attn_p, **self._folded_args())
-        return attn
+            return LtaeFunction.apply(x, batch_positions, pad_mask, attn_keep, None, spec,
+                                      *[params.get(k) for k in _lib.LTAE_PARAM_FIELDS])[1]
+        return ops.ltae_forward(x, batch_positions, pad_mask, params, spec, attn_keep=attn_keep,
+                                **self._folded_args(params)).attn
 
 
 class TemporalAggregator(nn.Module):

@@ -77,7 +77,7 @@ def _ltae(kw, seed, kind="ltae"):
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_ltae_train_mode_forward_with_injected_dropout(dtype):
+def test_ltae_train_mode_forward_from_a_spec_with_injected_dropout(dtype):
     """BatchNorm batch statistics + dropout masks on the attention and after the ReLU (tae.py:445-448, :837)."""
     kw = dict(in_channels=128, n_head=16, d_k=4, mlp=[256, 128], d_model=256)
     m, rng = _ltae(kw, 31)
@@ -91,15 +91,11 @@ def test_ltae_train_mode_forward_with_injected_dropout(dtype):
         oracle_config("ltae", kw), oracle_params(m), xr, pos, pad, training=True,
         attn_keep=np.ascontiguousarray(attn_keep.transpose(0, 1, 3, 4, 2)).reshape(16, n, 1, t),
         mlp_keep=np.ascontiguousarray(mlp_keep.transpose(0, 2, 3, 1)).reshape(n, 128))
-    params = m._front_params(torch.device("cuda"))
-    bn = m.mlp[2]
-    params.update({"mlp_weight": m.mlp[0].weight, "mlp_bias": m.mlp[0].bias, "bn_weight": bn.weight,
-                   "bn_bias": bn.bias, "bn_running_mean": bn.running_mean, "bn_running_var": bn.running_var,
-                   "out_norm_weight": m.out_norm.weight, "out_norm_bias": m.out_norm.bias})
+    spec = ops.LtaeSpec(n_head=16, d_k=4, d_model=256, has_inconv=True, c_out=128, pe_mode=_lib.PE_SINUSOID,
+                        bn_batch_stats=True, attn_drop_p=0.1, mlp_drop_p=0.2)
     out, attn, stats = ops.ltae_forward(
-        to_dev(x, dtype=dtype), to_dev(pos), to_dev(pad), params, n_head=16, d_k=4, d_model=256, has_inconv=True,
-        c_out=128, pe_mode=_lib.PE_SINUSOID, bn_batch_stats=True, attn_keep=to_dev(attn_keep), attn_drop_p=0.1,
-        mlp_keep=to_dev(mlp_keep), mlp_drop_p=0.2)
+        to_dev(x, dtype=dtype), to_dev(pos), to_dev(pad), m._params(torch.device("cuda")), spec,
+        attn_keep=to_dev(attn_keep), mlp_keep=to_dev(mlp_keep))[:3]
     tol = 1e-4 if dtype == torch.float32 else 1e-2
     assert rel_err(attn.cpu().numpy(), ref_attn) < (1e-4 if dtype == torch.float32 else 1e-3)
     assert rel_err(out.float().cpu().numpy(), ref_out) < tol

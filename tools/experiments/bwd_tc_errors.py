@@ -19,17 +19,14 @@ def case(c_in, lengths, hw=(4, 4), keep=True, seed=3):
     go = rng.standard_normal((n, 256)).astype(np.float32)
     ga = rng.standard_normal((16, b, t, h, w)).astype(np.float32)
     ak = (rng.uniform(size=(16, b, t, h, w)) >= 0.1).astype(np.uint8) if keep else None
-    params = m._front_params(torch.device("cuda"))
-    bn = m.mlp[2]
-    params.update({"mlp_weight": m.mlp[0].weight, "mlp_bias": m.mlp[0].bias, "bn_weight": bn.weight, "bn_bias": bn.bias,
-                   "bn_running_mean": bn.running_mean, "bn_running_var": bn.running_var,
-                   "out_norm_weight": m.out_norm.weight, "out_norm_bias": m.out_norm.bias})
+    params = m._params(torch.device("cuda"))
+    spec = ops.LtaeSpec(n_head=16, d_k=4, d_model=256, has_inconv=True, c_out=64, pe_mode=m._pe_mode(), zero_padded=True,
+                        attn_drop_p=0.1 if keep else 0.0)
     out = {}
     for name, opt in (("tc", 0), ("tc2", 0), ("gen", 1)):
         with _lib.option(_lib.OPT_LTAE_BWD_KERNEL, opt):
             r = ops.ltae_backward(to_dev(x, dtype=torch.bfloat16), to_dev(pos), to_dev(pad), params, to_dev(go), to_dev(ga),
-                                  n_head=16, d_k=4, d_model=256, has_inconv=True, c_out=64, pe_mode=m._pe_mode() if hasattr(m, "_pe_mode") else _lib.PE_SINUSOID,
-                                  zero_padded=True, attn_keep=None if ak is None else to_dev(ak), attn_drop_p=0.1 if keep else 0.0)
+                                  spec, attn_keep=None if ak is None else to_dev(ak))
             torch.cuda.synchronize()
             out[name] = ({k: v.float().cpu().numpy() for k, v in r.items() if torch.is_tensor(v)}, _lib.last_kernel())
     print(f"C={c_in} lengths={lengths} hw={hw} keep={keep}: kernels {out['tc'][1]} / {out['gen'][1]}")
