@@ -28,6 +28,72 @@ def synth_inputs(rng, b, t, c, h, w, lengths, doy=False, abs_rel=False):
     return x, positions, pad
 
 
+PAD_PATTERNS = ("suffix", "lead1", "lead16", "lead17", "mid_block", "ballot_edge", "alternate", "one_last", "one_mid",
+                "sparse_random", "all_padded")
+
+
+def pad_pattern(name, t, seed=0):
+    """[T] bool pad mask (True = padded) of one named pattern.  The kernels handle the mask as a set of frames in
+    16-frame blocks, 4-frame groups and two 32-frame ballot halves; each pattern puts its holes where one of those
+    decisions changes."""
+    pad = np.zeros(t, dtype=bool)
+    if name == "suffix":
+        pad[max(1, (2 * t) // 3):] = True
+    elif name.startswith("lead"):
+        pad[:int(name[4:])] = True         # lead16: the first 16-frame block holds no live frame
+    elif name == "mid_block":
+        pad[16:32] = True                  # live frames on both sides of a dead block (T > 32)
+    elif name == "ballot_edge":
+        pad[31:33] = True                  # the last frame of the low ballot half and the first of the high one
+        if t == 64:
+            pad[32:63] = True              # only frame 63 is live in the high half
+    elif name == "alternate":
+        pad[0::2] = True                   # every 4-frame group is partial, the first live frame is frame 1
+    elif name == "one_last":
+        pad[:t - 1] = True
+    elif name == "one_mid":
+        pad[:] = True
+        pad[t // 2] = False
+    elif name == "sparse_random":
+        pad = np.random.RandomState(1000 * seed + t).uniform(size=t) < 0.4
+        if pad.all():
+            pad[t // 3] = False
+    elif name == "all_padded":
+        pad[:] = True
+    else:
+        raise KeyError(name)
+    return pad
+
+
+def pattern_masks(t, names=PAD_PATTERNS, n=None, seed=0):
+    """[B, T] bool, one row per sample.  Without ``n``: the named patterns in order.  With ``n``: sample i takes pattern
+    i mod (len(names) + 1), the extra slot being a seeded random mask of random density, so that neighbouring samples
+    never share a mask."""
+    if n is None:
+        return np.stack([pad_pattern(name, t) for name in names])
+    rng = np.random.RandomState(seed + t)
+    rows = []
+    for i in range(n):
+        k = i % (len(names) + 1)
+        rows.append(pad_pattern(names[k], t) if k < len(names) else rng.uniform(size=t) < rng.uniform(0.0, 0.9))
+    return np.stack(rows)
+
+
+def synth_inputs_masked(rng, b, t, c, h, w, masks, zero_padded):
+    """Like ``synth_inputs`` but with an explicit [B, T] pad mask.  Positions increase over every frame, so a padded frame
+    keeps a plausible date, as a hole in a real series does.  ``zero_padded``: padded frames are exactly zero; otherwise
+    they carry non-zero data, which the reference counts in the input GroupNorm but never in the attention."""
+    pad = np.asarray(masks, dtype=bool).reshape(b, t)
+    x = np.maximum(rng.standard_normal((b, t, c, h, w)).astype(np.float32), 0)
+    if zero_padded:
+        x[pad] = 0
+    else:
+        x[pad] = 0.3 * rng.standard_normal(x[pad].shape).astype(np.float32)
+    gaps = rng.randint(2, 11, size=(b, t))
+    gaps[:, 0] = rng.randint(0, 11, size=b)
+    return x, np.cumsum(gaps, axis=1).astype(np.int64), pad
+
+
 def random_attention(rng, heads, pad, ha, wa):
     b, t = pad.shape
     logits = rng.standard_normal((heads, b, t, ha, wa)).astype(np.float32)

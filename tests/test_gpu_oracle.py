@@ -145,14 +145,14 @@ def test_persistent_ltae_many_tiles(name, zero_padded):
         assert rel_err(out.float().cpu().numpy(), ref_out) < 1e-2
 
 
-def test_tensor_core_ltae_train_mode_batch_statistics():
+def test_tensor_core_ltae_train_mode_batch_statistics(monkeypatch):
     kind, kw, (b, t, h, w), lengths, _ = LTAE_CASES["utae"]
     m, rng = _build(kind, kw, 77)
     x, pos, pad = synth_inputs(rng, b, t, 128, h, w, lengths)
     params = oracle_params(m)
     m.train()
     m.mlp[5].p = 0.0
-    c2s.modules.ATTENTION_DROPOUT = 0.0
+    monkeypatch.setattr(c2s.modules, "ATTENTION_DROPOUT", 0.0)  # restored behind the test: later tests train with 0.1
     with torch.no_grad():
         out, attn = m(to_dev(x, dtype=torch.bfloat16), batch_positions=to_dev(pos), pad_mask=to_dev(pad))
     ref_out, ref_attn, (rm, rv) = ltae_forward(oracle_config(kind, kw), params, bf16_round(x), pos, pad, training=True)
