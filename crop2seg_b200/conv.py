@@ -9,12 +9,13 @@ What runs where (``forward`` / ``smart_forward``, eval mode, CUDA tensors):
 
 * frames: ``smart_forward`` packs the valid frames with the device-side frame index (no ``nonzero`` sync, no dummy
   forward; ``staging.py``), runs the block in bf16 on the packed frames and scatters the result back;
-* convolution: every layer with 64 input (or <= 16, the model input) and 64 output channels runs as a hand-written tcgen05
-  implicit GEMM (``c2s_conv2d_forward``, ``csrc/c2s_conv.cu``): the 3x3 / stride 1 layers on rows of 128, 64 or 32 pixels
-  and the strided 4x4 layer of ``DownConvBlock`` from rows of 128, 64 or 32 pixels -- 96 % of the multiply-adds of U-TAE's
-  spatial encoder.  The two 128-channel layers of the last block (16 x 16 pixels) call ``torch.nn.functional.conv2d`` on a
-  reflect-padded bf16 tensor -- a plain cuDNN library convolution, stated here and in DESIGN.md as NOT part of the
-  hand-written path -- followed by ``c2s_group_stats``;
+* convolution: every layer of U-TAE's spatial encoder runs as a hand-written tcgen05 implicit GEMM
+  (``c2s_conv2d_forward``, ``csrc/c2s_conv.cu``): the 3x3 / stride 1 layers with 64 input (or <= 16, the model input) and
+  64 output channels on rows of 128, 64 or 32 pixels, the strided 4x4 layer of ``DownConvBlock`` from rows of 128, 64 or
+  32 pixels, and the 3x3 layers with 64 or 128 channels in and out on whole frames 16 pixels wide (the last block).
+  A layer outside what the kernels serve (another encoder configuration: other widths or resolutions) takes the library
+  branch of ``ConvLayer.forward``: ``torch.nn.functional.conv2d`` on a reflect-padded bf16 tensor -- a plain cuDNN
+  convolution, NOT part of the hand-written path -- followed by ``c2s_group_stats``;
 * GroupNorm + ReLU (+ the residual of ``DownConvBlock``): ``c2s_group_norm_relu``, one element-wise pass, fp32 statistics;
   between two tensor-core stages of one ``ConvLayer`` the pass is skipped: the next convolution normalises its input on
   the fly while it stages it (``c2s_conv_input_norm``).
@@ -58,7 +59,8 @@ def conv2d_supported(x: torch.Tensor, conv: nn.Conv2d) -> bool:
 def conv2d_reflect_forward(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor], *, kernel: int = 3,
                            stride: int = 1, padding: int = 1, with_stats: bool = True, in_norm=None):
     """``c2s_conv2d_forward``: raw convolution output [frames, c_out, H, W] (bf16) and the GroupNorm sums
-    [frames, 4, 2] (float32; quarter-of-the-channels granularity) of its fp32 values.
+    [frames, 4, 2] (float32; per quarter of the c_out channels, i.e. one group of ``GroupNorm(4, c_out)``) of its fp32
+    values.
 
     ``in_norm = (stats, group_norm_module, relu)``: x is the RAW output of the previous stage and the kernel reads
     ``relu(GroupNorm(x))`` on the fly (the previous stage's normalisation pass is skipped)."""
@@ -169,7 +171,7 @@ class ConvLayer(nn.Module):
                 raw, stats = conv2d_reflect_forward(src, conv.weight, conv.bias, kernel=conv.kernel_size[0],
                                                     stride=conv.stride[0], padding=conv.padding[0],
                                                     in_norm=None if pending is None else pending[1:])
-            else:  # library convolution (cuDNN through torch), see the module docstring
+            else:  # library convolution (cuDNN through torch) for shapes no kernel serves, see the module docstring
                 if pending is not None:
                     x = group_norm_relu(pending[0], pending[1], pending[2], relu=pending[3], out=pending[0])
                 pad = conv.padding[0]

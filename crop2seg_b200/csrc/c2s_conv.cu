@@ -21,6 +21,9 @@
 //       umma_commit frees ring slots and hands the accumulator to eight epilogue warps (tmem_ld32), which add the bias,
 //       store the raw (pre-normalisation) row as bf16 NCHW and keep the GroupNorm sums of their frame in registers (one
 //       atomic per warp and quarter of the channels per unit).
+//                        The same contract on whole 16-pixel-wide frames with 64 or 128 channels in and out
+//                        (conv3x3_w16_tc_kernel: padded frame resident, weights streamed by TMA, N = c_out; see there);
+//                        and the strided 4x4 layer of DownConvBlock (conv4x4s2_tc_kernel).
 //   c2s_group_stats      per-(frame, group) sum / sum of squares of a raw NCHW tensor (layers whose convolution ran elsewhere)
 //   c2s_group_norm_relu  y = relu((x - mean) * rstd * gamma + beta) [+ residual]: the second, element-wise pass
 //                        (GroupNorm needs the statistics of the whole frame before the first output element).
@@ -774,6 +777,327 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv4x4s2_tc_kernel(const Con
   if (warp == 0) tmem_dealloc(tacc, 256);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// 3x3 / stride 1 / reflect padding 1 on 16-pixel-wide frames (conv1 / conv2 of U-TAE's last down block, 16 x 16 pixels),
+// c_in and c_out in {64, 128}.  A 16-pixel row is too narrow for one image row per product, so a unit is a whole frame:
+//   * four producer warps store the frame reflect-padded to (H + 2) x 18 pixels, pixel-major, one slot [pixel][64 channels]
+//     per 64-channel K chunk, in the K-major 128-byte-swizzled layout of conv3x3_tc_kernel.  Two frame buffers: the next
+//     frame is staged while the current one computes;
+//   * output pixel (y, x) is accumulator row p = 18 y + x and tap (ky, kx) reads the same slot from row p + 18 ky + kx, so
+//     every tap is a start address.  M = 128 tiles cover p in [0, 18 H): tile t starts at min(128 t, 18 H - 128) -- the
+//     last tile overlaps the one before it rather than reading past the slot; the two junk columns of a row and the
+//     overlapped rows are computed and not stored;
+//   * the weights (c_out x 9 c_in bf16, 295 KB at 128 -> 128: too large to stay resident) stream from L2 by TMA, one
+//     [c_out][64] box per (tap, K chunk) through a ring of kWStages.  The loop is weight-stationary: each box serves every
+//     tile of the frame before the next one is waited for;
+//   * N = c_out (M 128 x N 128 x K 16 products for the 128-channel layers).  Tensor memory holds 512 / c_out tile
+//     accumulators in a ring; the issuer waits for a tile's accumulator just before its first product, so the products
+//     of a frame start while the epilogue still drains the previous one.
+constexpr int kW16Threads = 448;     // warp 0: MMA issuer, warp 1: weight TMA, warps 2-5: producers, warps 6-13: epilogue
+constexpr int kW16Rows = 18;         // padded row pitch in pixels
+constexpr int kW16MaxH = 16;
+// one K-chunk slot: (16 + 2) x 18 pixel rows of 128 B; the last tile reads up to row 18 H + 37 (325 at H = 16), below the
+// 328 rows of the slot
+constexpr int kW16Slot = ((kW16MaxH + 2) * kW16Rows * 128 + 1023) / 1024 * 1024;
+constexpr int kWStages = 3;
+constexpr int kW16AccCols = 512;
+
+__host__ __device__ constexpr size_t w16_smem_bytes(int kc, int n) {
+  return static_cast<size_t>(2) * kc * kW16Slot + static_cast<size_t>(kWStages) * n * 128 + 1024;
+}
+
+template <int KC, int N, bool NORM>
+__global__ void __launch_bounds__(kW16Threads, 1) conv3x3_w16_tc_kernel(const __grid_constant__ CUtensorMap wmap, const ConvArgs a) {
+  constexpr int CIN = KC * 64;
+  constexpr int kAccN = kW16AccCols / N;   // tile accumulators in tensor memory (4 or 8)
+  constexpr int kWBox = N * 128;           // one weight box [N][64] bf16
+  constexpr int kJ = 9 * KC;               // weight boxes per frame
+  extern __shared__ __align__(1024) unsigned char smem_raw[];
+  __shared__ __align__(8) unsigned long long bars[4 + 2 * kWStages + 2 * kAccN];  // in_full[2], in_empty[2], wfull, wempty, tfull, tempty
+  __shared__ uint32_t tmem_s;
+  __shared__ __align__(16) float s_bias[N];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const uint32_t base = (s32(smem_raw) + 1023u) & ~1023u;
+  unsigned char* sm = smem_raw + (base - s32(smem_raw));
+  const uint32_t wring = base + 2 * KC * kW16Slot;
+  const uint32_t bar0 = s32(&bars[0]);
+  auto in_full = [&](int b) { return bar0 + 8u * b; };
+  auto in_empty = [&](int b) { return bar0 + 8u * (2 + b); };
+  auto wfull = [&](int s) { return bar0 + 8u * (4 + s); };
+  auto wempty = [&](int s) { return bar0 + 8u * (4 + kWStages + s); };
+  auto tfull = [&](int b) { return bar0 + 8u * (4 + 2 * kWStages + b); };
+  auto tempty = [&](int b) { return bar0 + 8u * (4 + 2 * kWStages + kAccN + b); };
+  const int P = a.H * kW16Rows;                  // accumulator rows that hold outputs
+  const int n_tiles = (P + 127) / 128;
+  const int last_start = P > 128 ? P - 128 : 0;
+
+  if (tid == 0) {
+    for (int b = 0; b < 2; ++b) mbar_init(in_full(b), 4), mbar_init(in_empty(b), 1);   // one arrival per producer warp
+    for (int s = 0; s < kWStages; ++s) mbar_init(wfull(s), 1), mbar_init(wempty(s), 1);
+    for (int b = 0; b < kAccN; ++b) mbar_init(tfull(b), 1), mbar_init(tempty(b), 8);   // one arrival per epilogue warp
+    fence_mbarrier_init();
+  }
+  if (warp == 0) {
+    tmem_alloc(s32(&tmem_s), kW16AccCols);
+    tmem_relinquish();
+  }
+  if (tid < N) s_bias[tid] = a.bias != nullptr ? a.bias[tid] : 0.f;
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tacc = tmem_s;
+
+  if (warp == 0) {
+    // ---- MMA issuer ----------------------------------------------------------------------------------------------
+    if (elect_one()) {
+      static constexpr uint32_t idesc = umma_idesc_bf16(128, N);
+      const uint32_t w_lo0 = ((wring >> 4) & 0x3fffu) | (1u << 16);
+      uint32_t ws = 0, wphase = 0;             // weight stage of the next box; bit s = parity of stage s
+      uint32_t o = 0;                          // tiles issued
+#ifdef C2S_CONV_TIMING
+      long long dbg_in = 0, dbg_w = 0, dbg_tempty = 0, dbg_frames = 0;
+      const long long dbg_start = clock64();
+#endif
+      int i = 0;
+      for (int f = blockIdx.x; f < a.frames; f += gridDim.x, ++i) {
+        const uint32_t fb = i & 1;
+#ifdef C2S_CONV_TIMING
+        long long dbg_t = clock64();
+#endif
+        mbar_wait(in_full(fb), (i >> 1) & 1);
+#ifdef C2S_CONV_TIMING
+        dbg_in += clock64() - dbg_t;
+#endif
+        tc_fence_after();
+        const uint32_t a_lo0 = (((base + fb * KC * kW16Slot) >> 4) & 0x3fffu) | (1u << 16);
+        int j = 0;
+#pragma unroll 1
+        for (int ky = 0; ky < 3; ++ky) {
+#pragma unroll 1
+          for (int kx = 0; kx < 3; ++kx) {
+#pragma unroll 1
+            for (int kc = 0; kc < KC; ++kc, ++j) {
+#ifdef C2S_CONV_TIMING
+              dbg_t = clock64();
+#endif
+              mbar_wait(wfull(ws), (wphase >> ws) & 1u);
+#ifdef C2S_CONV_TIMING
+              dbg_w += clock64() - dbg_t;
+#endif
+              tc_fence_after();
+              const uint32_t b_lo = w_lo0 + ws * (kWBox >> 4);
+              // tap (ky, kx) = start row 18 ky + kx of the K chunk's slot (8 x 16 B per pixel row)
+              const uint32_t a_lo = a_lo0 + kc * (kW16Slot >> 4) + (ky * kW16Rows + kx) * 8;
+#pragma unroll 1
+              for (int t = 0; t < n_tiles; ++t) {
+                const uint32_t ot = o + t, buf = ot % kAccN;
+                if (j == 0) {
+#ifdef C2S_CONV_TIMING
+                  dbg_t = clock64();
+#endif
+                  if (ot >= kAccN) mbar_wait(tempty(buf), ((ot / kAccN) - 1u) & 1u);
+#ifdef C2S_CONV_TIMING
+                  dbg_tempty += clock64() - dbg_t;
+#endif
+                  tc_fence_after();
+                }
+                const uint32_t d_tmem = tacc + buf * N;
+                const uint32_t at = a_lo + min(t * 128, last_start) * 8;
+#pragma unroll
+                for (int ks = 0; ks < 4; ++ks)
+                  umma_bf16(d_tmem, desc_from(at + ks * 2), desc_from(b_lo + ks * 2), idesc, (j | ks) != 0);
+                if (j == kJ - 1) umma_commit(tfull(buf));
+              }
+              umma_commit(wempty(ws));         // the box is dead once the products issued so far are done
+              wphase ^= 1u << ws;
+              ws = ws + 1 == kWStages ? 0 : ws + 1;
+            }
+          }
+        }
+        umma_commit(in_empty(fb));
+        o += n_tiles;
+#ifdef C2S_CONV_TIMING
+        ++dbg_frames;
+#endif
+      }
+#ifdef C2S_CONV_TIMING
+      if (blockIdx.x == 0 && dbg_frames > 0)
+        printf("[conv3x3 W=16 c_in=%d c_out=%d H=%d] issuer of CTA 0: %lld frames, %lld cycles per frame; per frame: wait input "
+               "%lld, wait weights %lld, wait tempty %lld\n", CIN, N, a.H, dbg_frames, (clock64() - dbg_start) / dbg_frames,
+               dbg_in / dbg_frames, dbg_w / dbg_frames, dbg_tempty / dbg_frames);
+#endif
+    }
+  } else if (warp == 1) {
+    // ---- weight boxes: TMA from the prepared weights [N][9 CIN], box (tap, K chunk) = columns 64 j .. 64 j + 63 ---------
+    if (elect_one()) {
+      uint32_t s = 0, round = 0;               // stage of the next box, passes through the ring so far
+      for (int f = blockIdx.x; f < a.frames; f += gridDim.x) {
+        for (int j = 0; j < kJ; ++j) {
+          if (round > 0) mbar_wait(wempty(s), (round - 1u) & 1u);
+          mbar_expect_tx(wfull(s), kWBox);
+          tma_load_2d(wring + s * kWBox, &wmap, j * 64, 0, wfull(s));
+          if (++s == kWStages) s = 0, ++round;
+        }
+      }
+    }
+  } else if (warp <= 5) {
+    // ---- producers: one 8 channel x 8 pixel block per thread and step; thread = (channel block, first pixel block) ------
+    constexpr int CB = CIN / 8;
+    constexpr int TPB = 128 / CB;               // threads sharing a channel block (16 or 8)
+    const int ptid = tid - 64;
+    const int cb = ptid % CB, p0 = ptid / CB;   // pixel block pb = (row pb / 2, half pb & 1); this thread: p0, p0 + TPB, ..
+    const int piece = cb & 7;
+    const int nblk = 2 * a.H;
+    const bool active = p0 < nblk;
+    const size_t plane = static_cast<size_t>(a.H) * 16;
+    auto load_blk = [&](uint4 (&v)[8], int f, int pb) {
+      const __nv_bfloat16* src = a.x + (static_cast<size_t>(f) * CIN + cb * 8) * plane + (pb >> 1) * 16 + (pb & 1) * 8;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) v[k] = __ldg(reinterpret_cast<const uint4*>(src + k * plane));
+    };
+    // the next block to load: one block of latency hiding, across frame boundaries
+    int lf = blockIdx.x, lp = p0;
+    uint4 vn[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) vn[k] = make_uint4(0, 0, 0, 0);
+    if (active && lf < a.frames) load_blk(vn, lf, lp);
+    float sc[8], sh[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) sc[k] = 1.f, sh[k] = 0.f;
+    int i = 0;
+    for (int f = blockIdx.x; f < a.frames; f += gridDim.x, ++i) {
+      const uint32_t fb = i & 1;
+      if (NORM && active) {  // scale / shift of this thread's 8 channels in frame f, as in conv3x3_tc_kernel
+        const int cpg = CIN / a.in_groups, spg = a.in_sub / a.in_groups;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+          const int c = cb * 8 + k;
+          const int grp = c / cpg;
+          double t1 = 0.0, t2 = 0.0;
+          for (int s = 0; s < spg; ++s) {
+            t1 += a.in_stats[(static_cast<size_t>(f) * a.in_sub + grp * spg + s) * 2];
+            t2 += a.in_stats[(static_cast<size_t>(f) * a.in_sub + grp * spg + s) * 2 + 1];
+          }
+          const double n = static_cast<double>(cpg) * a.H * 16;
+          const double mean = t1 / n;
+          double var = t2 / n - mean * mean;
+          var = var < 0.0 ? 0.0 : var;
+          sc[k] = static_cast<float>(1.0 / sqrt(var + static_cast<double>(a.in_eps))) * a.in_gamma[c];
+          sh[k] = a.in_beta[c] - static_cast<float>(mean) * sc[k];
+        }
+      }
+      if (i >= 2) mbar_wait(in_empty(fb), ((i >> 1) - 1) & 1);
+      unsigned char* sl = sm + (fb * KC + (cb >> 3)) * kW16Slot;
+      for (int pb = p0; active && pb < nblk; pb += TPB) {
+        uint4 v[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v[k] = vn[k];
+        lp += TPB;
+        if (lp >= nblk) lf += gridDim.x, lp = p0;
+        if (lf < a.frames) load_blk(vn, lf, lp);
+        if (NORM) {  // the same arithmetic as group_norm_relu_kernel: fma in fp32, ReLU, round to bf16
+#pragma unroll
+          for (int k = 0; k < 8; ++k) {
+            float e[8];
+            Elem<__nv_bfloat16>::unpack(v[k], e);
+#pragma unroll
+            for (int m = 0; m < 8; ++m) {
+              e[m] = fmaf(e[m], sc[k], sh[k]);
+              if (a.in_relu) e[m] = fmaxf(e[m], 0.f);
+            }
+            v[k] = Elem<__nv_bfloat16>::pack(e);
+          }
+        }
+        const int y = pb >> 1, h = pb & 1;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const uint32_t sel = (j & 1) ? 0x7632u : 0x5410u;
+          // word j / 2 of channel k holds pixels (j & ~1, j | 1) of that channel
+          auto word = [&](int k) -> uint32_t {
+            return (j >> 1) == 0 ? v[k].x : ((j >> 1) == 1 ? v[k].y : ((j >> 1) == 2 ? v[k].z : v[k].w));
+          };
+          uint4 w;
+          w.x = __byte_perm(word(0), word(1), sel);
+          w.y = __byte_perm(word(2), word(3), sel);
+          w.z = __byte_perm(word(4), word(5), sel);
+          w.w = __byte_perm(word(6), word(7), sel);
+          // pixel (y, 8 h + j) -> padded (y + 1, 8 h + j + 1); reflected copies: column 0 = column 2, column 17 = column 15,
+          // row 0 = row 2, row H + 1 = row H - 1 (padded coordinates)
+          auto put_row = [&](int R) {
+            auto st = [&](int col) {
+              const int r = R * kW16Rows + col;
+              *reinterpret_cast<uint4*>(sl + r * 128 + ((piece ^ (r & 7)) << 4)) = w;
+            };
+            st(8 * h + j + 1);
+            if (h == 0 && j == 1) st(0);
+            if (h == 1 && j == 6) st(17);
+          };
+          put_row(y + 1);
+          if (y == 1) put_row(0);
+          if (y == a.H - 2) put_row(a.H + 1);
+        }
+      }
+      fence_proxy_async();  // generic stores -> tensor-core (async proxy) reads
+      __syncwarp();
+      if (lane == 0) mbar_arrive(in_full(fb));
+    }
+  } else {
+    // ---- epilogue: TMEM lanes 32 q .. 32 q + 31 = accumulator rows of a tile; the two warps of a quarter split the channels
+    constexpr int NH = N / 2, NCH = NH / 32, QW = N / 4;  // channels per warp, 32-column loads, channels per stats quarter
+    const int q = warp & 3, half = (warp - 6) >> 2;
+    const size_t cstride = static_cast<size_t>(a.H) * 16;
+    unsigned o = 0;
+    for (int f = blockIdx.x; f < a.frames; f += gridDim.x) {
+      float s1[2] = {0.f, 0.f}, s2[2] = {0.f, 0.f};  // the two stats quarters of this warp's channels
+      for (int t = 0; t < n_tiles; ++t, ++o) {
+        const unsigned buf = o % kAccN;
+        mbar_wait(tfull(buf), (o / kAccN) & 1u);
+        tc_fence_after();
+        uint32_t r[NCH][32];
+#pragma unroll
+        for (int cc = 0; cc < NCH; ++cc)
+          tmem_ld32(tacc + (static_cast<uint32_t>(q * 32) << 16) + buf * N + half * NH + cc * 32, r[cc]);
+        tmem_wait_ld();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(tempty(buf));  // the accumulator is in registers
+        const int p = min(t * 128, last_start) + q * 32 + lane;
+        const int y = p / kW16Rows, x = p - y * kW16Rows;
+        const bool valid = x < 16 && p < P && p >= t * 128;  // junk columns, tail rows, rows the previous tile stored
+        __nv_bfloat16* dst = a.y + ((static_cast<size_t>(f) * N + half * NH) * a.H + y) * 16 + x;
+#pragma unroll
+        for (int cc = 0; cc < NCH; ++cc) {
+#pragma unroll
+          for (int c4 = 0; c4 < 8; ++c4) {
+            const float4 b4 = *reinterpret_cast<const float4*>(&s_bias[half * NH + cc * 32 + c4 * 4]);
+            const float bb[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              const int c = cc * 32 + c4 * 4 + e;
+              const float v0 = valid ? __uint_as_float(r[cc][c4 * 4 + e]) + bb[e] : 0.f;
+              if (valid) dst[c * cstride] = __float2bfloat16_rn(v0);
+              s1[c / QW] += v0, s2[c / QW] = fmaf(v0, v0, s2[c / QW]);
+            }
+          }
+        }
+      }
+      if (a.stats != nullptr) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+          const float t1 = warp_sum(s1[k]), t2 = warp_sum(s2[k]);
+          if (lane == 0) {
+            atomicAdd(a.stats + (static_cast<size_t>(f) * kStatQuarters + half * 2 + k) * 2, t1);
+            atomicAdd(a.stats + (static_cast<size_t>(f) * kStatQuarters + half * 2 + k) * 2 + 1, t2);
+          }
+        }
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) tmem_dealloc(tacc, kW16AccCols);
+}
+
 // weight[c_out][c_in][3][3] fp32 -> wp[c_out][chunks * 64] bf16 with k = tap * CK + c (zero for c >= c_in and behind 9 CK)
 __global__ void conv_weight_prep_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wp, int c_out, int c_in, int ck,
                                         int k_total, int taps) {
@@ -894,6 +1218,11 @@ bool conv_is_down(const c2s_conv_desc& d) {
   return d.kernel == 4 && d.stride == 2 && d.padding == 1 && (d.W == 128 || d.W == 64 || d.W == 32) && d.H >= 4 && d.H % 2 == 0 && d.c_in == 64 &&
          d.c_out == kCN && d.dtype == C2S_BF16 && d.frames > 0;
 }
+// 3x3 / stride 1 / padding 1 on whole 16-pixel-wide frames, 64 or 128 channels in and out (conv3x3_w16_tc_kernel)
+bool conv_is_w16(const c2s_conv_desc& d) {
+  return d.kernel == 3 && d.stride == 1 && d.padding == 1 && d.W == 16 && d.H >= 2 && d.H <= kW16MaxH &&
+         (d.c_in == 64 || d.c_in == 128) && (d.c_out == 64 || d.c_out == 128) && d.dtype == C2S_BF16 && d.frames > 0;
+}
 
 }  // namespace
 }  // namespace c2s
@@ -902,7 +1231,7 @@ extern "C" {
 
 int c2s_conv2d_supported(const c2s_conv_desc* d) {
   if (d == nullptr) return 0;
-  if (c2s::conv_is_down(*d)) return 1;
+  if (c2s::conv_is_down(*d) || c2s::conv_is_w16(*d)) return 1;
   return d->kernel == 3 && d->stride == 1 && d->padding == 1 && (d->W == 128 || d->W == 64 || d->W == 32) && d->H >= 2 && d->c_out == c2s::kCN &&
          (d->c_in <= 16 || d->c_in == 64) && d->c_in >= 1 && d->dtype == C2S_BF16 && d->frames > 0;
 }
@@ -910,6 +1239,7 @@ int c2s_conv2d_supported(const c2s_conv_desc* d) {
 size_t c2s_conv2d_workspace_bytes(const c2s_conv_desc* d) {
   if (!c2s_conv2d_supported(d)) return 0;
   if (c2s::conv_is_down(*d)) return static_cast<size_t>(c2s::kCN) * c2s::kDChunks * 64 * sizeof(__nv_bfloat16);
+  if (c2s::conv_is_w16(*d)) return static_cast<size_t>(d->c_out) * 9 * d->c_in * sizeof(__nv_bfloat16);
   return static_cast<size_t>(c2s::kCN) * c2s::conv_chunks(c2s::conv_ck(d->c_in)) * 64 * sizeof(__nv_bfloat16);
 }
 
@@ -919,10 +1249,11 @@ int c2s_conv2d_forward(const c2s_conv_desc* desc, const void* x, const c2s_conv_
   C2S_CHECK_ARG(desc != nullptr && x != nullptr && weight != nullptr && y != nullptr, "c2s_conv2d_forward: NULL argument");
   const c2s_conv_desc& d = *desc;
   if (!c2s_conv2d_supported(desc))
-    C2S_UNSUPPORTED("c2s_conv2d_forward: serves 3x3 / stride 1 / reflect padding 1, W = 128, 64 or 32, c_out = 64, c_in <= 16 or 64, "
+    C2S_UNSUPPORTED("c2s_conv2d_forward: serves 3x3 / stride 1 / reflect padding 1, W = 128, 64 or 32, c_out = 64, c_in <= 16 or 64; "
+                    "3x3 / stride 1 / reflect padding 1, W = 16, H <= 16, c_in and c_out 64 or 128; "
                     "and 4x4 / stride 2 / padding 1, W = 128, 64 or 32, even H, 64 -> 64 channels; bf16 "
-                    "(got k=%d s=%d p=%d W=%d c_in=%d c_out=%d dtype=%d)", d.kernel, d.stride, d.padding, d.W, d.c_in, d.c_out,
-                    d.dtype);
+                    "(got k=%d s=%d p=%d H=%d W=%d c_in=%d c_out=%d dtype=%d)", d.kernel, d.stride, d.padding, d.H, d.W, d.c_in,
+                    d.c_out, d.dtype);
   C2S_CHECK_ARG(reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(y) % 16 == 0,
                 "c2s_conv2d_forward: x and y must be 16-byte aligned");
   const size_t need = c2s_conv2d_workspace_bytes(desc);
@@ -931,10 +1262,13 @@ int c2s_conv2d_forward(const c2s_conv_desc* desc, const void* x, const c2s_conv_
   int status = check_device();
   if (status != C2S_OK) return status;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
-  const bool down = conv_is_down(d);
-  const int ck = conv_ck(d.c_in), chunks = down ? kDChunks : conv_chunks(ck), k_total = chunks * 64;
+  const bool down = conv_is_down(d), w16 = conv_is_w16(d);
+  const int c_out = w16 ? d.c_out : kCN;
+  const int ck = w16 ? d.c_in : conv_ck(d.c_in), chunks = down ? kDChunks : conv_chunks(ck), k_total = chunks * 64;
   __nv_bfloat16* wp = static_cast<__nv_bfloat16*>(workspace);
-  conv_weight_prep_kernel<<<ceil_div(kCN * k_total, 256), 256, 0, stream>>>(weight, wp, kCN, d.c_in, ck, k_total, down ? 16 : 9);
+  if (w16)  // the weight boxes are loaded by TMA
+    C2S_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 16 == 0, "c2s_conv2d_forward: the workspace must be 16-byte aligned");
+  conv_weight_prep_kernel<<<ceil_div(c_out * k_total, 256), 256, 0, stream>>>(weight, wp, c_out, d.c_in, ck, k_total, down ? 16 : 9);
   C2S_LAUNCH_CHECK("conv_weight_prep");
   if (stats != nullptr) C2S_CUDA(cudaMemsetAsync(stats, 0, static_cast<size_t>(d.frames) * kStatQuarters * 2 * sizeof(float), stream));
   const int sms = sm_count();
@@ -948,6 +1282,39 @@ int c2s_conv2d_forward(const c2s_conv_desc* desc, const void* x, const c2s_conv_
                   in_norm->n_sub, d.c_in);
     a.in_stats = in_norm->stats, a.in_gamma = in_norm->gamma, a.in_beta = in_norm->beta;
     a.in_groups = in_norm->n_groups, a.in_sub = in_norm->n_sub, a.in_relu = in_norm->relu, a.in_eps = in_norm->eps;
+  }
+  if (w16) {  // one unit per frame
+    CUtensorMap wmap;
+    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(k_total), static_cast<cuuint64_t>(c_out)};
+    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(k_total) * sizeof(__nv_bfloat16)};
+    const cuuint32_t box[2] = {64, static_cast<cuuint32_t>(c_out)};
+    status = encode_tensor_map(&wmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, wp, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "prepared conv weights");
+    if (status != C2S_OK) return status;
+    const int grid_w = d.frames < sms ? d.frames : sms;
+    const size_t smem_w = w16_smem_bytes(d.c_in / 64, c_out);
+#define C2S_CONV_W16_LAUNCH(KC_, N_, NORM_)                                                       \
+  do {                                                                                            \
+    C2S_SMEM_ATTR((conv3x3_w16_tc_kernel<KC_, N_, NORM_>), smem_w);                               \
+    conv3x3_w16_tc_kernel<KC_, N_, NORM_><<<grid_w, kW16Threads, smem_w, stream>>>(wmap, a);      \
+  } while (0)
+    const bool norm = in_norm != nullptr;
+    if (d.c_in == 64 && c_out == 64) {
+      if (norm) C2S_CONV_W16_LAUNCH(1, 64, true);
+      else C2S_CONV_W16_LAUNCH(1, 64, false);
+    } else if (d.c_in == 64) {
+      if (norm) C2S_CONV_W16_LAUNCH(1, 128, true);
+      else C2S_CONV_W16_LAUNCH(1, 128, false);
+    } else if (c_out == 64) {
+      if (norm) C2S_CONV_W16_LAUNCH(2, 64, true);
+      else C2S_CONV_W16_LAUNCH(2, 64, false);
+    } else {
+      if (norm) C2S_CONV_W16_LAUNCH(2, 128, true);
+      else C2S_CONV_W16_LAUNCH(2, 128, false);
+    }
+#undef C2S_CONV_W16_LAUNCH
+    C2S_LAUNCH_CHECK("conv3x3_reflect_w16<tcgen05>");
+    return C2S_OK;
   }
   if (down) {  // units are bands of OUTPUT rows
     C2S_CHECK_ARG(in_norm == nullptr, "c2s_conv2d_forward: the strided layer reads a normalised input (no in_norm)");

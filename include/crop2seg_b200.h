@@ -398,10 +398,11 @@ typedef struct c2s_conv_desc {
   int32_t dtype;                   /* enum c2s_dtype of x and y                                  */
 } c2s_conv_desc;
 
-/* 1 when c2s_conv2d_forward serves the layer on the tensor cores (bf16, c_out = 64):
- *   3x3, stride 1, padding 1, W = 128 / 64 / 32, c_in <= 16 or c_in = 64   (in_conv, conv1 / conv2 of the down blocks)
- *   4x4, stride 2, padding 1, W = 128 / 64 / 32, even H, c_in = 64         (the strided layer of DownConvBlock, conv.py:252-263)
- * Other layers (128 channels) are the caller's business. */
+/* 1 when c2s_conv2d_forward serves the layer on the tensor cores (bf16):
+ *   3x3, stride 1, padding 1, W = 128 / 64 / 32, c_in <= 16 or c_in = 64, c_out = 64   (in_conv, conv1 / conv2 of the down blocks)
+ *   3x3, stride 1, padding 1, W = 16, 2 <= H <= 16, c_in and c_out 64 or 128           (conv1 / conv2 of U-TAE's last down block)
+ *   4x4, stride 2, padding 1, W = 128 / 64 / 32, even H, 64 -> 64 channels             (the strided layer of DownConvBlock, conv.py:252-263)
+ * Other layers are the caller's business. */
 int c2s_conv2d_supported(const c2s_conv_desc* desc);
 size_t c2s_conv2d_workspace_bytes(const c2s_conv_desc* desc); /* prepared bf16 weights */
 
@@ -419,8 +420,10 @@ typedef struct c2s_conv_input_norm {
  *   x      : [frames, c_in, H, W] bf16;  x' = x, or relu(GroupNorm(x)) rounded to bf16 when in_norm is given (3x3 only)
  *   weight : float32 [c_out, c_in, k, k] (nn.Conv2d.weight), bias float32 [c_out] | NULL
  *   y      : [frames, c_out, H / s, W / s] bf16, the RAW convolution output (GroupNorm needs the whole frame first)
- *   stats  : float32 [frames][4][2] = (sum, sum of squares) of the fp32 outputs per frame and quarter of the channels
- *            (written, not accumulated), for c2s_group_norm_relu / c2s_conv_input_norm with n_sub = 4; or NULL */
+ *   stats  : float32 [frames][4][2] = (sum, sum of squares) of the fp32 outputs per frame and quarter of the c_out channels
+ *            (16 or 32 channels; written, not accumulated), for c2s_group_norm_relu / c2s_conv_input_norm with n_sub = 4;
+ *            or NULL
+ *   workspace: c2s_conv2d_workspace_bytes, 16-byte aligned */
 int c2s_conv2d_forward(const c2s_conv_desc* desc, const void* x, const c2s_conv_input_norm* in_norm, const float* weight,
                        const float* bias, void* y, float* stats, void* workspace, size_t workspace_bytes, void* stream);
 

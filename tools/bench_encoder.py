@@ -2,7 +2,10 @@
 """Throughput of the shared conv encoder slice (SURVEY.md section 8f, rank 4): the tcgen05 3x3 reflect convolution at
 the full resolution, the normalisation pass, and U-TAE's ``in_conv`` block on packed frames.  One JSON line per record.
 
-    python tools/bench_encoder.py [--frames 1024] [--seconds 0.5]
+    python tools/bench_encoder.py [--frames 1024] [--seconds 0.5] [--last-block]
+
+``--last-block`` runs only the records of U-TAE's last down block (the 16 x 16 kernel against the library route it
+replaced, alternated in one run) and the four-block encoder total.
 
 ``cudnn_*`` lines time ``torch.nn.functional.conv2d`` on the same bf16 tensors (reflect padding done beforehand, outside
 the timed region for the NCHW line) -- a library yardstick, not part of the product path.
@@ -10,6 +13,8 @@ the timed region for the NCHW line) -- a library yardstick, not part of the prod
 import argparse
 import json
 import os
+import statistics
+import subprocess
 import sys
 
 import torch
@@ -41,9 +46,15 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--frames", type=int, default=1024)
     ap.add_argument("--seconds", type=float, default=0.5)
+    ap.add_argument("--last-block", action="store_true")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
+    print(json.dumps(card()), flush=True)
+    if args.last_block:
+        last_block(args.frames, args.seconds)
+        full_encoder(args.frames, args.seconds)
+        return
     n, H, W = args.frames, 128, 128
     peaks = {}
     p = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "MEASURED_PEAKS.json")
@@ -125,6 +136,54 @@ def main():
                       "ms_strided_layer": ms_down, "frames_per_s": n / ms * 1e3, "tflops": flops / ms * 1e-9}), flush=True)
     del x
     full_encoder(n, args.seconds)
+
+
+def card():
+    """The device the numbers below were taken on: name and power limit (nvidia-smi, read only)."""
+    rec = {"record": "card", "name": torch.cuda.get_device_name(0)}
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                           capture_output=True, text=True, timeout=30)
+        rec["power_limit_and_max_sm_clock"] = q.stdout.strip() if q.returncode == 0 else "unknown"
+    except (OSError, subprocess.TimeoutExpired):
+        rec["power_limit_and_max_sm_clock"] = "unknown"
+    return rec
+
+
+def library_conv(x, conv, n_groups):
+    """The route ConvLayer took for these layers before conv3x3_reflect_w16 served them: F.pad + cuDNN F.conv2d + group_stats."""
+    wb, bb = conv.weight.to(torch.bfloat16), conv.bias.to(torch.bfloat16)
+    raw = F.conv2d(F.pad(x, (1, 1, 1, 1), mode="reflect"), wb, bb)
+    return raw, cc.group_stats(raw, n_groups)
+
+
+def last_block(n, seconds, rounds=5):
+    """U-TAE's last down block (64 -> 128 channels, 32^2 -> 16^2): its two 128-channel layers on the 16-pixel-wide kernel
+    and on the library route, and the whole block, alternated round by round; the median of the rounds is reported."""
+    dev = torch.device("cuda", 0)
+    blk = c2s.DownConvBlock(64, 128, 4, 2, 1, pad_value=0, norm="group").to(dev).eval()
+    x32 = torch.randn((n, 64, 32, 32), device=dev).to(torch.bfloat16)
+    x1 = torch.randn((n, 64, 16, 16), device=dev).to(torch.bfloat16)
+    x2 = torch.randn((n, 128, 16, 16), device=dev).to(torch.bfloat16)
+    c1, c2 = blk.conv1.conv[0], blk.conv2.conv[0]
+    cases = {
+        "conv1 64->128 @16 conv3x3_reflect_w16<tcgen05>": (lambda: cc.conv2d_reflect_forward(x1, c1.weight, c1.bias), 64),
+        "conv1 64->128 @16 library route (F.pad + F.conv2d + group_stats)": (lambda: library_conv(x1, c1, 4), 64),
+        "conv2 128->128 @16 conv3x3_reflect_w16<tcgen05>": (lambda: cc.conv2d_reflect_forward(x2, c2.weight, c2.bias), 128),
+        "conv2 128->128 @16 library route (F.pad + F.conv2d + group_stats)": (lambda: library_conv(x2, c2, 4), 128),
+        "down3 block DownConvBlock(64, 128, 4, 2, 1) 32^2 -> 16^2": (lambda: blk(x32), None),
+    }
+    times = {k: [] for k in cases}
+    with torch.no_grad():
+        for _ in range(rounds):
+            for k, (fn, _c) in cases.items():
+                times[k].append(timed(fn, seconds / rounds))
+    for k, (fn, c_in) in cases.items():
+        ms = statistics.median(times[k])
+        rec = {"record": k, "frames": n, "ms": ms, "ms_rounds": [round(t, 4) for t in times[k]]}
+        if c_in is not None:
+            rec["tflops"] = 2.0 * n * 16 * 16 * 128 * c_in * 9 / ms * 1e-9
+        print(json.dumps(rec), flush=True)
 
 
 def full_encoder(n, seconds):

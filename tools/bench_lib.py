@@ -264,9 +264,9 @@ def encoder(dev, frames=1024, min_seconds=1.0, seed=1234):
                                           "a 32-cycle tensor floor (tools/ubench/umma_rowshift.cu), i.e. at most 0.67 of "
                                           "the nominal rate with 64 output channels"}}
     del x, x64
-    # the four blocks of the spatial encoder one after the other (utae.py:128-149): every 64 -> 64 layer runs on the
-    # tensor-core kernels (3x3 with 128 / 64 / 32-pixel rows, strided 4x4 with parity-split rows); the two 128-channel layers
-    # of the last block (3.8 % of the multiply-adds) are library convolutions, said so in conv.py
+    # the four blocks of the spatial encoder one after the other (utae.py:128-149): every layer runs on the tensor-core
+    # kernels (3x3 with 128 / 64 / 32-pixel rows, strided 4x4 with parity-split rows, 3x3 on whole 16 x 16 frames for the
+    # 128-channel layers of the last block); the share of the multiply-adds they serve is read from conv2d_supported
     blocks = [("in_conv", blk, (10, 128)),
               ("down1", c2s.DownConvBlock(64, 64, 4, 2, 1, pad_value=0, norm="group").to(dev).eval(), (64, 128)),
               ("down2", c2s.DownConvBlock(64, 64, 4, 2, 1, pad_value=0, norm="group").to(dev).eval(), (64, 64)),
@@ -283,9 +283,28 @@ def encoder(dev, frames=1024, min_seconds=1.0, seed=1234):
     rec["spatial_encoder"] = {"workload": "U-TAE spatial encoder (in_conv + 3 DownConvBlock, widths [64,64,64,128]) on packed frames, "
                                           "block by block", "ms_per_block": per, "ms": total,
                               "frames_per_s": world * frames / (total * 1e-3), "tflops": 2.0 * frames * macs / total * 1e-9,
-                              "hand_written_share_of_macs": 1.0 - 16 * 16 * (9 * 64 * 128 + 9 * 128 * 128) / macs}
+                              "hand_written_share_of_macs": _hand_written_share(blocks, dev)}
     torch.cuda.empty_cache()
     return rec
+
+
+def _hand_written_share(blocks, dev):
+    """Share of the convolution multiply-adds of ``blocks`` that ``conv2d_supported`` routes to the hand-written kernels."""
+    from crop2seg_b200 import conv as cc
+    total = hand = 0
+    for _, b, (c, r) in blocks:
+        h = r
+        for layer in ([b.conv] if isinstance(b, c2s.ConvBlock) else [b.down, b.conv1, b.conv2]):
+            for ci, _, _ in layer._plan:
+                conv = layer.conv[ci]
+                k, st, p = conv.kernel_size[0], conv.stride[0], conv.padding[0]
+                ho = (h + 2 * p - k) // st + 1
+                macs = ho * ho * conv.out_channels * conv.in_channels * k * k
+                total += macs
+                if cc.conv2d_supported(torch.empty((1, conv.in_channels, h, h), device=dev, dtype=torch.bfloat16), conv):
+                    hand += macs
+                h = ho
+    return hand / total
 
 
 # ------------------------------------------------------------------------------------------------ configs[4]
