@@ -443,6 +443,7 @@ __global__ void __launch_bounds__(kPipeMaxConsumers + 32, (S >= 4 && sizeof(T) =
 #pragma unroll
       for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
     }
+    fence_proxy_async();  // the stage's shared loads before the producer's next bulk copy into it (see agg_backward_pipe)
     __syncwarp();
     if (lane == 0) mbar_arrive(s32(&bars[16 + s]));  // the stage's data now lives in registers
 
@@ -734,6 +735,7 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
 #pragma unroll
       for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
     }
+    fence_proxy_async();  // the stage's shared loads before the producer's next bulk copy into it
     __syncwarp();
     if (lane == 0) mbar_arrive(s32(&bars[16 + s]));
 

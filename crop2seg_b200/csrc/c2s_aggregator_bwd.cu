@@ -400,6 +400,10 @@ agg_backward_pipe_kernel(const AggBwdArgs a, int n_stages, int n_consumers, int 
         r[jj] = fmaf(ly1, tp[trow1 + cj], ly0 * tp[trow0 + cj]);
       }
     }
+    // the stage's reads (generic proxy) must be performed before the producer's next bulk copy (async proxy) into it:
+    // without the fence the arrive can overtake the shared loads and the first frames of a time chunk read their
+    // successors' rows
+    fence_proxy_async();
     __syncwarp();
     if (lane == 0) mbar_arrive(s32(&bars[16 + s]));  // the stage's data now lives in registers
     ++i;

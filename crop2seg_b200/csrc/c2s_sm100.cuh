@@ -49,7 +49,8 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 // ---------------------------------------------------------------------------------------------
 // bulk and tensor copies (TMA): global -> shared complete on an mbarrier transaction count
 // ---------------------------------------------------------------------------------------------
-// generic-proxy writes to shared memory before async-proxy (TMA, tcgen05) accesses of the same bytes
+// generic-proxy accesses of shared memory (writes, and reads of a buffer about to be refilled) before async-proxy (TMA,
+// tcgen05) accesses of the same bytes
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // 1-D bulk copy (UBLKCP in SASS)

@@ -15,6 +15,9 @@ algorithm, including the [N,T,D] activations and head-major copies the fused ker
     TemporalAggregator.forward          src/backbones/temporal_aggregator.py:14-77
 
 Parity status: pinned against the committed reference outputs (tests/test_oracle_golden.py).
+
+Precision: float32 unless x is float64; then, with float64 parameters, every step runs in float64 on x's device, which
+makes it the high-precision reference of the kernels' tests (tests/test_gpu_training_float64.py).
 """
 from __future__ import annotations
 
@@ -28,8 +31,16 @@ def _t(a) -> torch.Tensor:
     return a if isinstance(a, torch.Tensor) else torch.from_numpy(a)
 
 
+def _real(a) -> torch.Tensor:
+    """float64 stays float64 (a high-precision reference), every other type computes in float32."""
+    a = _t(a)
+    return a if a.dtype == torch.float64 else a.float()
+
+
 def _sinusoid(pos_rows, denom, repeat, fc_w=None, fc_b=None):
-    table = pos_rows[:, :, None] / denom[None, None, :]  # positional_encoding.py:29-31
+    # positional_encoding.py:29-31; the reference's denom is a float32 attribute, so the angle is a float32 quotient
+    # even where the rest of the table is computed in float64
+    table = (pos_rows[:, :, None] / denom[None, None, :].float()).to(denom.dtype)
     table[:, :, 0::2] = torch.sin(table[:, :, 0::2])
     table[:, :, 1::2] = torch.cos(table[:, :, 1::2])
     table = table.repeat(1, 1, repeat)  # :35-38
@@ -37,14 +48,14 @@ def _sinusoid(pos_rows, denom, repeat, fc_w=None, fc_b=None):
 
 
 def _doy(pos_rows, fc_w, fc_b, repeat):
-    onehot = F.one_hot(pos_rows.to(torch.int64), num_classes=365).to(torch.float32)  # positional_encoding.py:63
+    onehot = F.one_hot(pos_rows.to(torch.int64), num_classes=365).to(fc_w.dtype)  # positional_encoding.py:63
     return F.linear(onehot, fc_w, fc_b).repeat(1, 1, repeat)  # :66-71
 
 
 def ltae_forward_torch(cfg, params: Dict, x, positions=None, pad_mask=None, attn_only: bool = False,
                        training: bool = False, attn_keep=None, mlp_keep=None, attn_drop_p: float = 0.1,
                        mlp_drop_p: float = 0.2, materialise: bool = True):
-    """``LTAE.forward`` (or ``LTAE4WTAE.forward`` with ``attn_only``) on CPU tensors, differentiable.
+    """``LTAE.forward`` (or ``LTAE4WTAE.forward`` with ``attn_only``), differentiable, on x's device and precision.
 
     ``cfg`` is an ``oracle.LtaeConfig``; ``params`` is keyed like the reference ``state_dict``.
     ``training``: BatchNorm1d batch statistics (tae.py:445) and the two dropouts with INJECTED keep masks (torch's
@@ -55,20 +66,20 @@ def ltae_forward_torch(cfg, params: Dict, x, positions=None, pad_mask=None, attn
     ``pad_mask.repeat``, :772) so that the CPU timing is the reference's, not a cheaper one.
     """
     p = {k: _t(v) for k, v in params.items()}
-    x = _t(x).float()
+    x = _real(x)
     b, t, c, hh, ww = x.shape
     h, dk, d = cfg.n_head, cfg.d_k, cfg.width
     rows = x.permute(0, 3, 4, 1, 2).reshape(b * hh * ww, t, c)  # tae.py:460
     n = rows.shape[0]
     pad_rows = None
     if pad_mask is not None:
-        pad_rows = _t(pad_mask).bool()[:, None, None, :].expand(b, hh, ww, t).reshape(n, t)  # :453-457
+        pad_rows = _t(pad_mask).to(x.device).bool()[:, None, None, :].expand(b, hh, ww, t).reshape(n, t)  # :453-457
     e = F.group_norm(rows.permute(0, 2, 1), h, p["in_norm.weight"], p["in_norm.bias"], 1e-5)  # :461  [N,C,T]
     if cfg.d_model is not None:
         e = F.conv1d(e, p["inconv.weight"], p["inconv.bias"])  # :463-464
     e = e.permute(0, 2, 1)  # [N,T,D]
     if cfg.positional_encoding:
-        pos = _t(positions)
+        pos = _t(positions).to(x.device)
 
         def per_pixel(q):
             return q[:, None, None, :].expand(b, hh, ww, t).reshape(n, t)
@@ -99,7 +110,7 @@ def ltae_forward_torch(cfg, params: Dict, x, positions=None, pad_mask=None, attn
         s = s.masked_fill(pad_rows.repeat(h, 1).unsqueeze(1), -1e6)  # :831
     a = torch.softmax(s, dim=2)  # :836
     if training and attn_keep is not None:  # :837 nn.Dropout(0.1): zero and rescale, BEFORE the attention is returned
-        ak = _t(attn_keep).to(torch.float32).permute(0, 1, 3, 4, 2).reshape(h * n, 1, t)
+        ak = _t(attn_keep).to(device=a.device, dtype=a.dtype).permute(0, 1, 3, 4, 2).reshape(h * n, 1, t)
         a = a * ak / (1.0 - attn_drop_p)
     attn = a.view(h, b, hh, ww, t).permute(0, 1, 4, 2, 3).contiguous()  # :490-493
     if attn_only:
@@ -115,7 +126,7 @@ def ltae_forward_torch(cfg, params: Dict, x, positions=None, pad_mask=None, attn
                          False, 0.1, 1e-5)  # :445 (eval)
     y = F.relu(y)  # :447
     if training and mlp_keep is not None:  # :448 nn.Dropout(0.2)
-        mk = _t(mlp_keep).to(torch.float32).permute(0, 2, 3, 1).reshape(n, -1)
+        mk = _t(mlp_keep).to(device=y.device, dtype=y.dtype).permute(0, 2, 3, 1).reshape(n, -1)
         y = y * mk / (1.0 - mlp_drop_p)
     y = F.group_norm(y[:, :, None], h, p["out_norm.weight"], p["out_norm.bias"], 1e-5)[:, :, 0]  # :488
     out = y.view(b, hh, ww, -1).permute(0, 3, 1, 2).contiguous()  # :494
@@ -125,17 +136,17 @@ def ltae_forward_torch(cfg, params: Dict, x, positions=None, pad_mask=None, attn
 
 
 def temporal_aggregator_torch(x, pad_mask=None, attn_mask=None, mode: str = "att_group"):
-    """``TemporalAggregator(mode).forward`` on CPU tensors (temporal_aggregator.py:14-77)."""
-    x = _t(x).float()
+    """``TemporalAggregator(mode).forward`` (temporal_aggregator.py:14-77) on x's device and precision."""
+    x = _real(x)
     b, t, c, hh, ww = x.shape
     keep = None
     if pad_mask is not None and bool(_t(pad_mask).any()):
-        keep = (~_t(pad_mask).bool()).float()
+        keep = (~_t(pad_mask).to(x.device).bool()).to(x.dtype)
     if mode == "mean":
         if keep is None:
             return x.mean(dim=1)
         return (x * keep[:, :, None, None, None]).sum(dim=1) / keep.sum(dim=1)[:, None, None, None]
-    attn = _t(attn_mask).float()
+    attn = _real(attn_mask)
     nh = attn.shape[0]
     if mode == "att_mean":
         a = F.interpolate(attn.mean(dim=0), size=(hh, ww), mode="bilinear", align_corners=False)

@@ -22,15 +22,19 @@ UNSUPPORTED = {"ltae_two_queries"}  # num_queries > 1: crashes in every shipped 
 def _run_ltae(cfg, inp, params, dtype=torch.float32, zero_padded=False):
     m = module_from_fixture(cfg, params)
     m.assume_zero_padded = zero_padded
+    rate = c2s.modules.ATTENTION_DROPOUT
     if cfg["train"]:
         m.train()
         c2s.modules.ATTENTION_DROPOUT = 0.0
         m.mlp[5].p = 0.0
     else:
         m.eval()
-    with torch.no_grad():
-        res = m(to_dev(inp["x"], dtype=dtype), batch_positions=to_dev(inp.get("positions")),
-                pad_mask=to_dev(inp.get("pad_mask")))
+    try:
+        with torch.no_grad():
+            res = m(to_dev(inp["x"], dtype=dtype), batch_positions=to_dev(inp.get("positions")),
+                    pad_mask=to_dev(inp.get("pad_mask")))
+    finally:
+        c2s.modules.ATTENTION_DROPOUT = rate  # a process-wide rate: later training-mode tests apply 0.1
     return m, res
 
 
