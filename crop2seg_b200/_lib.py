@@ -26,7 +26,8 @@ EXPORTS = (
     "c2s_abi_version", "c2s_last_error", "c2s_launch_count", "c2s_reset_launch_count", "c2s_last_kernel",
     "c2s_last_ltae_kernel", "c2s_set_option", "c2s_get_option",
     "c2s_agg_workspace_bytes", "c2s_agg_forward", "c2s_agg_backward_workspace_bytes", "c2s_agg_backward",
-    "c2s_agg_skipconv_workspace_bytes", "c2s_agg_skipconv_forward", "c2s_pad_mask",
+    "c2s_agg_skipconv_workspace_bytes", "c2s_agg_skipconv_forward", "c2s_agg_skipconv_backward_workspace_bytes",
+    "c2s_agg_skipconv_backward", "c2s_pad_mask",
     "c2s_ltae_workspace_bytes", "c2s_ltae_forward", "c2s_ltae_backward_workspace_bytes", "c2s_ltae_backward",
     "c2s_ltae_mlp_backward_workspace_bytes", "c2s_ltae_mlp_backward", "c2s_ltae_inconv_grad", "c2s_ltae_fold_backward",
     "c2s_ltae_rows_forward",
@@ -45,6 +46,13 @@ class AggDesc(ctypes.Structure):
 class SkipConvParams(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in ("conv_weight", "conv_bias", "bn_weight", "bn_bias", "bn_running_mean",
                                                "bn_running_var")] + [("bn_eps", ctypes.c_float)]
+
+
+SKIPCONV_BWD_IO_FIELDS = ("grad_x", "grad_attn", "grad_conv_weight", "grad_conv_bias", "grad_bn_weight", "grad_bn_bias")
+
+
+class SkipConvBwdIo(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_void_p) for n in SKIPCONV_BWD_IO_FIELDS]
 
 
 class TileDesc(ctypes.Structure):
@@ -152,6 +160,11 @@ def load() -> ctypes.CDLL:
         lib.c2s_agg_skipconv_forward.restype = i32
         lib.c2s_agg_skipconv_forward.argtypes = [ctypes.POINTER(AggDesc), vp, vp, vp, ctypes.POINTER(SkipConvParams), vp,
                                                  vp, sz, vp]
+        lib.c2s_agg_skipconv_backward_workspace_bytes.restype = sz
+        lib.c2s_agg_skipconv_backward_workspace_bytes.argtypes = [ctypes.POINTER(AggDesc)]
+        lib.c2s_agg_skipconv_backward.restype = i32
+        lib.c2s_agg_skipconv_backward.argtypes = [ctypes.POINTER(AggDesc), vp, vp, vp, ctypes.POINTER(SkipConvParams), vp,
+                                                  vp, ctypes.POINTER(SkipConvBwdIo), vp, sz, vp]
         lib.c2s_ltae_rows_forward.restype = i32
         lib.c2s_ltae_rows_forward.argtypes = [vp, vp, vp, i32, vp, vp]
         lib.c2s_ltae_inconv_grad.restype = i32

@@ -2,6 +2,9 @@
 
 * ``AggregateFunction``: forward AND backward are CUDA kernels (``c2s_agg_forward`` / ``c2s_agg_backward``) --
   the aggregations move 97.7 % of the hot path's bytes.
+* ``AggregateSkipConvFunction``: the aggregation fused with the decoder's skip convolution, BatchNorm frozen (running
+  statistics); forward ``c2s_agg_skipconv_forward``, backward ``c2s_agg_skipconv_backward``, which recomputes the skip
+  map on chip from x, so only the output is saved besides the inputs.
 * ``LtaeFunction``: the forward is the fused CUDA kernel (train-mode BatchNorm statistics and injected dropout masks
   included).  The backward has three stages:
     M  ``c2s_ltae_mlp_backward`` (CUDA, ``csrc/c2s_ltae_mlp_bwd.cu``): the rows after the attention (MLP Linear,
@@ -40,6 +43,30 @@ class AggregateFunction(torch.autograd.Function):
         gx, gattn = ops.temporal_aggregate_backward(x, pad, attn, grad_out, ctx.mode, need_x=ctx.needs_input_grad[0],
                                                     need_attn=ctx.needs_input_grad[1])
         return gx, gattn, None, None
+
+
+class AggregateSkipConvFunction(torch.autograd.Function):
+    """apply(x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_running_mean, bn_running_var, bn_eps)"""
+
+    @staticmethod
+    def forward(ctx, x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_running_mean, bn_running_var, bn_eps):
+        out = ops.temporal_aggregate_skip_conv_forward(x, pad_mask, attn, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                       bn_running_mean, bn_running_var, bn_eps)
+        ctx.bn_eps = bn_eps
+        ctx.save_for_backward(x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_running_mean,
+                              bn_running_var, out)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        x, attn, pad, cw, cb, bw, bb, rm, rv, out = ctx.saved_tensors
+        need = [ctx.needs_input_grad[i] for i in (0, 1, 3, 4, 5, 6)]
+        gx, gattn, gcw, gcb, gbw, gbb = ops.temporal_aggregate_skip_conv_backward(
+            x, pad, attn, cw, cb, bw, bb, rm, rv, ctx.bn_eps, out, grad_out, need=need)
+
+        def cast(g, p):
+            return None if g is None else g.to(p.dtype)
+        return (gx, cast(gattn, attn), None, cast(gcw, cw), cast(gcb, cb), cast(gbw, bw), cast(gbb, bb), None, None, None)
 
 
 # ------------------------------------------------------------------------------------------------------------

@@ -396,8 +396,9 @@ class TemporalAggregator(nn.Module):
         """``skip_conv(self(x, pad_mask, attn_mask))`` in one kernel, for the decoder's ``UpConvBlock.skip_conv`` =
         ``Sequential(Conv2d(d, d, 1), BatchNorm2d(d), ReLU())`` (conv.py:378-382; SURVEY.md section 8f, rank 1).
 
-        Inference only (``skip_conv`` in eval mode: running statistics); ``att_group``, bf16 features with 64 channels.
-        A maintainer replaces ``self.up_blocks[i](out, skip)`` by the block's own forward with the already-convolved
+        ``skip_conv`` in eval mode (running statistics); ``att_group``, bf16 features with 64 channels.  Differentiable
+        w.r.t. x, attn_mask and the convolution / BatchNorm affine parameters with the BatchNorm frozen (fine-tuning
+        with the decoder's BatchNorm in eval mode); batch statistics are not served.  A maintainer replaces ``self.up_blocks[i](out, skip)`` by the block's own forward with the already-convolved
         skip (INTEGRATION.md, "Fused skip convolution").
         """
         if self.mode != "att_group":

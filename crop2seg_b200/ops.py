@@ -131,21 +131,48 @@ def temporal_aggregate_skip_conv(x: torch.Tensor, pad_mask: Optional[torch.Tenso
                                  bn_weight: Optional[torch.Tensor], bn_bias: Optional[torch.Tensor],
                                  bn_running_mean: torch.Tensor, bn_running_var: torch.Tensor, bn_eps: float = 1e-5
                                  ) -> torch.Tensor:
-    """``relu(BatchNorm2d_eval(Conv2d_1x1(TemporalAggregator('att_group')(x, pad_mask, attn_mask))))`` in one kernel:
-    the aggregation of utae.py:225-227 followed by ``UpConvBlock.skip_conv`` (conv.py:378-382, 408), the skip map never
-    leaving the chip (``c2s_agg_skipconv_forward``).  Inference only; bf16 x[B,T,64,H,W], 16 heads, x2/x4/x8
-    up-sampling, H*W % 128 == 0 -- other shapes raise (use the two modules separately)."""
+    """``relu(BatchNorm2d_eval(Conv2d_1x1(TemporalAggregator('att_group')(x, pad_mask, attn_mask))))`` in one kernel,
+    differentiable w.r.t. x, attn_mask, the convolution and the BatchNorm affine (both directions are CUDA kernels;
+    the BatchNorm stays frozen: running statistics)."""
+    tensors = (x, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias)
+    if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors):
+        from .autograd import AggregateSkipConvFunction
+        return AggregateSkipConvFunction.apply(x, attn_mask, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                               bn_running_mean, bn_running_var, bn_eps)
+    return temporal_aggregate_skip_conv_forward(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                bn_running_mean, bn_running_var, bn_eps)
+
+
+def _skipconv_inputs(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_running_mean, bn_running_var,
+                     bn_eps, keep):
+    """Checked inputs of the fused skip convolution: x, attention, uint8 pad mask, ``c2s_agg_desc`` and
+    ``c2s_skipconv_params`` (the float32 parameter copies it points to are kept alive in ``keep``)."""
     x, attn, desc = _agg_inputs(x, attn_mask, "att_group")
     b, t, c, h, w = x.shape
     if tuple(conv_weight.shape[:2]) != (c, c) or conv_weight.numel() != c * c:
         raise RuntimeError(f"crop2seg_b200: skip convolution must be 1x1 {c}->{c}, got {tuple(conv_weight.shape)}")
     pad = _mask_u8(pad_mask, (b, t), "pad_mask", x.device)
-    keep = []
     params = _lib.SkipConvParams(
         conv_weight=_f32(conv_weight, x.device, keep), conv_bias=_f32(conv_bias, x.device, keep),
         bn_weight=_f32(bn_weight, x.device, keep), bn_bias=_f32(bn_bias, x.device, keep),
         bn_running_mean=_f32(bn_running_mean, x.device, keep), bn_running_var=_f32(bn_running_var, x.device, keep),
         bn_eps=float(bn_eps))
+    return x, attn, pad, desc, params
+
+
+def temporal_aggregate_skip_conv_forward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: torch.Tensor,
+                                         conv_weight: torch.Tensor, conv_bias: Optional[torch.Tensor],
+                                         bn_weight: Optional[torch.Tensor], bn_bias: Optional[torch.Tensor],
+                                         bn_running_mean: torch.Tensor, bn_running_var: torch.Tensor, bn_eps: float = 1e-5
+                                         ) -> torch.Tensor:
+    """``relu(BatchNorm2d_eval(Conv2d_1x1(TemporalAggregator('att_group')(x, pad_mask, attn_mask))))`` in one kernel:
+    the aggregation of utae.py:225-227 followed by ``UpConvBlock.skip_conv`` (conv.py:378-382, 408), the skip map never
+    leaving the chip (``c2s_agg_skipconv_forward``).  Running statistics; bf16 x[B,T,64,H,W], 16 heads, x2/x4/x8
+    up-sampling, H*W % 128 == 0 -- other shapes raise (use the two modules separately)."""
+    keep = []
+    x, attn, pad, desc, params = _skipconv_inputs(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                  bn_running_mean, bn_running_var, bn_eps, keep)
+    b, t, c, h, w = x.shape
     out = torch.empty((b, c, h, w), dtype=x.dtype, device=x.device)
     lib = _lib.load()
     with torch.cuda.device(x.device):
@@ -156,6 +183,45 @@ def temporal_aggregate_skip_conv(x: torch.Tensor, pad_mask: Optional[torch.Tenso
                                               _stream(x.device))
     _lib.check(status, "c2s_agg_skipconv_forward")
     return out
+
+
+def temporal_aggregate_skip_conv_backward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: torch.Tensor,
+                                          conv_weight: torch.Tensor, conv_bias: Optional[torch.Tensor],
+                                          bn_weight: Optional[torch.Tensor], bn_bias: Optional[torch.Tensor],
+                                          bn_running_mean: torch.Tensor, bn_running_var: torch.Tensor, bn_eps: float,
+                                          out: torch.Tensor, grad_out: torch.Tensor, need=(True,) * 6
+                                          ) -> Tuple[Optional[torch.Tensor], ...]:
+    """Backward of :func:`temporal_aggregate_skip_conv_forward` (``c2s_agg_skipconv_backward``) from its output ``out``:
+    ``(grad_x, grad_attn, grad_conv_weight, grad_conv_bias, grad_bn_weight, grad_bn_bias)``, each None where ``need``
+    (same order) says so or the parameter is None.  grad_x is bf16 like x, the others float32; grad_attn is accumulated
+    with float atomics (as in :func:`temporal_aggregate_backward`), the parameter gradients are deterministic."""
+    keep = []
+    x, attn, pad, desc, params = _skipconv_inputs(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                  bn_running_mean, bn_running_var, bn_eps, keep)
+    b, t, c, h, w = x.shape
+    if tuple(out.shape) != (b, c, h, w) or tuple(grad_out.shape) != (b, c, h, w):
+        raise RuntimeError(f"crop2seg_b200: out {tuple(out.shape)} / grad_out {tuple(grad_out.shape)} must be {(b, c, h, w)}")
+    o = out.to(dtype=x.dtype).contiguous()
+    gout = grad_out.to(dtype=x.dtype).contiguous()
+    f32 = dict(dtype=torch.float32, device=x.device)
+    want = [bool(n) for n in need]
+    want[3] = want[3] and conv_bias is not None
+    want[4] = want[4] and bn_weight is not None
+    want[5] = want[5] and bn_bias is not None
+    res = [torch.empty_like(x) if want[0] else None, torch.zeros_like(attn) if want[1] else None,
+           torch.empty((c, c), **f32) if want[2] else None] + [torch.empty(c, **f32) if k else None for k in want[3:]]
+    io = _lib.SkipConvBwdIo(**{k: _ptr(r) for k, r in zip(_lib.SKIPCONV_BWD_IO_FIELDS, res)})
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        ws_bytes = lib.c2s_agg_skipconv_backward_workspace_bytes(ctypes.byref(desc))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        status = lib.c2s_agg_skipconv_backward(ctypes.byref(desc), x.data_ptr(), attn.data_ptr(), _ptr(pad),
+                                               ctypes.byref(params), o.data_ptr(), gout.data_ptr(), ctypes.byref(io),
+                                               ws.data_ptr(), ws_bytes, _stream(x.device))
+    _lib.check(status, "c2s_agg_skipconv_backward")
+    if res[2] is not None:
+        res[2] = res[2].view(conv_weight.shape)
+    return tuple(res)
 
 
 def temporal_aggregate_backward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: Optional[torch.Tensor],

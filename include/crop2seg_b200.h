@@ -85,8 +85,8 @@ int c2s_agg_forward(const c2s_agg_desc* desc, const void* x, const float* attn,
 /* TemporalAggregator(att_group) fused with the decoder's skip convolution (SURVEY.md section 8f, rank 1):
  *   out[B,C,H,W] = relu( BatchNorm2d_eval( Conv2d_1x1( aggregate(x, attn, pad) ) ) )
  * = UpConvBlock.skip_conv (conv.py:378-382, applied at conv.py:408) on the skip map of utae.py:225-229, without the
- * skip map being written to and re-read from HBM.  Inference only (running statistics).  Serves what the shipped
- * models use: att_group, bfloat16, C = 64, 16 heads, x2/x4/x8 up-sampling, H*W % 128 == 0; anything else returns
+ * skip map being written to and re-read from HBM.  Running statistics (c2s_agg_skipconv_backward below).  Serves what
+ * the shipped models use: att_group, bfloat16, C = 64, 16 heads, x2/x4/x8 up-sampling, H*W % 128 == 0; anything else returns
  * C2S_ERR_UNSUPPORTED (run c2s_agg_forward and the convolution separately). */
 typedef struct c2s_skipconv_params {
   const float* conv_weight;      /* skip_conv.0.weight [C,C,1,1]                               */
@@ -101,6 +101,25 @@ size_t c2s_agg_skipconv_workspace_bytes(const c2s_agg_desc* desc);
 int c2s_agg_skipconv_forward(const c2s_agg_desc* desc, const void* x, const float* attn, const uint8_t* pad_mask,
                              const c2s_skipconv_params* params, void* out, void* workspace, size_t workspace_bytes,
                              void* stream);
+
+/* Backward of c2s_agg_skipconv_forward with the BatchNorm frozen (eval mode: running statistics), i.e. what autograd
+ * derives from relu(BatchNorm2d_eval(Conv2d_1x1(aggregate(x, attn, pad)))) with the skip map rounded to bf16 as the
+ * forward rounds it.  `out` is the forward's output (its ReLU decision), grad_out [B,C,H,W] bf16.  x is read once; the
+ * skip map is recomputed on chip and never written.  Same shapes as the forward; anything else returns
+ * C2S_ERR_BAD_ARGUMENT.  Every output pointer may be NULL (that gradient is skipped). */
+typedef struct c2s_skipconv_bwd_io {
+  void* grad_x;             /* out [B,T,C,H,W] bf16, exactly 0 on padded frames                                         */
+  float* grad_attn;         /* acc [16,B,T,ha,wa], ZERO-FILLED by the caller; float atomics as in c2s_agg_backward      */
+  float* grad_conv_weight;  /* out [C,C] (skip_conv.0.weight)        deterministic: fixed-order reduction, no atomics   */
+  float* grad_conv_bias;    /* out [C]   (skip_conv.0.bias)                                                              */
+  float* grad_bn_weight;    /* out [C]   (skip_conv.1.weight)                                                            */
+  float* grad_bn_bias;      /* out [C]   (skip_conv.1.bias)                                                              */
+} c2s_skipconv_bwd_io;
+/* Scratch bytes: prepared weights plus one partial of the parameter gradients per (sample, 128-pixel block). */
+size_t c2s_agg_skipconv_backward_workspace_bytes(const c2s_agg_desc* desc);
+int c2s_agg_skipconv_backward(const c2s_agg_desc* desc, const void* x, const float* attn, const uint8_t* pad_mask,
+                              const c2s_skipconv_params* params, const void* out, const void* grad_out,
+                              const c2s_skipconv_bwd_io* io, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Backward of TemporalAggregator.forward (what autograd derives from temporal_aggregator.py:14-77):
  *   grad_x[b,t,c]        = resize(attn)[c // (C/n_heads), b, t] * (pad ? 0 : 1) * grad_out[b,c]      (x's dtype)
