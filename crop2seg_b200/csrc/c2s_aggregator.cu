@@ -23,7 +23,6 @@ namespace c2s {
 namespace {
 
 constexpr int kAggThreads = 256;
-constexpr int kAggMaxT = 1024;  // frames per series the frame list in shared memory can hold
 
 struct AggArgs {
   const void* x;
@@ -544,286 +543,6 @@ size_t attn_elems(const c2s_agg_desc* d, int heads, int h, int w) {
 
 // The AvgPool2d branch is taken when x is not taller than the attention map is wide
 // (temporal_aggregator.py:26-29 compares x.shape[-2] with the attention width).
-// ---------------------------------------------------------------------------------------------------
-// Aggregation fused with the decoder's skip convolution (SURVEY.md section 8f, rank 1):
-//   y[b,o,p] = relu( scale[o] * sum_c W[o,c] * skip[b,c,p] + shift[o] ),   skip = TemporalAggregator(att_group)
-// which is UpConvBlock.skip_conv = Conv2d(d,d,1) -> BatchNorm2d (eval) -> ReLU (conv.py:378-382) applied to the
-// aggregator's output (utae.py:225-229) without the skip map ever visiting HBM.  One CTA = one sample x ALL 64
-// channels x 128 pixels: the producer issues ONE 3-D tensor-map copy per valid frame (box = 128 pixels x 64 channels
-// x 1 frame, 16 KB per stage; 64 separate 256-byte bulk copies per frame were issue-bound at a third of the HBM
-// rate), the consumers accumulate 4 channels x 8 pixels each exactly like agg_pipe_kernel, then the
-// [64 x 128] skip tile goes to shared memory as bf16 (the value the unfused bf16 path would have stored) and the
-// 1x1 convolution runs as mma.sync m16n8k16 with W split into bf16 hi + lo (two products, fp32 accumulation).
-// ---------------------------------------------------------------------------------------------------
-constexpr int kScC = 64;            // channels of the skip map (= in and out channels of the 1x1 convolution)
-constexpr int kScPB = 128;          // pixels per CTA
-constexpr int kScConsumers = 256;   // thread = (head, 8-pixel vector)
-constexpr int kScStageBytes = kScC * kScPB * 2;
-constexpr int kScTileStride = kScPB * 2 + 16;  // bytes per channel row of the epilogue tile (padded: ldmatrix conflict-free)
-
-struct SkipConvArgs {
-  AggArgs a;
-  const uint4* wfrag;  // [hi|lo][m-tile 4][k-step 4][lane 32] A fragments of W (bf16 pairs)
-  const float* scale;  // [64]  gamma / sqrt(var + eps)
-  const float* shift;  // [64]  (conv_bias - mean) * scale + beta
-  int n_stages;
-  int tap_floats;      // per head and stage: staged attention rows of the pixel block (0: taps from global memory)
-};
-
-// W[o][c] fp32 -> mma.sync A fragments (row-major 16x16 tiles), bf16 hi and the bf16 residual
-// plus (third block) the scale / shift of conv bias + eval BatchNorm
-__global__ void skipconv_prep_kernel(const float* __restrict__ w, uint4* __restrict__ frag, const float* conv_bias,
-                                     const float* bn_w, const float* bn_b, const float* bn_mean, const float* bn_var,
-                                     float eps, float* scale, float* shift) {
-  if (blockIdx.x == 2) {
-    const int o = threadIdx.x;
-    if (o < kScC) {
-      const float sc = (bn_w ? bn_w[o] : 1.f) / sqrtf(bn_var[o] + eps);
-      scale[o] = sc;
-      shift[o] = ((conv_bias ? conv_bias[o] : 0.f) - bn_mean[o]) * sc + (bn_b ? bn_b[o] : 0.f);
-    }
-    return;
-  }
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;  // (mt, ks, lane)
-  if (idx >= 4 * 4 * 32) return;
-  const int lane = idx & 31, ks = (idx >> 5) & 3, mt = idx >> 7;
-  const int r0 = mt * 16 + (lane >> 2), c0 = ks * 16 + (lane & 3) * 2;
-  uint32_t hi[4], lo[4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {  // a0:(r, c) a1:(r+8, c) a2:(r, c+8) a3:(r+8, c+8)
-    const int r = r0 + (q & 1) * 8, c = c0 + (q >> 1) * 8;
-    const float v0 = w[r * kScC + c], v1 = w[r * kScC + c + 1];
-    const __nv_bfloat16 h0 = __float2bfloat16_rn(v0), h1 = __float2bfloat16_rn(v1);
-    hi[q] = Elem<__nv_bfloat16>::pack2(__bfloat162float(h0), __bfloat162float(h1));
-    lo[q] = Elem<__nv_bfloat16>::pack2(v0 - __bfloat162float(h0), v1 - __bfloat162float(h1));
-  }
-  frag[idx] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-  frag[4 * 4 * 32 + idx] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-}
-
-template <int S, bool TAPS>
-__global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(const __grid_constant__ CUtensorMap map_x,
-                                                                             const __grid_constant__ CUtensorMap map_att,
-                                                                             const SkipConvArgs k) {
-  using T = __nv_bfloat16;
-  constexpr int VEC = 8;
-  constexpr int NCOL = Window<VEC, S>::kCols;
-  const AggArgs& a = k.a;
-  extern __shared__ __align__(128) unsigned char pipe_smem[];  // stages, then the epilogue tile
-  __shared__ short frames[kAggMaxT];
-  __shared__ int n_frames_s;
-  __shared__ __align__(8) unsigned long long bars[2 * 16];
-
-  const int b = blockIdx.y, pblk = blockIdx.x;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int n_cwarps = kScConsumers / 32;
-  const int n_stages = k.n_stages;
-  constexpr bool taps = TAPS;
-  const uint32_t stage_stride = kScStageBytes + 16u * k.tap_floats * 4u;
-  int r_lo = 0, n_rows_att = 0;  // attention rows [r_lo, r_lo + n_rows_att) feed this pixel block (as in agg_pipe_kernel)
-  if (taps) {
-    int i0, i1;
-    float l1;
-    source_index(a.sy, (pblk * kScPB) / a.W, a.ha, i0, i1, l1);
-    r_lo = i0;
-    source_index(a.sy, (pblk * kScPB + kScPB - 1) / a.W, a.ha, i0, i1, l1);
-    n_rows_att = i1 - r_lo + 1;
-  }
-
-  if (threadIdx.x < 32) {
-    int count = 0;
-    for (int base = 0; base < a.T; base += 32) {
-      const int t = base + threadIdx.x;
-      const bool valid = t < a.T && (a.pad == nullptr || a.pad[b * a.T + t] == 0);
-      const unsigned m = __ballot_sync(0xffffffffu, valid);
-      if (valid) frames[count + __popc(m & ((1u << threadIdx.x) - 1u))] = static_cast<short>(t);
-      count += __popc(m);
-    }
-    if (threadIdx.x == 0) {
-      n_frames_s = count;
-      for (int s = 0; s < n_stages; ++s) {
-        mbar_init(s32(&bars[s]), 1);
-        mbar_init(s32(&bars[16 + s]), n_cwarps);
-      }
-      fence_mbarrier_init();
-    }
-  }
-  __syncthreads();
-  const int n_frames = n_frames_s;
-  const uint32_t stage0 = s32(pipe_smem);
-
-  if (warp == n_cwarps) {  // ---- producer: one box {128 pixels, 64 channels, 1 frame} per valid frame and, with staged
-    // taps, one box {tap_floats of the map from row r_lo, 1 frame, 16 heads} of the attention (16 separate bulk copies
-    // of 128-256 bytes per frame were measured: issue-bound, slower than the global-memory taps)
-    if (lane == 0) {
-      const uint32_t tap_bytes = taps ? 16u * k.tap_floats * 4u : 0u;
-      for (int i = 0; i < n_frames; ++i) {
-        const int s = i % n_stages, round = i / n_stages;
-        if (round > 0) mbar_wait(s32(&bars[16 + s]), (round - 1) & 1);
-        const uint32_t full = s32(&bars[s]);
-        mbar_expect_tx(full, kScStageBytes + tap_bytes);
-        tma_load_3d(stage0 + s * stage_stride, &map_x, pblk * kScPB, 0, b * a.T + frames[i], full);
-        if (taps) tma_load_3d(stage0 + s * stage_stride + kScStageBytes, &map_att, r_lo * a.wa, b * a.T + frames[i], 0, full);
-      }
-    }
-    return;
-  }
-
-  // ---- consumers: thread = (attention head, 8-pixel vector) -----------------------------------------------------------
-  const int head = threadIdx.x >> 4, pv = threadIdx.x & 15;
-  const int p0 = pblk * kScPB + pv * VEC;
-  const int y = p0 / a.W;
-  const int x0 = p0 - y * a.W;
-  int iy0, iy1;
-  float ly1;
-  source_index(a.sy, y, a.ha, iy0, iy1, ly1);
-  const float ly0 = 1.f - ly1;
-  const int row0 = iy0 * a.wa, row1 = iy1 * a.wa;
-  float lx1[VEC];
-#pragma unroll
-  for (int j = 0; j < VEC; ++j) {
-    int i0, i1;
-    source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
-  }
-  int col[NCOL];
-  {
-    int cmin = x0 / S - 1;
-    if constexpr (VEC < S) cmin += ((x0 % S) >= S / 2) ? 1 : 0;
-#pragma unroll
-    for (int j = 0; j < NCOL; ++j) {
-      int cj = cmin + j;
-      cj = cj < 0 ? 0 : cj;
-      col[j] = cj > a.wa - 1 ? a.wa - 1 : cj;
-    }
-  }
-  const int amap = a.ha * a.wa;
-  const float* ab = a.attn + (static_cast<size_t>(head) * a.B + b) * a.T * amap;
-
-  float acc[4][VEC];
-#pragma unroll
-  for (int c = 0; c < 4; ++c)
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) acc[c][j] = 0.f;
-
-  float top_n[NCOL], bot_n[NCOL];
-  const int trow0 = (iy0 - r_lo) * a.wa, trow1 = (iy1 - r_lo) * a.wa;  // staged taps: rows inside the slice
-  if (!taps && n_frames > 0) {
-    const float* ap = ab + static_cast<size_t>(frames[0]) * amap;
-#pragma unroll
-    for (int j = 0; j < NCOL; ++j) top_n[j] = __ldg(ap + row0 + col[j]), bot_n[j] = __ldg(ap + row1 + col[j]);
-  }
-  const uint32_t my_off = (head * 4) * (kScPB * 2) + pv * 16;
-  for (int i = 0; i < n_frames; ++i) {
-    float r[NCOL];
-    if (!taps) {
-#pragma unroll
-      for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, bot_n[j], ly0 * top_n[j]);
-      if (i + 1 < n_frames) {
-        const float* ap = ab + static_cast<size_t>(frames[i + 1]) * amap;
-#pragma unroll
-        for (int j = 0; j < NCOL; ++j) top_n[j] = __ldg(ap + row0 + col[j]), bot_n[j] = __ldg(ap + row1 + col[j]);
-      }
-    }
-    const int s = i % n_stages;
-    mbar_wait(s32(&bars[s]), (i / n_stages) & 1);
-    uint4 xv[4];
-    const uint32_t base = stage0 + s * stage_stride + my_off;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) xv[c] = lds_v4(base + c * (kScPB * 2));
-    if (taps) {
-      const float* tp = reinterpret_cast<const float*>(pipe_smem + s * stage_stride + kScStageBytes) + head * k.tap_floats;
-#pragma unroll
-      for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
-    }
-    fence_proxy_async();  // the stage's shared loads before the producer's next bulk copy into it
-    __syncwarp();
-    if (lane == 0) mbar_arrive(s32(&bars[16 + s]));
-
-    float w[VEC];
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) {
-      const int i0w = (VEC >= S) ? (j / S + ((j % S) < S / 2 ? 0 : 1)) : 0;
-      w[j] = fmaf(lx1[j], r[i0w + 1], (1.f - lx1[j]) * r[i0w]);
-    }
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      float f[VEC];
-      Elem<T>::unpack(xv[c], f);
-#pragma unroll
-      for (int j = 0; j < VEC; ++j) acc[c][j] = fmaf(w[j], f[j], acc[c][j]);
-    }
-  }
-
-  // ---- epilogue: skip tile [64 channels][128 pixels] bf16 -> shared memory, 1x1 convolution on the tensor cores -------
-  const uint32_t tile = stage0 + n_stages * stage_stride;
-#pragma unroll
-  for (int c = 0; c < 4; ++c) {
-    const uint4 v = Elem<T>::pack(acc[c]);
-    asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(tile + (head * 4 + c) * kScTileStride + pv * 16), "r"(v.x),
-                 "r"(v.y), "r"(v.z), "r"(v.w)
-                 : "memory");
-  }
-  asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");  // the producer warp has left; consumers only
-
-  // warp w: pixels [16 w, 16 w + 16) = two n-tiles; all four m-tiles of output channels; K = 64 channels in 4 steps
-  float d[4][2][4];
-#pragma unroll
-  for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 2; ++nt)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) d[mt][nt][e] = 0.f;
-#pragma unroll
-  for (int ks = 0; ks < 4; ++ks) {
-    // B fragments: ldmatrix.x4.trans of the four 8x8 blocks (k 0-7 | 8-15) x (n 0-7 | 8-15) of this k-step
-    const int mrow = ks * 16 + (lane & 7) + ((lane >> 3) & 1) * 8;  // channel row this lane addresses
-    const int ncol = warp * 16 + (lane >> 4) * 8;                   // first pixel of the 8x8 block
-    uint32_t bf[4];
-    ldsm_x4_trans(bf, tile + mrow * kScTileStride + ncol * 2);
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt) {
-      const uint4 h4 = __ldg(k.wfrag + (mt * 4 + ks) * 32 + lane);
-      const uint4 l4 = __ldg(k.wfrag + 4 * 4 * 32 + (mt * 4 + ks) * 32 + lane);
-      const uint32_t ah[4] = {h4.x, h4.y, h4.z, h4.w}, al[4] = {l4.x, l4.y, l4.z, l4.w};
-#pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        mma_bf16(d[mt][nt], ah, bf[2 * nt], bf[2 * nt + 1]);
-        mma_bf16(d[mt][nt], al, bf[2 * nt], bf[2 * nt + 1]);
-      }
-    }
-  }
-  // D fragment: rows lane/4 and lane/4 + 8 of the m-tile, columns 2 (lane % 4), +1 of the n-tile
-  T* op = static_cast<T*>(a.out) + static_cast<size_t>(b) * kScC * a.hw + static_cast<size_t>(pblk) * kScPB + warp * 16 + (lane & 3) * 2;
-#pragma unroll
-  for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-    for (int hrow = 0; hrow < 2; ++hrow) {
-      const int o = mt * 16 + (lane >> 2) + hrow * 8;
-      const float sc = __ldg(k.scale + o), sh = __ldg(k.shift + o);
-#pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        const float v0 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2], sh), 0.f), v1 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2 + 1], sh), 0.f);
-        *reinterpret_cast<uint32_t*>(op + static_cast<size_t>(o) * a.hw + nt * 8) = Elem<T>::pack2(v0, v1);
-      }
-    }
-}
-
-template <int S, bool TAPS>
-int launch_skipconv_t(const CUtensorMap& map_x, const CUtensorMap& map_att, const SkipConvArgs& k, cudaStream_t stream, const char* name) {
-  const size_t smem = static_cast<size_t>(k.n_stages) * (kScStageBytes + 16 * k.tap_floats * 4) + kScC * kScTileStride;
-  C2S_SMEM_ATTR((agg_skipconv_kernel<S, TAPS>), 227 * 1024);  // once per instantiation and device (smem varies per call)
-  dim3 grid(k.a.hw / kScPB, k.a.B);
-  agg_skipconv_kernel<S, TAPS><<<grid, kScConsumers + 32, smem, stream>>>(map_x, map_att, k);
-  C2S_LAUNCH_CHECK(name);
-  return C2S_OK;
-}
-
-template <int S>
-int launch_skipconv(const CUtensorMap& map_x, const CUtensorMap& map_att, const SkipConvArgs& k, cudaStream_t stream, const char* name) {
-  return k.tap_floats > 0 ? launch_skipconv_t<S, true>(map_x, map_att, k, stream, name)
-                          : launch_skipconv_t<S, false>(map_x, map_att, k, stream, name);
-}
-
 bool uses_pool(const c2s_agg_desc* d) { return d->mode == C2S_AGG_ATT_GROUP && !(d->H > d->wa); }
 
 }  // namespace
@@ -952,87 +671,6 @@ int c2s_agg_forward(const c2s_agg_desc* d, const void* x, const float* attn, con
                     : launch_cpt<__nv_bfloat16, 1>(a, cpt, scale_class, stream);
   }
   return vec == 4 ? launch_cpt<float, 4>(a, cpt, scale_class, stream) : launch_cpt<float, 1>(a, cpt, scale_class, stream);
-}
-
-
-size_t c2s_agg_skipconv_workspace_bytes(const c2s_agg_desc* d) {
-  (void)d;
-  return 2 * 4 * 4 * 32 * sizeof(uint4) + 2 * c2s::kScC * sizeof(float);  // W fragments (hi, lo), scale, shift
-}
-
-int c2s_agg_skipconv_forward(const c2s_agg_desc* d, const void* x, const float* attn, const uint8_t* pad_mask,
-                             const c2s_skipconv_params* p, void* out, void* workspace, size_t workspace_bytes,
-                             void* stream_ptr) {
-  using namespace c2s;
-  C2S_CHECK_ARG(d != nullptr && p != nullptr, "c2s_agg_skipconv_forward: desc/params is NULL");
-  C2S_CHECK_ARG(x != nullptr && out != nullptr && attn != nullptr, "c2s_agg_skipconv_forward: x/attn/out is NULL");
-  C2S_CHECK_ARG(p->conv_weight != nullptr && p->bn_running_mean != nullptr && p->bn_running_var != nullptr,
-                "c2s_agg_skipconv_forward: conv weight and BatchNorm running statistics are required");
-  C2S_CHECK_ARG(d->B > 0 && d->T > 0 && d->H > 0 && d->W > 0, "c2s_agg_skipconv_forward: non-positive dimension");
-  C2S_CHECK_ARG(workspace != nullptr && workspace_bytes >= c2s_agg_skipconv_workspace_bytes(d),
-                "c2s_agg_skipconv_forward: needs %zu workspace bytes", c2s_agg_skipconv_workspace_bytes(d));
-  C2S_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 16 == 0, "c2s_agg_skipconv_forward: workspace must be 16-byte aligned");
-  int scale_class = 0;
-  for (int s : {2, 4, 8})
-    if (d->H == s * d->ha && d->W == s * d->wa) scale_class = s;
-  const int hw = d->H * d->W;
-  if (d->mode != C2S_AGG_ATT_GROUP || d->dtype != C2S_BF16 || d->C != kScC || d->n_heads != 16 || scale_class == 0 ||
-      hw % kScPB != 0 || d->W % 8 != 0 || d->T > kAggMaxT || d->B > 65535 || reinterpret_cast<uintptr_t>(x) % 16 != 0 ||
-      reinterpret_cast<uintptr_t>(out) % 16 != 0)
-    C2S_UNSUPPORTED("c2s_agg_skipconv_forward: the fused path serves att_group, bf16, C=64, 16 heads, x2/x4/x8 up-sampling, "
-                    "H*W %% 128 == 0 (got mode %d dtype %d C %d heads %d %dx%d from %dx%d); run c2s_agg_forward and the "
-                    "convolution separately", d->mode, d->dtype, d->C, d->n_heads, d->H, d->W, d->ha, d->wa);
-  int status = check_device();
-  if (status != C2S_OK) return status;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
-
-  SkipConvArgs k{};
-  AggArgs& a = k.a;
-  a.x = x, a.pad = pad_mask, a.out = out, a.attn = attn;
-  a.B = d->B, a.T = d->T, a.C = d->C, a.H = d->H, a.W = d->W, a.hw = hw;
-  a.n_heads = d->n_heads, a.ha = d->ha, a.wa = d->wa, a.cpg = d->C / d->n_heads;
-  a.sy = static_cast<float>(d->ha) / static_cast<float>(d->H);
-  a.sx = static_cast<float>(d->wa) / static_cast<float>(d->W);
-  uint4* wfrag = static_cast<uint4*>(workspace);
-  float* scale = reinterpret_cast<float*>(wfrag + 2 * 4 * 4 * 32);
-  float* shift = scale + kScC;
-  skipconv_prep_kernel<<<3, 256, 0, stream>>>(p->conv_weight, wfrag, p->conv_bias, p->bn_weight, p->bn_bias,
-                                              p->bn_running_mean, p->bn_running_var, p->bn_eps, scale, shift);
-  C2S_LAUNCH_CHECK("skipconv_prep");
-  k.wfrag = wfrag, k.scale = scale, k.shift = shift;
-  k.n_stages = 4;
-  {  // staged attention rows: the rows a 128-pixel block can touch, per head (16-byte aligned slices of the map)
-    const int rows_out = (kScPB + d->W - 1) / d->W + 1;
-    int rows_att = rows_out / scale_class + 3;
-    rows_att = rows_att > d->ha ? d->ha : rows_att;
-    const int tap_floats = ((rows_att * d->wa + 3) / 4) * 4;
-    // x2: measured slower with staged taps here (0.151 vs 0.109 ms at 32 x 32), so that level keeps the global-memory taps
-    const bool taps = option(C2S_OPT_AGG_TAPS) == 0 && d->wa % 4 == 0 && reinterpret_cast<uintptr_t>(attn) % 16 == 0 &&
-                      tap_floats <= 256 && scale_class >= 4;
-    k.tap_floats = taps ? tap_floats : 0;
-  }
-  CUtensorMap map_x;  // x as [B*T][C][H*W] bf16; box = 128 pixels x 64 channels x 1 frame, dense in shared memory
-  const cuuint64_t dims[3] = {static_cast<cuuint64_t>(hw), static_cast<cuuint64_t>(kScC), static_cast<cuuint64_t>(d->B) * d->T};
-  const cuuint64_t strides[2] = {static_cast<cuuint64_t>(hw) * 2, static_cast<cuuint64_t>(kScC) * hw * 2};
-  const cuuint32_t box[3] = {kScPB, kScC, 1};
-  status = encode_tensor_map(&map_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
-                             CU_TENSOR_MAP_L2_PROMOTION_NONE, "skip features");
-  if (status != C2S_OK) return status;
-  CUtensorMap map_att = map_x;  // attention as [16 heads][B*T][ha*wa] fp32; box = tap_floats of one map x 1 frame x 16 heads
-  if (k.tap_floats > 0) {
-    const cuuint64_t amap = static_cast<cuuint64_t>(d->ha) * d->wa;
-    const cuuint64_t adims[3] = {amap, static_cast<cuuint64_t>(d->B) * d->T, 16};
-    const cuuint64_t astrides[2] = {amap * 4, static_cast<cuuint64_t>(d->B) * d->T * amap * 4};
-    const cuuint32_t abox[3] = {static_cast<cuuint32_t>(k.tap_floats), 1, 16};
-    status = encode_tensor_map(&map_att, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, attn, adims, astrides, abox,
-                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, "attention");
-    if (status != C2S_OK) return status;
-  }
-  switch (scale_class) {
-    case 2: return launch_skipconv<2>(map_x, map_att, k, stream, "agg_skipconv<x2>");
-    case 4: return launch_skipconv<4>(map_x, map_att, k, stream, "agg_skipconv<x4>");
-    default: return launch_skipconv<8>(map_x, map_att, k, stream, "agg_skipconv<x8>");
-  }
 }
 
 }  // extern "C"

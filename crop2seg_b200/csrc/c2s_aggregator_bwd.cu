@@ -576,489 +576,6 @@ __global__ void unpool_grad_kernel(const float* __restrict__ gpooled, float* __r
 
 bool bwd_uses_pool(const c2s_agg_desc* d) { return d->mode == C2S_AGG_ATT_GROUP && !(d->H > d->wa); }
 
-// ---------------------------------------------------------------------------------------------------
-// Backward of the aggregation fused with the skip convolution (agg_skipconv_kernel of c2s_aggregator.cu) with the
-// BatchNorm in eval mode, for one sample and pixel p (s = the bf16 skip map, z = W s + b, alpha = gamma / sqrt(var + eps)):
-//   g_y = grad_out * [out > 0]                      grad_s = W^T (alpha * g_y)
-//   grad_bn_bias = sum g_y   grad_bn_weight = sum g_y (z - mean) / sqrt(var + eps)
-//   grad_conv_bias = alpha * sum g_y                grad_conv_weight = alpha * sum_p g_y s^T
-// then the aggregator's backward with grad_out = grad_s.  One CTA = one sample x 64 channels x 128 pixels, as in the
-// forward.  Before any frame arrives grad_s is formed on the tensor cores from grad_out and out alone (the A operand is
-// (alpha W)^T as bf16 hi + lo; g_y is exact in bf16).  The valid frames then stream once through the TMA ring: the
-// consumers write grad_x, scatter the bilinear adjoint into grad_attn (as agg_backward_pipe_kernel) and re-accumulate s
-// with the forward's arithmetic in the forward's frame order, so the bf16 s is the forward's bit for bit.  After the
-// sweep, z = W s (hi + lo, the forward's products) gives the BatchNorm sums and g_y s^T the weight gradient; each CTA
-// writes its partials to the workspace and skipconv_bwd_finish_kernel reduces them in a fixed order (deterministic).
-// ---------------------------------------------------------------------------------------------------
-constexpr int kSbC = 64;                       // channels of the skip map (in and out channels of the 1x1 convolution)
-constexpr int kSbPB = 128;                     // pixels per CTA
-constexpr int kSbConsumers = 256;              // thread = (attention head, 8-pixel vector)
-constexpr int kSbStageBytes = kSbC * kSbPB * 2;
-constexpr int kSbTileStride = kSbPB * 2 + 16;  // bytes per channel row of a bf16 tile (padded: ldmatrix conflict-free)
-constexpr int kSbGsStride = kSbPB + 4;         // floats per channel row of the fp32 grad_s tile
-constexpr int kSbFrags = 4 * 4 * 32;           // uint4 A fragments of one 64 x 64 bf16 matrix (m-tile, k-step, lane)
-constexpr int kSbPartial = kSbC * kSbC + 2 * kSbC;  // floats per CTA: g_y s^T, sum g_y, sum g_y (z - mean)
-constexpr int kSbMaxStages = 6;  // one CTA per SM (the grad_s and s registers rule out two): 96 KB of x in flight
-
-struct SkipConvBwdArgs {
-  const float* attn;
-  const uint8_t* pad;
-  const __nv_bfloat16* out;
-  const __nv_bfloat16* gout;
-  __nv_bfloat16* gx;
-  float* gattn;
-  const uint4* wfrag;   // [hi|lo] A fragments of W            (z = W s)
-  const uint4* afrag;   // [hi|lo] A fragments of (alpha W)^T  (grad_s = (alpha W)^T g_y)
-  const float* zshift;  // [64] conv_bias - running_mean
-  float* partial;       // [CTAs][kSbPartial] or nullptr (no parameter gradient wanted)
-  int B, T, H, W, hw, ha, wa;
-  float sy, sx;
-  int tap_floats;       // per head and stage: staged attention rows of the pixel block (0: taps from global memory)
-  int n_stages;
-};
-
-// A fragments (row-major 16 x 16 tiles, mma.sync m16n8k16) of W and of (alpha W)^T, each as bf16 hi + bf16 residual,
-// in the order of skipconv_prep_kernel (c2s_aggregator.cu); block 2: the per-channel constants
-__global__ void skipconv_bwd_prep_kernel(const float* __restrict__ w, const float* conv_bias, const float* bn_w,
-                                         const float* bn_mean, const float* bn_var, float eps, uint4* __restrict__ wfrag,
-                                         uint4* __restrict__ afrag, float* alpha, float* inv_std, float* zshift) {
-  if (blockIdx.x == 2) {
-    const int o = threadIdx.x;
-    if (o < kSbC) {
-      const float is = 1.f / sqrtf(bn_var[o] + eps);
-      inv_std[o] = is;
-      alpha[o] = (bn_w ? bn_w[o] : 1.f) / sqrtf(bn_var[o] + eps);  // the forward's scale, same arithmetic
-      zshift[o] = (conv_bias ? conv_bias[o] : 0.f) - bn_mean[o];
-    }
-    return;
-  }
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;  // (mt, ks, lane)
-  if (idx >= kSbFrags) return;
-  const int lane = idx & 31, ks = (idx >> 5) & 3, mt = idx >> 7;
-  const int r0 = mt * 16 + (lane >> 2), c0 = ks * 16 + (lane & 3) * 2;
-  for (int which = 0; which < 2; ++which) {
-    uint32_t hi[4], lo[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {  // a0:(r, c) a1:(r+8, c) a2:(r, c+8) a3:(r+8, c+8)
-      const int r = r0 + (q & 1) * 8, c = c0 + (q >> 1) * 8;
-      float v0, v1;
-      if (which == 0) {
-        v0 = w[r * kSbC + c], v1 = w[r * kSbC + c + 1];
-      } else {  // (alpha W)^T [c_in = r][c_out = c]
-        const float a0 = (bn_w ? bn_w[c] : 1.f) / sqrtf(bn_var[c] + eps), a1 = (bn_w ? bn_w[c + 1] : 1.f) / sqrtf(bn_var[c + 1] + eps);
-        v0 = a0 * w[c * kSbC + r], v1 = a1 * w[(c + 1) * kSbC + r];
-      }
-      const __nv_bfloat16 h0 = __float2bfloat16_rn(v0), h1 = __float2bfloat16_rn(v1);
-      hi[q] = Elem<__nv_bfloat16>::pack2(__bfloat162float(h0), __bfloat162float(h1));
-      lo[q] = Elem<__nv_bfloat16>::pack2(v0 - __bfloat162float(h0), v1 - __bfloat162float(h1));
-    }
-    uint4* f = which == 0 ? wfrag : afrag;
-    f[idx] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-    f[kSbFrags + idx] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-  }
-}
-
-// [64 rows][128 pixels] = A[64 x 64] (hi + lo fragments) x tile[64 channels][128 pixels] (bf16, row stride kSbTileStride);
-// warp w: pixels [16 w, 16 w + 16).  D fragment: rows mt*16 + lane/4 (+8), pixels 16 w + 8 nt + 2 (lane % 4) (+1).
-__device__ __forceinline__ void skipconv_tile_mma(float (&d)[4][2][4], const uint4* frag, uint32_t tile, int warp, int lane) {
-#pragma unroll
-  for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 2; ++nt)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) d[mt][nt][e] = 0.f;
-#pragma unroll
-  for (int ks = 0; ks < 4; ++ks) {
-    const int mrow = ks * 16 + (lane & 7) + ((lane >> 3) & 1) * 8;
-    const int ncol = warp * 16 + (lane >> 4) * 8;
-    uint32_t bf[4];
-    ldsm_x4_trans(bf, tile + mrow * kSbTileStride + ncol * 2);
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt) {
-      const uint4 h4 = __ldg(frag + (mt * 4 + ks) * 32 + lane);
-      const uint4 l4 = __ldg(frag + kSbFrags + (mt * 4 + ks) * 32 + lane);
-      const uint32_t ah[4] = {h4.x, h4.y, h4.z, h4.w}, al[4] = {l4.x, l4.y, l4.z, l4.w};
-#pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        mma_bf16(d[mt][nt], ah, bf[2 * nt], bf[2 * nt + 1]);
-        mma_bf16(d[mt][nt], al, bf[2 * nt], bf[2 * nt + 1]);
-      }
-    }
-  }
-}
-
-__device__ __forceinline__ void sts_v4(uint32_t addr, const uint4& v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
-template <int S, bool TAPS>
-__global__ void __launch_bounds__(kSbConsumers + 32, 1) agg_skipconv_backward_kernel(const __grid_constant__ CUtensorMap map_x,
-                                                                                      const __grid_constant__ CUtensorMap map_att,
-                                                                                      const SkipConvBwdArgs a) {
-  using T = __nv_bfloat16;
-  constexpr int VEC = 8;
-  constexpr int M = VEC / S;  // attention cells per thread
-  constexpr int NCOL = M + 2;
-  extern __shared__ __align__(128) unsigned char sb_smem[];  // stages | g_y tile (bf16) | grad_s (fp32), later the s tile
-  __shared__ short frames[1024];
-  __shared__ uint8_t s_pad[1024];
-  __shared__ int n_frames_s;
-  __shared__ __align__(8) unsigned long long bars[2 * kSbMaxStages];
-
-  const int b = blockIdx.y, pblk = blockIdx.x;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int n_cwarps = kSbConsumers / 32;
-  const int n_stages = a.n_stages;
-  const uint32_t stage_stride = kSbStageBytes + 16u * a.tap_floats * 4u;
-  int r_lo = 0;  // first attention row of the staged slice (the rows of the block's first pixel)
-  if (TAPS) {
-    int i1;
-    float l1;
-    source_index(a.sy, (pblk * kSbPB) / a.W, a.ha, r_lo, i1, l1);
-  }
-
-  if (threadIdx.x < 32) {  // ordered list of the frames that are not padded
-    int count = 0;
-    for (int base = 0; base < a.T; base += 32) {
-      const int t = base + threadIdx.x;
-      const bool valid = t < a.T && (a.pad == nullptr || a.pad[b * a.T + t] == 0);
-      if (t < a.T) s_pad[t] = !valid;
-      const unsigned m = __ballot_sync(0xffffffffu, valid);
-      if (valid) frames[count + __popc(m & ((1u << threadIdx.x) - 1u))] = static_cast<short>(t);
-      count += __popc(m);
-    }
-    if (threadIdx.x == 0) {
-      n_frames_s = count;
-      for (int s = 0; s < n_stages; ++s) {
-        mbar_init(s32(&bars[s]), 1);
-        mbar_init(s32(&bars[n_stages + s]), n_cwarps);
-      }
-      fence_mbarrier_init();
-    }
-  }
-  __syncthreads();
-  const int n_frames = n_frames_s;
-  const uint32_t stage0 = s32(sb_smem);
-
-  if (warp == n_cwarps) {  // ---- producer: one box {128 pixels, 64 channels, 1 frame} (+ the attention rows) per frame
-    if (lane == 0) {
-      const uint32_t tap_bytes = TAPS ? 16u * a.tap_floats * 4u : 0u;
-      for (int i = 0; i < n_frames; ++i) {
-        const int s = i % n_stages, round = i / n_stages;
-        if (round > 0) mbar_wait(s32(&bars[n_stages + s]), (round - 1) & 1);
-        const uint32_t full = s32(&bars[s]);
-        mbar_expect_tx(full, kSbStageBytes + tap_bytes);
-        tma_load_3d(stage0 + s * stage_stride, &map_x, pblk * kSbPB, 0, b * a.T + frames[i], full);
-        if (TAPS) tma_load_3d(stage0 + s * stage_stride + kSbStageBytes, &map_att, r_lo * a.wa, b * a.T + frames[i], 0, full);
-      }
-    }
-    return;
-  }
-
-  // ---- consumers: thread = (attention head, 8-pixel vector) ------------------------------------------------------------
-  const int head = threadIdx.x >> 4, pv = threadIdx.x & 15;
-  const int p0 = pblk * kSbPB + pv * VEC;
-  const uint32_t gy_tile = stage0 + n_stages * stage_stride;
-  const uint32_t gs_tile = gy_tile + kSbC * kSbTileStride;  // grad_s fp32 [64][kSbGsStride]; after the sweep the s tile
-  float* gs_smem = reinterpret_cast<float*>(sb_smem + n_stages * stage_stride + kSbC * kSbTileStride);
-  const size_t plane = static_cast<size_t>(b) * kSbC * a.hw + p0;
-
-  // g_y = grad_out masked by the forward's ReLU decision (bf16, exact) -> shared tile
-#pragma unroll
-  for (int c = 0; c < 4; ++c) {
-    const size_t off = plane + static_cast<size_t>(head * 4 + c) * a.hw;
-    const uint4 g = ld_stream_v4(a.gout + off), o = ld_stream_v4(a.out + off);
-    const uint32_t gw[4] = {g.x, g.y, g.z, g.w}, ow[4] = {o.x, o.y, o.z, o.w};
-    uint32_t m[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {  // bf16 pairs: a positive bf16 has a clear sign bit and a non-zero magnitude
-      const uint32_t lo_pos = ((ow[q] & 0x8000u) == 0 && (ow[q] & 0x7fffu) != 0) ? 0x0000ffffu : 0u;
-      const uint32_t hi_pos = ((ow[q] & 0x80000000u) == 0 && (ow[q] & 0x7fff0000u) != 0) ? 0xffff0000u : 0u;
-      m[q] = gw[q] & (lo_pos | hi_pos);
-    }
-    sts_v4(gy_tile + (head * 4 + c) * kSbTileStride + pv * 16, make_uint4(m[0], m[1], m[2], m[3]));
-  }
-  asm volatile("bar.sync 1, %0;" ::"n"(kSbConsumers) : "memory");  // consumers only (the producer warp has its own loop)
-  {  // grad_s = (alpha W)^T g_y -> shared memory (fp32)
-    float d[4][2][4];
-    skipconv_tile_mma(d, a.afrag, gy_tile, warp, lane);
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-      for (int hrow = 0; hrow < 2; ++hrow)
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt) {
-          const int c = mt * 16 + (lane >> 2) + hrow * 8, p = warp * 16 + nt * 8 + (lane & 3) * 2;
-          *reinterpret_cast<float2*>(gs_smem + c * kSbGsStride + p) = make_float2(d[mt][nt][hrow * 2], d[mt][nt][hrow * 2 + 1]);
-        }
-  }
-  asm volatile("bar.sync 1, %0;" ::"n"(kSbConsumers) : "memory");
-  float gs[4][VEC];
-#pragma unroll
-  for (int c = 0; c < 4; ++c) {
-    const float4 v0 = *reinterpret_cast<const float4*>(gs_smem + (head * 4 + c) * kSbGsStride + pv * VEC);
-    const float4 v1 = *reinterpret_cast<const float4*>(gs_smem + (head * 4 + c) * kSbGsStride + pv * VEC + 4);
-    gs[c][0] = v0.x, gs[c][1] = v0.y, gs[c][2] = v0.z, gs[c][3] = v0.w;
-    gs[c][4] = v1.x, gs[c][5] = v1.y, gs[c][6] = v1.z, gs[c][7] = v1.w;
-  }
-
-  // bilinear geometry (identical to agg_skipconv_kernel)
-  const int y = p0 / a.W;
-  const int x0 = p0 - y * a.W;
-  int iy0, iy1;
-  float ly1;
-  source_index(a.sy, y, a.ha, iy0, iy1, ly1);
-  const float ly0 = 1.f - ly1;
-  const int row0 = iy0 * a.wa, row1 = iy1 * a.wa;
-  float lx1[VEC];
-#pragma unroll
-  for (int j = 0; j < VEC; ++j) {
-    int i0, i1;
-    source_index(a.sx, x0 + j, a.wa, i0, i1, lx1[j]);
-  }
-  const int cmin = x0 / S - 1;
-  int col[NCOL];
-#pragma unroll
-  for (int j = 0; j < NCOL; ++j) {
-    const int cj = cmin + j;
-    col[j] = cj < 0 ? 0 : (cj > a.wa - 1 ? a.wa - 1 : cj);
-  }
-  const int amap = a.ha * a.wa;
-  const size_t abase = (static_cast<size_t>(head) * a.B + b) * a.T * amap;
-  const int trow0 = (iy0 - r_lo) * a.wa, trow1 = (iy1 - r_lo) * a.wa;
-  // 16 lanes of a head cover the 128 pixels in order: a lane's left / right neighbour in the image row sits next to it
-  const int lanes_per_row = a.W / VEC;
-  const int lane_in_row = (p0 / VEC) % lanes_per_row;
-  const bool has_left = pv > 0 && lane_in_row > 0;
-  const bool has_right = pv < 15 && lane_in_row < lanes_per_row - 1;
-  const size_t frame_stride = static_cast<size_t>(kSbC) * a.hw;
-  T* gxb = a.gx != nullptr ? a.gx + static_cast<size_t>(b) * a.T * frame_stride + static_cast<size_t>(head * 4) * a.hw + p0 : nullptr;
-
-  float acc[4][VEC];
-#pragma unroll
-  for (int c = 0; c < 4; ++c)
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) acc[c][j] = 0.f;
-
-  const uint32_t my_off = (head * 4) * (kSbPB * 2) + pv * 16;
-  for (int i = 0; i < n_frames; ++i) {
-    const int t = frames[i];
-    float r[NCOL];
-    if (!TAPS) {
-      const float* ap = a.attn + abase + static_cast<size_t>(t) * amap;
-#pragma unroll
-      for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, __ldg(ap + row1 + col[j]), ly0 * __ldg(ap + row0 + col[j]));
-    }
-    const int s = i % n_stages;
-    mbar_wait(s32(&bars[s]), (i / n_stages) & 1);
-    uint4 xv[4];
-    const uint32_t base = stage0 + s * stage_stride + my_off;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) xv[c] = lds_v4(base + c * (kSbPB * 2));
-    if (TAPS) {
-      const float* tp = reinterpret_cast<const float*>(sb_smem + s * stage_stride + kSbStageBytes) + head * a.tap_floats;
-#pragma unroll
-      for (int j = 0; j < NCOL; ++j) r[j] = fmaf(ly1, tp[trow1 + col[j]], ly0 * tp[trow0 + col[j]]);
-    }
-    fence_proxy_async();  // the stage's shared loads before the producer's next bulk copy into it
-    __syncwarp();
-    if (lane == 0) mbar_arrive(s32(&bars[n_stages + s]));
-
-    float w[VEC];
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) {
-      const int i0w = j / S + ((j % S) < S / 2 ? 0 : 1);
-      w[j] = fmaf(lx1[j], r[i0w + 1], (1.f - lx1[j]) * r[i0w]);
-    }
-    float g[VEC];  // sum_c x * grad_s of this thread's pixels
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) g[j] = 0.f;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      float f[VEC], dx[VEC];
-      Elem<T>::unpack(xv[c], f);
-#pragma unroll
-      for (int j = 0; j < VEC; ++j) {
-        acc[c][j] = fmaf(w[j], f[j], acc[c][j]);  // the forward's accumulation
-        g[j] = fmaf(f[j], gs[c][j], g[j]);
-        dx[j] = w[j] * gs[c][j];
-      }
-      if (gxb != nullptr) st_stream_v4(gxb + static_cast<size_t>(t) * frame_stride + static_cast<size_t>(c) * a.hw, Elem<T>::pack(dx));
-    }
-    if (a.gattn == nullptr) continue;
-    // horizontal adjoint into the NCOL-column window, then edge columns travel to the neighbouring lanes
-    float* gp = a.gattn + abase + static_cast<size_t>(t) * amap;
-    float win[NCOL];
-#pragma unroll
-    for (int jj = 0; jj < NCOL; ++jj) win[jj] = 0.f;
-#pragma unroll
-    for (int j = 0; j < VEC; ++j) {
-      const int i0w = j / S + ((j % S) < S / 2 ? 0 : 1);
-      win[i0w] = fmaf(g[j], 1.f - lx1[j], win[i0w]);
-      win[i0w + 1] = fmaf(g[j], lx1[j], win[i0w + 1]);
-    }
-    const float from_left = __shfl_up_sync(0xffffffffu, win[NCOL - 1], 1);
-    const float from_right = __shfl_down_sync(0xffffffffu, win[0], 1);
-    float own[M];
-#pragma unroll
-    for (int q = 0; q < M; ++q) own[q] = win[q + 1];
-    if (has_left) own[0] += from_left;
-    if (has_right) own[M - 1] += from_right;
-#pragma unroll
-    for (int q = 0; q < M; ++q) {
-      const int cj = cmin + 1 + q;  // own columns are always inside [0, wa)
-      atomicAdd(gp + row0 + cj, ly0 * own[q]);
-      if (ly1 != 0.f) atomicAdd(gp + row1 + cj, ly1 * own[q]);
-    }
-    if (!has_left) {  // edge columns nobody picked up (image border: clamped; head or row boundary)
-      atomicAdd(gp + row0 + col[0], ly0 * win[0]);
-      if (ly1 != 0.f) atomicAdd(gp + row1 + col[0], ly1 * win[0]);
-    }
-    if (!has_right) {
-      atomicAdd(gp + row0 + col[NCOL - 1], ly0 * win[NCOL - 1]);
-      if (ly1 != 0.f) atomicAdd(gp + row1 + col[NCOL - 1], ly1 * win[NCOL - 1]);
-    }
-  }
-  if (gxb != nullptr && n_frames < a.T) {  // padded frames receive exactly zero
-    const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-    for (int t = 0; t < a.T; ++t)
-      if (s_pad[t])
-#pragma unroll
-        for (int c = 0; c < 4; ++c) st_stream_v4(gxb + static_cast<size_t>(t) * frame_stride + static_cast<size_t>(c) * a.hw, z);
-  }
-  if (a.partial == nullptr) return;
-
-  // ---- parameter gradients of the tile: the s tile (bf16, the forward's value) replaces grad_s in shared memory -------
-  asm volatile("bar.sync 1, %0;" ::"n"(kSbConsumers) : "memory");  // every consumer has its grad_s in registers
-  const uint32_t s_tile = gs_tile;
-#pragma unroll
-  for (int c = 0; c < 4; ++c) sts_v4(s_tile + (head * 4 + c) * kSbTileStride + pv * 16, Elem<T>::pack(acc[c]));
-  asm volatile("bar.sync 1, %0;" ::"n"(kSbConsumers) : "memory");
-  float* part = a.partial + (static_cast<size_t>(b) * gridDim.x + pblk) * kSbPartial;
-  float(*red)[8][kSbC] = reinterpret_cast<float(*)[8][kSbC]>(sb_smem);  // per-warp sums; the stages are drained by now
-  {  // z - mean = W s + (bias - mean): sums of g_y and g_y (z - mean) per output channel
-    float d[4][2][4];
-    skipconv_tile_mma(d, a.wfrag, s_tile, warp, lane);
-    const unsigned char* gyb = sb_smem + n_stages * stage_stride;
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-      for (int hrow = 0; hrow < 2; ++hrow) {
-        const int o = mt * 16 + (lane >> 2) + hrow * 8;
-        const float zs = __ldg(a.zshift + o);
-        float sg = 0.f, sgz = 0.f;
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt) {
-          const int p = warp * 16 + nt * 8 + (lane & 3) * 2;
-          const __nv_bfloat162 gy2 = *reinterpret_cast<const __nv_bfloat162*>(gyb + o * kSbTileStride + p * 2);
-          const float g0 = __low2float(gy2), g1 = __high2float(gy2);
-          sg += g0 + g1;
-          sgz = fmaf(g0, d[mt][nt][hrow * 2] + zs, sgz);
-          sgz = fmaf(g1, d[mt][nt][hrow * 2 + 1] + zs, sgz);
-        }
-        sg += __shfl_xor_sync(0xffffffffu, sg, 1);
-        sg += __shfl_xor_sync(0xffffffffu, sg, 2);
-        sgz += __shfl_xor_sync(0xffffffffu, sgz, 1);
-        sgz += __shfl_xor_sync(0xffffffffu, sgz, 2);
-        if ((lane & 3) == 0) red[0][warp][o] = sg, red[1][warp][o] = sgz;
-      }
-  }
-  {  // g_y s^T [64 out][64 in] over the 128 pixels: warp w takes m-tile w / 2 and n-tiles 4 (w % 2) .. + 3, K = pixels
-    const int mt = warp >> 1, nt0 = (warp & 1) * 4;
-    float d[4][4];
-#pragma unroll
-    for (int n = 0; n < 4; ++n)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) d[n][e] = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < kSbPB / 16; ++ks) {
-      uint32_t af[4];
-      ldsm_x4(af, gy_tile + (mt * 16 + (lane & 15)) * kSbTileStride + (ks * 16 + (lane >> 4) * 8) * 2);
-#pragma unroll
-      for (int np = 0; np < 2; ++np) {  // two n-tiles per ldmatrix.x4: (n 0-7 | 8-15) x (k 0-7 | 8-15)
-        uint32_t bf[4];
-        const int crow = (nt0 + 2 * np) * 8 + (lane & 7) + ((lane >> 4) & 1) * 8;
-        ldsm_x4(bf, s_tile + crow * kSbTileStride + (ks * 16 + ((lane >> 3) & 1) * 8) * 2);
-        mma_bf16(d[2 * np], af, bf[0], bf[1]);
-        mma_bf16(d[2 * np + 1], af, bf[2], bf[3]);
-      }
-    }
-#pragma unroll
-    for (int n = 0; n < 4; ++n)
-#pragma unroll
-      for (int hrow = 0; hrow < 2; ++hrow) {
-        const int o = mt * 16 + (lane >> 2) + hrow * 8, c = (nt0 + n) * 8 + (lane & 3) * 2;
-        *reinterpret_cast<float2*>(part + o * kSbC + c) = make_float2(d[n][hrow * 2], d[n][hrow * 2 + 1]);
-      }
-  }
-  asm volatile("bar.sync 1, %0;" ::"n"(kSbConsumers) : "memory");
-  if (threadIdx.x < 2 * kSbC) {  // fixed order over the warps
-    const int q = threadIdx.x / kSbC, o = threadIdx.x % kSbC;
-    float v = 0.f;
-#pragma unroll
-    for (int w8 = 0; w8 < 8; ++w8) v += red[q][w8][o];
-    part[kSbC * kSbC + q * kSbC + o] = v;
-  }
-}
-
-// Sum of the CTA partials in a fixed order (warp w takes CTAs w, w + 8, ...; the 8 warp sums are added in order), then
-// the chain to the parameters: grad_conv_weight = alpha g_y s^T, grad_conv_bias = alpha sum g_y, grad_bn_bias = sum g_y,
-// grad_bn_weight = sum g_y (z - mean) / sqrt(var + eps).
-__global__ void __launch_bounds__(256) skipconv_bwd_finish_kernel(const float* __restrict__ partial, int n_ctas,
-                                                                  const float* __restrict__ alpha, const float* __restrict__ inv_std,
-                                                                  float* gw, float* gb, float* gbn_w, float* gbn_b) {
-  __shared__ float sums[8][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int e = blockIdx.x * 32 + lane;
-  float v = 0.f;
-  if (e < kSbPartial)
-    for (int i = warp; i < n_ctas; i += 8) v += partial[static_cast<size_t>(i) * kSbPartial + e];
-  sums[warp][lane] = v;
-  __syncthreads();
-  if (warp != 0 || e >= kSbPartial) return;
-  float total = 0.f;
-#pragma unroll
-  for (int w8 = 0; w8 < 8; ++w8) total += sums[w8][lane];
-  if (e < kSbC * kSbC) {
-    if (gw != nullptr) gw[e] = alpha[e / kSbC] * total;
-  } else if (e < kSbC * kSbC + kSbC) {
-    const int o = e - kSbC * kSbC;
-    if (gb != nullptr) gb[o] = alpha[o] * total;
-    if (gbn_b != nullptr) gbn_b[o] = total;
-  } else {
-    const int o = e - kSbC * kSbC - kSbC;
-    if (gbn_w != nullptr) gbn_w[o] = inv_std[o] * total;
-  }
-}
-
-size_t skipconv_bwd_smem(int n_stages, int tap_floats) {  // stages | g_y tile | grad_s (then s) tile
-  return static_cast<size_t>(n_stages) * (kSbStageBytes + 16 * tap_floats * 4) + kSbC * kSbTileStride + kSbC * kSbGsStride * 4;
-}
-
-template <int S, bool TAPS>
-int launch_skipconv_bwd_t(const CUtensorMap& map_x, const CUtensorMap& map_att, const SkipConvBwdArgs& k, cudaStream_t stream,
-                          const char* name) {
-  const size_t smem = skipconv_bwd_smem(k.n_stages, k.tap_floats);
-  C2S_SMEM_ATTR((agg_skipconv_backward_kernel<S, TAPS>), 227 * 1024);  // once per instantiation and device
-  dim3 grid(k.hw / kSbPB, k.B);
-  agg_skipconv_backward_kernel<S, TAPS><<<grid, kSbConsumers + 32, smem, stream>>>(map_x, map_att, k);
-  C2S_LAUNCH_CHECK(name);
-  return C2S_OK;
-}
-
-template <int S>
-int launch_skipconv_bwd(const CUtensorMap& map_x, const CUtensorMap& map_att, const SkipConvBwdArgs& k, cudaStream_t stream,
-                        const char* name) {
-  return k.tap_floats > 0 ? launch_skipconv_bwd_t<S, true>(map_x, map_att, k, stream, name)
-                          : launch_skipconv_bwd_t<S, false>(map_x, map_att, k, stream, name);
-}
-
-// workspace: W and (alpha W)^T fragments, alpha / inv_std / zshift, then the CTA partials (16-byte aligned throughout)
-constexpr size_t kSbFixedBytes = 2 * 2 * kSbFrags * sizeof(uint4) + 3 * kSbC * sizeof(float);
-size_t skipconv_bwd_ctas(const c2s_agg_desc* d) {
-  return d->B > 0 && d->H > 0 && d->W > 0 ? static_cast<size_t>(d->B) * ((static_cast<size_t>(d->H) * d->W) / kSbPB) : 0;
-}
-
 }  // namespace
 }  // namespace c2s
 
@@ -1216,101 +733,6 @@ int c2s_agg_backward(const c2s_agg_desc* d, const void* x, const float* attn, co
     unpool_grad_kernel<<<ceil_div(n_in, 256), 256, 0, stream>>>(gpool, grad_attn, d->ha, d->wa, d->H, d->W, pool_k, n_in);
     C2S_LAUNCH_CHECK("avg_unpool");
   }
-  return C2S_OK;
-}
-
-size_t c2s_agg_skipconv_backward_workspace_bytes(const c2s_agg_desc* d) {
-  if (d == nullptr) return 0;
-  return c2s::kSbFixedBytes + c2s::skipconv_bwd_ctas(d) * c2s::kSbPartial * sizeof(float);
-}
-
-int c2s_agg_skipconv_backward(const c2s_agg_desc* d, const void* x, const float* attn, const uint8_t* pad_mask,
-                              const c2s_skipconv_params* p, const void* out, const void* grad_out,
-                              const c2s_skipconv_bwd_io* io, void* workspace, size_t workspace_bytes, void* stream_ptr) {
-  using namespace c2s;
-  C2S_CHECK_ARG(d != nullptr && p != nullptr && io != nullptr, "c2s_agg_skipconv_backward: desc/params/io is NULL");
-  C2S_CHECK_ARG(x != nullptr && attn != nullptr && out != nullptr && grad_out != nullptr,
-                "c2s_agg_skipconv_backward: x/attn/out/grad_out is NULL");
-  C2S_CHECK_ARG(p->conv_weight != nullptr && p->bn_running_mean != nullptr && p->bn_running_var != nullptr,
-                "c2s_agg_skipconv_backward: conv weight and BatchNorm running statistics are required");
-  C2S_CHECK_ARG(d->B > 0 && d->T > 0 && d->H > 0 && d->W > 0, "c2s_agg_skipconv_backward: non-positive dimension");
-  int scale_class = 0;
-  for (int s : {2, 4, 8})
-    if (d->H == s * d->ha && d->W == s * d->wa) scale_class = s;
-  const int hw = d->H * d->W;
-  auto al16 = [](const void* q) { return q == nullptr || reinterpret_cast<uintptr_t>(q) % 16 == 0; };
-  C2S_CHECK_ARG(d->mode == C2S_AGG_ATT_GROUP && d->dtype == C2S_BF16 && d->C == kSbC && d->n_heads == 16 && scale_class != 0 &&
-                    hw % kSbPB == 0 && d->W % 8 == 0 && d->T <= 1024 && d->B <= 65535 && al16(x) && al16(out) &&
-                    al16(grad_out) && al16(io->grad_x),
-                "c2s_agg_skipconv_backward: the fused backward serves what the fused forward serves: att_group, bf16, C=64, "
-                "16 heads, x2/x4/x8 up-sampling, H*W %% 128 == 0, 16-byte aligned tensors (got mode %d dtype %d C %d heads "
-                "%d %dx%d from %dx%d)", d->mode, d->dtype, d->C, d->n_heads, d->H, d->W, d->ha, d->wa);
-  const bool want_params = io->grad_conv_weight != nullptr || io->grad_conv_bias != nullptr || io->grad_bn_weight != nullptr ||
-                           io->grad_bn_bias != nullptr;
-  if (!want_params && io->grad_x == nullptr && io->grad_attn == nullptr) return C2S_OK;  // nothing asked for
-  const size_t need = c2s_agg_skipconv_backward_workspace_bytes(d);
-  C2S_CHECK_ARG(workspace != nullptr && workspace_bytes >= need && reinterpret_cast<uintptr_t>(workspace) % 16 == 0,
-                "c2s_agg_skipconv_backward: needs %zu workspace bytes, 16-byte aligned", need);
-  int status = check_device();
-  if (status != C2S_OK) return status;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
-
-  uint4* wfrag = static_cast<uint4*>(workspace);
-  uint4* afrag = wfrag + 2 * kSbFrags;
-  float* alpha = reinterpret_cast<float*>(afrag + 2 * kSbFrags);
-  float* inv_std = alpha + kSbC;
-  float* zshift = inv_std + kSbC;
-  float* partial = reinterpret_cast<float*>(static_cast<char*>(workspace) + kSbFixedBytes);
-  skipconv_bwd_prep_kernel<<<3, 256, 0, stream>>>(p->conv_weight, p->conv_bias, p->bn_weight, p->bn_running_mean,
-                                                  p->bn_running_var, p->bn_eps, wfrag, afrag, alpha, inv_std, zshift);
-  C2S_LAUNCH_CHECK("agg_skipconv_backward<prep>");
-
-  SkipConvBwdArgs k{};
-  k.attn = attn, k.pad = pad_mask;
-  k.out = static_cast<const __nv_bfloat16*>(out), k.gout = static_cast<const __nv_bfloat16*>(grad_out);
-  k.gx = static_cast<__nv_bfloat16*>(io->grad_x), k.gattn = io->grad_attn;
-  k.wfrag = wfrag, k.afrag = afrag, k.zshift = zshift, k.partial = want_params ? partial : nullptr;
-  k.B = d->B, k.T = d->T, k.H = d->H, k.W = d->W, k.hw = hw, k.ha = d->ha, k.wa = d->wa;
-  k.sy = static_cast<float>(d->ha) / static_cast<float>(d->H);
-  k.sx = static_cast<float>(d->wa) / static_cast<float>(d->W);
-  {  // staged attention rows: the rows a 128-pixel block can touch, per head (as in c2s_agg_skipconv_forward)
-    const int rows_out = (kSbPB + d->W - 1) / d->W + 1;
-    int rows_att = rows_out / scale_class + 3;
-    rows_att = rows_att > d->ha ? d->ha : rows_att;
-    const int tap_floats = ((rows_att * d->wa + 3) / 4) * 4;
-    const bool taps = option(C2S_OPT_AGG_TAPS) == 0 && d->wa % 4 == 0 && reinterpret_cast<uintptr_t>(attn) % 16 == 0 &&
-                      tap_floats <= 256;
-    k.tap_floats = taps ? tap_floats : 0;
-  }
-  k.n_stages = kSbMaxStages;  // fewer if the staged rows make them too large for one CTA (227 KB with the static part)
-  while (k.n_stages > 2 && skipconv_bwd_smem(k.n_stages, k.tap_floats) > 220 * 1024) --k.n_stages;
-  CUtensorMap map_x;  // x as [B*T][C][H*W] bf16; box = 128 pixels x 64 channels x 1 frame
-  const cuuint64_t dims[3] = {static_cast<cuuint64_t>(hw), static_cast<cuuint64_t>(kSbC), static_cast<cuuint64_t>(d->B) * d->T};
-  const cuuint64_t strides[2] = {static_cast<cuuint64_t>(hw) * 2, static_cast<cuuint64_t>(kSbC) * hw * 2};
-  const cuuint32_t box[3] = {kSbPB, kSbC, 1};
-  status = encode_tensor_map(&map_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE,
-                             CU_TENSOR_MAP_L2_PROMOTION_NONE, "skip features");
-  if (status != C2S_OK) return status;
-  CUtensorMap map_att = map_x;  // attention as [16 heads][B*T][ha*wa] fp32; box = tap_floats of one map x 1 frame x 16 heads
-  if (k.tap_floats > 0) {
-    const cuuint64_t amap = static_cast<cuuint64_t>(d->ha) * d->wa;
-    const cuuint64_t adims[3] = {amap, static_cast<cuuint64_t>(d->B) * d->T, 16};
-    const cuuint64_t astrides[2] = {amap * 4, static_cast<cuuint64_t>(d->B) * d->T * amap * 4};
-    const cuuint32_t abox[3] = {static_cast<cuuint32_t>(k.tap_floats), 1, 16};
-    status = encode_tensor_map(&map_att, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, attn, adims, astrides, abox,
-                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, "attention");
-    if (status != C2S_OK) return status;
-  }
-  switch (scale_class) {
-    case 2: status = launch_skipconv_bwd<2>(map_x, map_att, k, stream, "agg_skipconv_backward<x2>"); break;
-    case 4: status = launch_skipconv_bwd<4>(map_x, map_att, k, stream, "agg_skipconv_backward<x4>"); break;
-    default: status = launch_skipconv_bwd<8>(map_x, map_att, k, stream, "agg_skipconv_backward<x8>"); break;
-  }
-  if (status != C2S_OK || !want_params) return status;
-  skipconv_bwd_finish_kernel<<<ceil_div(kSbPartial, 32), 256, 0, stream>>>(
-      partial, static_cast<int>(skipconv_bwd_ctas(d)), alpha, inv_std, io->grad_conv_weight, io->grad_conv_bias,
-      io->grad_bn_weight, io->grad_bn_bias);
-  C2S_LAUNCH_CHECK("agg_skipconv_backward<reduce>");
   return C2S_OK;
 }
 

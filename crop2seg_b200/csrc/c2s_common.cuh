@@ -140,6 +140,9 @@ __device__ __forceinline__ float warp_max(float v) {
   return v;
 }
 
+// frames per series the aggregator kernels' frame list in shared memory can hold
+constexpr int kAggMaxT = 1024;
+
 // ATen area_pixel_compute_source_index(scale, dst, align_corners=false) + the i0/i1/lambda split of upsample_bilinear2d
 // (nn.Upsample of the attention masks, reference temporal_aggregator.py:17-19).  The aggregator's forward and backward
 // must agree on it.

@@ -131,6 +131,43 @@ def test_parameter_gradients_are_deterministic_and_null_outputs_are_skipped():
         assert gx_only[1:] == (None,) * 5 and torch.equal(gx_only[0], first[0])
 
 
+@pytest.mark.parametrize("global_taps", [False, True])
+@pytest.mark.parametrize("name", sorted(CASES))
+def test_backward_recomputes_the_forward_skip_map_bit_for_bit(name, global_taps):
+    """The weight gradient relies on the backward's skip map s being the forward's.  With an identity convolution and a
+    neutral BatchNorm (eps = 0) the forward's output is exactly relu(s); a grad_out that is 1 on every channel of one
+    pixel p makes grad_conv_weight[o, c] = s_bwd[c, p] exactly for every o with out[o, p] > 0 (one non-zero term,
+    alpha = 1).  x has both signs, so relu(s) is zero on a part of the channels."""
+    from crop2seg_b200 import _lib, ops
+    from c2s_testlib import bf16_round, random_attention, synth_inputs, to_dev
+    b, t, res, ares, lengths = CASES[name]
+    rng = np.random.RandomState(31 + res)
+    _, _, pad = synth_inputs(rng, b, t, 64, res, res, lengths)
+    x = bf16_round(rng.standard_normal((b, t, 64, res, res)).astype(np.float32))
+    attn = random_attention(rng, 16, pad, ares, ares)
+    conv, bn = nn.Conv2d(64, 64, 1).cuda(), nn.BatchNorm2d(64, eps=0.0).cuda().eval()  # BatchNorm: weight 1, bias 0,
+    with torch.no_grad():                                                                # mean 0, var 1
+        conv.weight.copy_(torch.eye(64).view(64, 64, 1, 1))
+        conv.bias.zero_()
+    args = (to_dev(x, dtype=torch.bfloat16), to_dev(pad), to_dev(attn), conv.weight, conv.bias, bn.weight, bn.bias,
+            bn.running_mean, bn.running_var, bn.eps)
+    # first and last pixel of the second 128-pixel block, a right-border column and an interior pixel
+    pixels = [128, 255, (res // 2) * res + res - 1, (res // 2 + 1) * res + res // 2 + 3]
+    with torch.no_grad(), _lib.option(_lib.OPT_AGG_TAPS, int(global_taps)):
+        out = ops.temporal_aggregate_skip_conv(*args)
+        for b0 in [i for i, n in enumerate(lengths) if n > 0]:
+            for p in pixels:
+                gout = torch.zeros_like(out)
+                gout[b0, :, p // res, p % res] = 1
+                gw = ops.temporal_aggregate_skip_conv_backward(*args, out, gout)[2].view(64, 64)
+                s_fwd = out[b0, :, p // res, p % res].float()
+                pos = s_fwd > 0
+                assert pos.any() and (~pos).any(), (b0, p)
+                g = gw[pos]  # rows o with out[o, p] > 0
+                assert torch.equal(g[:, pos], s_fwd[pos].expand_as(g[:, pos])), (b0, p)
+                assert (g[:, ~pos] <= 0).all(), (b0, p)
+
+
 def test_unsupported_shapes_raise():
     import crop2seg_b200 as c2s
     from crop2seg_b200 import ops
