@@ -27,7 +27,8 @@ EXPORTS = (
     "c2s_last_ltae_kernel", "c2s_set_option", "c2s_get_option",
     "c2s_agg_workspace_bytes", "c2s_agg_forward", "c2s_agg_backward_workspace_bytes", "c2s_agg_backward",
     "c2s_agg_skipconv_workspace_bytes", "c2s_agg_skipconv_forward", "c2s_agg_skipconv_backward_workspace_bytes",
-    "c2s_agg_skipconv_backward", "c2s_pad_mask",
+    "c2s_agg_skipconv_backward", "c2s_agg_skipconv_bstats_workspace_bytes", "c2s_agg_skipconv_bstats_forward",
+    "c2s_agg_skipconv_bstats_backward_workspace_bytes", "c2s_agg_skipconv_bstats_backward", "c2s_pad_mask",
     "c2s_ltae_workspace_bytes", "c2s_ltae_forward", "c2s_ltae_backward_workspace_bytes", "c2s_ltae_backward",
     "c2s_ltae_mlp_backward_workspace_bytes", "c2s_ltae_mlp_backward", "c2s_ltae_inconv_grad", "c2s_ltae_fold_backward",
     "c2s_ltae_rows_forward",
@@ -165,6 +166,16 @@ def load() -> ctypes.CDLL:
         lib.c2s_agg_skipconv_backward.restype = i32
         lib.c2s_agg_skipconv_backward.argtypes = [ctypes.POINTER(AggDesc), vp, vp, vp, ctypes.POINTER(SkipConvParams), vp,
                                                   vp, ctypes.POINTER(SkipConvBwdIo), vp, sz, vp]
+        lib.c2s_agg_skipconv_bstats_workspace_bytes.restype = sz
+        lib.c2s_agg_skipconv_bstats_workspace_bytes.argtypes = [ctypes.POINTER(AggDesc)]
+        lib.c2s_agg_skipconv_bstats_forward.restype = i32
+        lib.c2s_agg_skipconv_bstats_forward.argtypes = [ctypes.POINTER(AggDesc), vp, vp, vp, ctypes.POINTER(SkipConvParams),
+                                                        vp, vp, vp, vp, vp, sz, vp]
+        lib.c2s_agg_skipconv_bstats_backward_workspace_bytes.restype = sz
+        lib.c2s_agg_skipconv_bstats_backward_workspace_bytes.argtypes = [ctypes.POINTER(AggDesc)]
+        lib.c2s_agg_skipconv_bstats_backward.restype = i32
+        lib.c2s_agg_skipconv_bstats_backward.argtypes = [ctypes.POINTER(AggDesc), vp, vp, vp, ctypes.POINTER(SkipConvParams),
+                                                         vp, vp, vp, vp, vp, ctypes.POINTER(SkipConvBwdIo), vp, sz, vp]
         lib.c2s_ltae_rows_forward.restype = i32
         lib.c2s_ltae_rows_forward.argtypes = [vp, vp, vp, i32, vp, vp]
         lib.c2s_ltae_inconv_grad.restype = i32

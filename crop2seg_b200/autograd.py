@@ -5,6 +5,9 @@
 * ``AggregateSkipConvFunction``: the aggregation fused with the decoder's skip convolution, BatchNorm frozen (running
   statistics); forward ``c2s_agg_skipconv_forward``, backward ``c2s_agg_skipconv_backward``, which recomputes the skip
   map on chip from x, so only the output is saved besides the inputs.
+* ``AggregateSkipConvBatchStatsFunction``: the same block with batch statistics (BatchNorm in training mode); forward
+  ``c2s_agg_skipconv_bstats_forward``, backward ``c2s_agg_skipconv_bstats_backward``, which also reads the saved
+  pre-BatchNorm z.
 * ``LtaeFunction``: the forward is the fused CUDA kernel (train-mode BatchNorm statistics and injected dropout masks
   included).  The backward has three stages:
     M  ``c2s_ltae_mlp_backward`` (CUDA, ``csrc/c2s_ltae_mlp_bwd.cu``): the rows after the attention (MLP Linear,
@@ -67,6 +70,33 @@ class AggregateSkipConvFunction(torch.autograd.Function):
         def cast(g, p):
             return None if g is None else g.to(p.dtype)
         return (gx, cast(gattn, attn), None, cast(gcw, cw), cast(gcb, cb), cast(gbw, bw), cast(gbb, bb), None, None, None)
+
+
+class AggregateSkipConvBatchStatsFunction(torch.autograd.Function):
+    """apply(x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_eps) -> (out, batch_mean, batch_var)
+
+    The same block with its BatchNorm normalising by batch statistics; the pre-BatchNorm z (bf16) is saved for the
+    backward next to the output.  The running statistics are the caller's (batch_mean / batch_var are not differentiable)."""
+
+    @staticmethod
+    def forward(ctx, x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, bn_eps):
+        out, z, mean, var = ops.temporal_aggregate_skip_conv_bstats_forward(x, pad_mask, attn, conv_weight, conv_bias,
+                                                                            bn_weight, bn_bias, bn_eps)
+        ctx.bn_eps = bn_eps
+        ctx.save_for_backward(x, attn, pad_mask, conv_weight, conv_bias, bn_weight, bn_bias, z, mean, var, out)
+        ctx.mark_non_differentiable(mean, var)
+        return out, mean, var
+
+    @staticmethod
+    def backward(ctx, grad_out, _grad_mean, _grad_var):
+        x, attn, pad, cw, cb, bw, bb, z, mean, var, out = ctx.saved_tensors
+        need = [ctx.needs_input_grad[i] for i in (0, 1, 3, 4, 5, 6)]
+        gx, gattn, gcw, gcb, gbw, gbb = ops.temporal_aggregate_skip_conv_bstats_backward(
+            x, pad, attn, cw, cb, bw, bb, ctx.bn_eps, z, mean, var, out, grad_out, need=need)
+
+        def cast(g, p):
+            return None if g is None else g.to(p.dtype)
+        return (gx, cast(gattn, attn), None, cast(gcw, cw), cast(gcb, cb), cast(gbw, bw), cast(gbb, bb), None)
 
 
 # ------------------------------------------------------------------------------------------------------------

@@ -11,6 +11,11 @@
 // The backward recomputes the skip map with the same prologue, producer, bilinear geometry, tap interpolation, weights
 // and accumulation as the forward, in the forward's frame order, so its bf16 s is the forward's bit for bit: the
 // BatchNorm-weight and conv-weight gradients rely on that.
+//
+// With the BatchNorm in training mode (batch statistics) the statistics must be complete before any output can be
+// normalised, and the x sweep is too expensive to repeat, so the pre-BatchNorm z = W s + b crosses HBM once in bf16 (the
+// value the unfused bf16 convolution stores): the sweep (BSTATS instantiation) writes z and per-CTA mean / M2 partials,
+// skipconv_bstats_finish_kernel merges them, skipconv_bstats_apply_kernel writes relu(scale z + shift).
 #include <initializer_list>
 
 #include "c2s_sm100.cuh"
@@ -41,10 +46,11 @@ struct SkipConvArgs {
   SkipConvShape g;
   const float* attn;   // [16 heads, B, T, ha, wa]
   const uint8_t* pad;  // [B, T] or nullptr
-  __nv_bfloat16* out;
+  __nv_bfloat16* out;  // BSTATS: z
   const uint4* wfrag;  // [hi|lo][m-tile 4][k-step 4][lane 32] A fragments of W (bf16 pairs)
   const float* scale;  // [64]  gamma / sqrt(var + eps)
-  const float* shift;  // [64]  (conv_bias - mean) * scale + beta
+  const float* shift;  // [64]  (conv_bias - mean) * scale + beta; BSTATS: conv_bias or nullptr
+  float* partial;      // BSTATS: [mean | M2][64][CTAs] of the tile's z
 };
 
 struct SkipConvBwdArgs {
@@ -57,9 +63,20 @@ struct SkipConvBwdArgs {
   float* gattn;
   const uint4* wfrag;   // [hi|lo] A fragments of W            (z = W s)
   const uint4* afrag;   // [hi|lo] A fragments of (alpha W)^T  (grad_s = (alpha W)^T g_y)
-  const float* zshift;  // [64] conv_bias - running_mean
+  const float* zshift;  // [64] conv_bias - running_mean; BSTATS: -batch mean of z
   float* partial;       // [CTAs][kScPartial] or nullptr (no parameter gradient wanted)
 };
+
+// the backward's inputs with batch statistics: a separate parameter, empty for the eval instantiation (whose code and
+// registers stay those of a kernel without it)
+template <bool BSTATS>
+struct SkipConvBstatsIn {
+  const __nv_bfloat16* z;  // the forward's pre-BatchNorm z [B,64,H,W]
+  const float* inv_std;    // [64] 1 / sqrt(batch var + eps)
+  const float* gmean;      // [2][64] mean_N(g_y), mean_N(g_y zhat)
+};
+template <>
+struct SkipConvBstatsIn<false> {};
 
 // ---------------------------------------------------------------------------------------------------------------------
 // weight preparation
@@ -280,10 +297,97 @@ __device__ __forceinline__ void skipconv_tile_mma(float (&d)[4][2][4], const uin
   }
 }
 
+// g_y = grad_out masked by the forward's ReLU decision, 8 bf16 pixels (exact): a positive bf16 has a clear sign bit and a
+// non-zero magnitude
+__device__ __forceinline__ uint4 relu_masked(const uint4& gv, const uint4& o) {
+  const uint32_t gw[4] = {gv.x, gv.y, gv.z, gv.w}, ow[4] = {o.x, o.y, o.z, o.w};
+  uint32_t m[4];
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const uint32_t lo_pos = ((ow[q] & 0x8000u) == 0 && (ow[q] & 0x7fffu) != 0) ? 0x0000ffffu : 0u;
+    const uint32_t hi_pos = ((ow[q] & 0x80000000u) == 0 && (ow[q] & 0x7fff0000u) != 0) ? 0xffff0000u : 0u;
+    m[q] = gw[q] & (lo_pos | hi_pos);
+  }
+  return make_uint4(m[0], m[1], m[2], m[3]);
+}
+
+// Reduction of one value per thread over a 256-thread block in a fixed order (deterministic); thread 0 gets the result
+template <class V, class Merge>
+__device__ __forceinline__ V block_reduce_fixed(V v, Merge merge) {
+  __shared__ V vals[256];
+  vals[threadIdx.x] = v;
+  __syncthreads();
+  for (int stride = 128; stride > 0; stride >>= 1) {
+    if (threadIdx.x < stride) vals[threadIdx.x] = merge(vals[threadIdx.x], vals[threadIdx.x + stride]);
+    __syncthreads();
+  }
+  return vals[0];
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // forward
 // ---------------------------------------------------------------------------------------------------------------------
-template <int S, bool TAPS>
+// Batch-statistics epilogue of the sweep: z = W s + bias -> bf16 (no BatchNorm, no ReLU), and per output channel the mean
+// and M2 of the bf16-rounded z over the tile's 128 pixels: two passes over the registers (the mean first, then the
+// squared deviations from it), not sums of z and z^2, whose difference cancels in fp32.  `red` holds 2 x 8 x 64 floats.
+__device__ __forceinline__ void skipconv_z_epilogue(float (&d)[4][2][4], const float* bias, __nv_bfloat16* op, int hw,
+                                                    int warp, int lane, float* red, float* partial, int cta, int n_ctas) {
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int hrow = 0; hrow < 2; ++hrow) {
+      const int o = mt * 16 + (lane >> 2) + hrow * 8;
+      const float bz = bias != nullptr ? __ldg(bias + o) : 0.f;
+      float sum = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < 2; ++nt) {
+        float* v = &d[mt][nt][hrow * 2];
+        v[0] = __bfloat162float(__float2bfloat16_rn(v[0] + bz));
+        v[1] = __bfloat162float(__float2bfloat16_rn(v[1] + bz));
+        *reinterpret_cast<uint32_t*>(op + static_cast<size_t>(o) * hw + nt * 8) = Elem<__nv_bfloat16>::pack2(v[0], v[1]);
+        sum += v[0] + v[1];
+      }
+      sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+      sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+      if ((lane & 3) == 0) red[warp * kScC + o] = sum;
+    }
+  asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");
+  auto tile_mean = [&](int o) {
+    float s = 0.f;
+#pragma unroll
+    for (int w8 = 0; w8 < 8; ++w8) s += red[w8 * kScC + o];
+    return s * (1.f / kScPB);
+  };
+#pragma unroll
+  for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+    for (int hrow = 0; hrow < 2; ++hrow) {
+      const int o = mt * 16 + (lane >> 2) + hrow * 8;
+      const float mean = tile_mean(o);
+      float q = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const float dv = d[mt][nt][hrow * 2 + e] - mean;
+          q = fmaf(dv, dv, q);
+        }
+      q += __shfl_xor_sync(0xffffffffu, q, 1);
+      q += __shfl_xor_sync(0xffffffffu, q, 2);
+      if ((lane & 3) == 0) red[8 * kScC + warp * kScC + o] = q;
+    }
+  asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");
+  if (threadIdx.x < kScC) {
+    const int o = threadIdx.x;
+    float m2 = 0.f;
+#pragma unroll
+    for (int w8 = 0; w8 < 8; ++w8) m2 += red[8 * kScC + w8 * kScC + o];
+    partial[static_cast<size_t>(o) * n_ctas + cta] = tile_mean(o);
+    partial[static_cast<size_t>(kScC + o) * n_ctas + cta] = m2;
+  }
+}
+
+template <int S, bool TAPS, bool BSTATS>
 __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(const __grid_constant__ CUtensorMap map_x,
                                                                              const __grid_constant__ CUtensorMap map_att,
                                                                              const SkipConvArgs k) {
@@ -362,18 +466,70 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
   float d[4][2][4];
   skipconv_tile_mma(d, k.wfrag, tile, warp, lane);
   T* op = k.out + static_cast<size_t>(b) * kScC * g.hw + static_cast<size_t>(pblk) * kScPB + warp * 16 + (lane & 3) * 2;
+  if constexpr (BSTATS) {  // the stages are drained: every consumer has passed the barrier above
+    skipconv_z_epilogue(d, k.shift, op, g.hw, warp, lane, reinterpret_cast<float*>(pipe_smem), k.partial,
+                        b * gridDim.x + pblk, gridDim.x * gridDim.y);
+  } else {
 #pragma unroll
-  for (int mt = 0; mt < 4; ++mt)
+    for (int mt = 0; mt < 4; ++mt)
 #pragma unroll
-    for (int hrow = 0; hrow < 2; ++hrow) {
-      const int o = mt * 16 + (lane >> 2) + hrow * 8;
-      const float sc = __ldg(k.scale + o), sh = __ldg(k.shift + o);
+      for (int hrow = 0; hrow < 2; ++hrow) {
+        const int o = mt * 16 + (lane >> 2) + hrow * 8;
+        const float sc = __ldg(k.scale + o), sh = __ldg(k.shift + o);
 #pragma unroll
-      for (int nt = 0; nt < 2; ++nt) {
-        const float v0 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2], sh), 0.f), v1 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2 + 1], sh), 0.f);
-        *reinterpret_cast<uint32_t*>(op + static_cast<size_t>(o) * g.hw + nt * 8) = Elem<T>::pack2(v0, v1);
+        for (int nt = 0; nt < 2; ++nt) {
+          const float v0 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2], sh), 0.f), v1 = fmaxf(fmaf(sc, d[mt][nt][hrow * 2 + 1], sh), 0.f);
+          *reinterpret_cast<uint32_t*>(op + static_cast<size_t>(o) * g.hw + nt * 8) = Elem<T>::pack2(v0, v1);
+        }
       }
-    }
+  }
+}
+
+// Chan's parallel merge of (count, mean, M2) summaries
+struct MeanM2 {
+  float n, mean, m2;
+};
+__device__ __forceinline__ MeanM2 chan_merge(const MeanM2& a, const MeanM2& b) {
+  const float n = a.n + b.n;
+  if (b.n == 0.f) return a;
+  const float delta = b.mean - a.mean, fb = b.n / n;
+  return MeanM2{n, fmaf(delta, fb, a.mean), a.m2 + b.m2 + delta * delta * a.n * fb};
+}
+
+// One block per channel: the CTA partials merged in a fixed order (thread i takes CTAs i, i + 256, ...; then a fixed
+// tree), so the statistics are bit-identical from run to run.  Writes the batch mean, the biased variance and the scale /
+// shift of BatchNorm-affine + ReLU.
+__global__ void __launch_bounds__(256) skipconv_bstats_finish_kernel(const float* __restrict__ partial, int n_ctas,
+                                                                     const float* bn_w, const float* bn_b, float eps,
+                                                                     float* mean, float* var, float* scale, float* shift) {
+  const int o = blockIdx.x;
+  MeanM2 acc{0.f, 0.f, 0.f};
+  for (int i = threadIdx.x; i < n_ctas; i += 256)
+    acc = chan_merge(acc, MeanM2{static_cast<float>(kScPB), partial[static_cast<size_t>(o) * n_ctas + i],
+                                 partial[static_cast<size_t>(kScC + o) * n_ctas + i]});
+  acc = block_reduce_fixed(acc, chan_merge);
+  if (threadIdx.x != 0) return;
+  const float v = acc.m2 / acc.n;
+  const float sc = (bn_w ? bn_w[o] : 1.f) / sqrtf(v + eps);
+  mean[o] = acc.mean, var[o] = v;
+  scale[o] = sc, shift[o] = (bn_b ? bn_b[o] : 0.f) - acc.mean * sc;
+}
+
+// out = relu(scale z + shift), 8 bf16 pixels per thread; blockIdx.x = (sample, channel) plane, 32-bit offsets inside it.
+// out may be z (plain loads: no read-only path on data this kernel writes).
+__global__ void __launch_bounds__(256) skipconv_bstats_apply_kernel(const __nv_bfloat16* z, __nv_bfloat16* out,
+                                                                    const float* __restrict__ scale,
+                                                                    const float* __restrict__ shift, int hw_vec) {
+  const int v = blockIdx.y * 256 + threadIdx.x;
+  if (v >= hw_vec) return;
+  const int o = blockIdx.x % kScC;
+  const size_t off = static_cast<size_t>(blockIdx.x) * hw_vec * kScVec + static_cast<uint32_t>(v) * kScVec;
+  const float sc = __ldg(scale + o), sh = __ldg(shift + o);
+  float f[kScVec];
+  Elem<__nv_bfloat16>::unpack(*reinterpret_cast<const uint4*>(z + off), f);
+#pragma unroll
+  for (int j = 0; j < kScVec; ++j) f[j] = fmaxf(fmaf(sc, f[j], sh), 0.f);
+  st_stream_v4(out + off, Elem<__nv_bfloat16>::pack(f));
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -389,18 +545,30 @@ __global__ void __launch_bounds__(kScConsumers + 32, 2) agg_skipconv_kernel(cons
 // with the forward's code in the forward's frame order.  After the sweep, z = W s (hi + lo, the forward's products) gives
 // the BatchNorm sums and g_y s^T the weight gradient; each CTA writes its partials to the workspace and
 // skipconv_bwd_finish_kernel reduces them in a fixed order (deterministic).
+//
+// BSTATS (BatchNorm with batch statistics mean mu and variance var; zhat = (z - mu) / sqrt(var + eps), alpha as above
+// with var):
+//   g_z = alpha * g_z',  g_z' = g_y - mean_N(g_y) - zhat * mean_N(g_y zhat)
+//   grad_s = (alpha W)^T g_z'   grad_conv_weight = alpha * sum_p g_z' s^T   grad_conv_bias = 0
+//   grad_bn_bias = sum g_y      grad_bn_weight = sum g_y zhat
+// The two means are global, so skipconv_bstats_bwd_sums_kernel and its finish run first.  The prologue forms g_z' per
+// pixel in fp32 from grad_out, out and the forward's z; it is not exact in bf16, so it goes to shared memory as bf16 hi +
+// lo tiles and both products (grad_s and g_z' s^T) take the two.  (The expanded form (alpha W)^T g_y - (.. W)^T z + const
+// would lose g_z' to cancellation when grad_out is nearly constant per channel.)  The sweep is unchanged.
 // ---------------------------------------------------------------------------------------------------------------------
-template <int S, bool TAPS>
+template <int S, bool TAPS, bool BSTATS>
 __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_kernel(const __grid_constant__ CUtensorMap map_x,
                                                                                       const __grid_constant__ CUtensorMap map_att,
-                                                                                      const SkipConvBwdArgs a) {
+                                                                                      const SkipConvBwdArgs a,
+                                                                                      const SkipConvBstatsIn<BSTATS> bs) {
   using T = __nv_bfloat16;
   using Geom = SkipGeom<S>;
   constexpr int VEC = kScVec;
   constexpr int M = VEC / S;  // attention cells per thread
   constexpr int NCOL = Geom::NCOL;
   const SkipConvShape& g = a.g;
-  extern __shared__ __align__(128) unsigned char sb_smem[];  // stages | g_y tile (bf16) | grad_s (fp32), later the s tile
+  // stages | g_y tile (bf16; BSTATS: g_z' hi) | grad_s (fp32), later the s tile | BSTATS: g_z' lo tile
+  extern __shared__ __align__(128) unsigned char sb_smem[];
   __shared__ short frames[kAggMaxT];
   __shared__ uint8_t s_pad[kAggMaxT];
   __shared__ int n_frames_s;
@@ -426,26 +594,45 @@ __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_ke
   const uint32_t gs_tile = gy_tile + kScC * kScTileStride;  // grad_s fp32 [64][kScGsStride]; after the sweep the s tile
   float* gs_smem = reinterpret_cast<float*>(sb_smem + n_stages * stage_stride + kScC * kScTileStride);
   const size_t plane = static_cast<size_t>(b) * kScC * g.hw + p0;
+  const uint32_t glo_tile = gs_tile + kScC * kScGsStride * 4;  // BSTATS
 
-  // g_y = grad_out masked by the forward's ReLU decision (bf16, exact) -> shared tile
+  // g_y = grad_out masked by the forward's ReLU decision (bf16, exact) -> shared tile; BSTATS: g_z' as hi + lo tiles
 #pragma unroll
   for (int c = 0; c < 4; ++c) {
-    const size_t off = plane + static_cast<size_t>(head * 4 + c) * g.hw;
-    const uint4 gv = ld_stream_v4(a.gout + off), o = ld_stream_v4(a.out + off);
-    const uint32_t gw[4] = {gv.x, gv.y, gv.z, gv.w}, ow[4] = {o.x, o.y, o.z, o.w};
-    uint32_t m[4];
+    const int ch = head * 4 + c;
+    const size_t off = plane + static_cast<size_t>(ch) * g.hw;
+    if constexpr (BSTATS) {
+      float gf[VEC], zf[VEC], hi[VEC], lo[VEC];
+      Elem<T>::unpack(relu_masked(ld_stream_v4(a.gout + off), ld_stream_v4(a.out + off)), gf);
+      Elem<T>::unpack(ld_stream_v4(bs.z + off), zf);
+      const float is = __ldg(bs.inv_std + ch), zs = __ldg(a.zshift + ch);
+      const float m1 = __ldg(bs.gmean + ch), m2 = __ldg(bs.gmean + kScC + ch);
 #pragma unroll
-    for (int q = 0; q < 4; ++q) {  // bf16 pairs: a positive bf16 has a clear sign bit and a non-zero magnitude
-      const uint32_t lo_pos = ((ow[q] & 0x8000u) == 0 && (ow[q] & 0x7fffu) != 0) ? 0x0000ffffu : 0u;
-      const uint32_t hi_pos = ((ow[q] & 0x80000000u) == 0 && (ow[q] & 0x7fff0000u) != 0) ? 0xffff0000u : 0u;
-      m[q] = gw[q] & (lo_pos | hi_pos);
+      for (int j = 0; j < VEC; ++j) {
+        const float gz = gf[j] - m1 - (zf[j] + zs) * is * m2;
+        hi[j] = __bfloat162float(__float2bfloat16_rn(gz));
+        lo[j] = gz - hi[j];
+      }
+      sts_v4(gy_tile + ch * kScTileStride + pv * 16, Elem<T>::pack(hi));
+      sts_v4(glo_tile + ch * kScTileStride + pv * 16, Elem<T>::pack(lo));
+    } else {
+      sts_v4(gy_tile + ch * kScTileStride + pv * 16, relu_masked(ld_stream_v4(a.gout + off), ld_stream_v4(a.out + off)));
     }
-    sts_v4(gy_tile + (head * 4 + c) * kScTileStride + pv * 16, make_uint4(m[0], m[1], m[2], m[3]));
   }
   asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");  // consumers only (the producer warp has its own loop)
-  {  // grad_s = (alpha W)^T g_y -> shared memory (fp32)
+  {  // grad_s = (alpha W)^T g_y (BSTATS: g_z' hi + lo) -> shared memory (fp32)
     float d[4][2][4];
     skipconv_tile_mma(d, a.afrag, gy_tile, warp, lane);
+    if constexpr (BSTATS) {
+      float dl[4][2][4];
+      skipconv_tile_mma(dl, a.afrag, glo_tile, warp, lane);
+#pragma unroll
+      for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+          for (int e = 0; e < 4; ++e) d[mt][nt][e] += dl[mt][nt][e];
+    }
 #pragma unroll
     for (int mt = 0; mt < 4; ++mt)
 #pragma unroll
@@ -572,7 +759,7 @@ __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_ke
   asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");
   float* part = a.partial + (static_cast<size_t>(b) * gridDim.x + pblk) * kScPartial;
   float(*red)[8][kScC] = reinterpret_cast<float(*)[8][kScC]>(sb_smem);  // per-warp sums; the stages are drained by now
-  {  // z - mean = W s + (bias - mean): sums of g_y and g_y (z - mean) per output channel
+  if constexpr (!BSTATS) {  // z - mean = W s + (bias - mean): sums of g_y and g_y (z - mean) per output channel
     float d[4][2][4];
     skipconv_tile_mma(d, a.wfrag, s_tile, warp, lane);
     const unsigned char* gyb = sb_smem + n_stages * stage_stride;
@@ -608,8 +795,9 @@ __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_ke
       for (int e = 0; e < 4; ++e) d[n][e] = 0.f;
 #pragma unroll
     for (int ks = 0; ks < kScPB / 16; ++ks) {
-      uint32_t af[4];
+      uint32_t af[4], al[4];
       ldsm_x4(af, gy_tile + (mt * 16 + (lane & 15)) * kScTileStride + (ks * 16 + (lane >> 4) * 8) * 2);
+      if constexpr (BSTATS) ldsm_x4(al, glo_tile + (mt * 16 + (lane & 15)) * kScTileStride + (ks * 16 + (lane >> 4) * 8) * 2);
 #pragma unroll
       for (int np = 0; np < 2; ++np) {  // two n-tiles per ldmatrix.x4: (n 0-7 | 8-15) x (k 0-7 | 8-15)
         uint32_t bf[4];
@@ -617,6 +805,10 @@ __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_ke
         ldsm_x4(bf, s_tile + crow * kScTileStride + (ks * 16 + ((lane >> 3) & 1) * 8) * 2);
         mma_bf16(d[2 * np], af, bf[0], bf[1]);
         mma_bf16(d[2 * np + 1], af, bf[2], bf[3]);
+        if constexpr (BSTATS) {
+          mma_bf16(d[2 * np], al, bf[0], bf[1]);
+          mma_bf16(d[2 * np + 1], al, bf[2], bf[3]);
+        }
       }
     }
 #pragma unroll
@@ -627,6 +819,7 @@ __global__ void __launch_bounds__(kScConsumers + 32, 1) agg_skipconv_backward_ke
         *reinterpret_cast<float2*>(part + o * kScC + c) = make_float2(d[n][hrow * 2], d[n][hrow * 2 + 1]);
       }
   }
+  if constexpr (BSTATS) return;  // the BatchNorm sums came from skipconv_bstats_bwd_sums_kernel
   asm volatile("bar.sync 1, %0;" ::"n"(kScConsumers) : "memory");
   if (threadIdx.x < 2 * kScC) {  // fixed order over the warps
     const int q = threadIdx.x / kScC, o = threadIdx.x % kScC;
@@ -665,6 +858,58 @@ __global__ void __launch_bounds__(256) skipconv_bwd_finish_kernel(const float* _
     const int o = e - kScC * kScC - kScC;
     if (gbn_w != nullptr) gbn_w[o] = inv_std[o] * total;
   }
+}
+
+// BSTATS pre-pass with the main kernel's tiling (one sample x 128 pixels; thread = 4 channels x 8 pixels): per CTA and
+// channel, sum g_y and sum g_y zhat -> partial [2][64][CTAs]
+__global__ void __launch_bounds__(kScConsumers) skipconv_bstats_bwd_sums_kernel(
+    const __nv_bfloat16* __restrict__ gout, const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __restrict__ z,
+    const float* __restrict__ inv_std, const float* __restrict__ zshift, int hw, float* __restrict__ partial) {
+  const int head = threadIdx.x >> 4, pv = threadIdx.x & 15;
+  const int n_ctas = gridDim.x * gridDim.y, cta = blockIdx.y * gridDim.x + blockIdx.x;
+  const size_t plane = static_cast<size_t>(blockIdx.y) * kScC * hw + blockIdx.x * kScPB + pv * kScVec;
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    const int ch = head * 4 + c;
+    const size_t off = plane + static_cast<size_t>(ch) * hw;
+    float gf[kScVec], zf[kScVec];
+    Elem<__nv_bfloat16>::unpack(relu_masked(ld_stream_v4(gout + off), ld_stream_v4(out + off)), gf);
+    Elem<__nv_bfloat16>::unpack(ld_stream_v4(z + off), zf);
+    const float is = __ldg(inv_std + ch), zs = __ldg(zshift + ch);
+    float sg = 0.f, sgz = 0.f;
+#pragma unroll
+    for (int j = 0; j < kScVec; ++j) {
+      sg += gf[j];
+      sgz = fmaf(gf[j], (zf[j] + zs) * is, sgz);
+    }
+#pragma unroll
+    for (int m = 1; m < 16; m <<= 1) {  // the 16 lanes of this channel group, fixed order
+      sg += __shfl_xor_sync(0xffffffffu, sg, m);
+      sgz += __shfl_xor_sync(0xffffffffu, sgz, m);
+    }
+    if (pv == 0) {
+      partial[static_cast<size_t>(ch) * n_ctas + cta] = sg;
+      partial[static_cast<size_t>(kScC + ch) * n_ctas + cta] = sgz;
+    }
+  }
+}
+
+// One block per channel, fixed order: grad_bn_bias = sum g_y, grad_bn_weight = sum g_y zhat, and their means over the
+// N = B H W pixels for the main kernel's g_z'
+__global__ void __launch_bounds__(256) skipconv_bstats_bwd_means_kernel(const float* __restrict__ partial, int n_ctas,
+                                                                        float* gmean, float* gbn_w, float* gbn_b) {
+  const int o = blockIdx.x;
+  float2 acc = make_float2(0.f, 0.f);
+  for (int i = threadIdx.x; i < n_ctas; i += 256) {
+    acc.x += partial[static_cast<size_t>(o) * n_ctas + i];
+    acc.y += partial[static_cast<size_t>(kScC + o) * n_ctas + i];
+  }
+  acc = block_reduce_fixed(acc, [](float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); });
+  if (threadIdx.x != 0) return;
+  const float inv_n = 1.f / (static_cast<float>(n_ctas) * kScPB);
+  gmean[o] = acc.x * inv_n, gmean[kScC + o] = acc.y * inv_n;
+  if (gbn_b != nullptr) gbn_b[o] = acc.x;
+  if (gbn_w != nullptr) gbn_w[o] = acc.y;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -728,39 +973,51 @@ int skipconv_plan(const c2s_agg_desc* d, const void* x, const float* attn, std::
                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, "attention");
 }
 
-template <int S, bool TAPS>
+template <int S, bool TAPS, bool BSTATS>
 int launch_skipconv_t(const SkipConvPlan& p, const SkipConvArgs& k, cudaStream_t stream, const char* name) {
   const size_t smem = static_cast<size_t>(k.g.n_stages) * (kScStageBytes + 16 * k.g.tap_floats * 4) + kScC * kScTileStride;
-  C2S_SMEM_ATTR((agg_skipconv_kernel<S, TAPS>), 227 * 1024);  // once per instantiation and device (smem varies per call)
+  C2S_SMEM_ATTR((agg_skipconv_kernel<S, TAPS, BSTATS>), 227 * 1024);  // once per instantiation and device (smem varies per call)
   dim3 grid(k.g.hw / kScPB, k.g.B);
-  agg_skipconv_kernel<S, TAPS><<<grid, kScConsumers + 32, smem, stream>>>(p.map_x, p.map_att, k);
+  agg_skipconv_kernel<S, TAPS, BSTATS><<<grid, kScConsumers + 32, smem, stream>>>(p.map_x, p.map_att, k);
   C2S_LAUNCH_CHECK(name);
   return C2S_OK;
 }
 
-template <int S>
+template <int S, bool BSTATS>
 int launch_skipconv(const SkipConvPlan& p, const SkipConvArgs& k, cudaStream_t stream, const char* name) {
-  return k.g.tap_floats > 0 ? launch_skipconv_t<S, true>(p, k, stream, name) : launch_skipconv_t<S, false>(p, k, stream, name);
+  return k.g.tap_floats > 0 ? launch_skipconv_t<S, true, BSTATS>(p, k, stream, name)
+                            : launch_skipconv_t<S, false, BSTATS>(p, k, stream, name);
 }
 
-size_t skipconv_bwd_smem(int n_stages, int tap_floats) {  // stages | g_y tile | grad_s (then s) tile
-  return static_cast<size_t>(n_stages) * (kScStageBytes + 16 * tap_floats * 4) + kScC * kScTileStride + kScC * kScGsStride * 4;
+// stages | g_y tile | grad_s (then s) tile | BSTATS: g_z' lo tile
+size_t skipconv_bwd_smem(int n_stages, int tap_floats, bool bstats) {
+  return static_cast<size_t>(n_stages) * (kScStageBytes + 16 * tap_floats * 4) + kScC * kScTileStride + kScC * kScGsStride * 4 +
+         (bstats ? kScC * kScTileStride : 0);
 }
 
-template <int S, bool TAPS>
-int launch_skipconv_bwd_t(const SkipConvPlan& p, const SkipConvBwdArgs& k, cudaStream_t stream, const char* name) {
-  const size_t smem = skipconv_bwd_smem(k.g.n_stages, k.g.tap_floats);
-  C2S_SMEM_ATTR((agg_skipconv_backward_kernel<S, TAPS>), 227 * 1024);  // once per instantiation and device
+template <int S, bool TAPS, bool BSTATS>
+int launch_skipconv_bwd_t(const SkipConvPlan& p, const SkipConvBwdArgs& k, const SkipConvBstatsIn<BSTATS>& bs,
+                          cudaStream_t stream, const char* name) {
+  const size_t smem = skipconv_bwd_smem(k.g.n_stages, k.g.tap_floats, BSTATS);
+  C2S_SMEM_ATTR((agg_skipconv_backward_kernel<S, TAPS, BSTATS>), 227 * 1024);  // once per instantiation and device
   dim3 grid(k.g.hw / kScPB, k.g.B);
-  agg_skipconv_backward_kernel<S, TAPS><<<grid, kScConsumers + 32, smem, stream>>>(p.map_x, p.map_att, k);
+  agg_skipconv_backward_kernel<S, TAPS, BSTATS><<<grid, kScConsumers + 32, smem, stream>>>(p.map_x, p.map_att, k, bs);
   C2S_LAUNCH_CHECK(name);
   return C2S_OK;
 }
 
-template <int S>
-int launch_skipconv_bwd(const SkipConvPlan& p, const SkipConvBwdArgs& k, cudaStream_t stream, const char* name) {
-  return k.g.tap_floats > 0 ? launch_skipconv_bwd_t<S, true>(p, k, stream, name)
-                            : launch_skipconv_bwd_t<S, false>(p, k, stream, name);
+template <int S, bool BSTATS>
+int launch_skipconv_bwd(const SkipConvPlan& p, const SkipConvBwdArgs& k, const SkipConvBstatsIn<BSTATS>& bs,
+                        cudaStream_t stream, const char* name) {
+  return k.g.tap_floats > 0 ? launch_skipconv_bwd_t<S, true, BSTATS>(p, k, bs, stream, name)
+                            : launch_skipconv_bwd_t<S, false, BSTATS>(p, k, bs, stream, name);
+}
+
+// stages for the backward's ring: fewer if the staged rows make them too large for one CTA (227 KB with the static part)
+int skipconv_bwd_stages(int tap_floats, bool bstats) {
+  int n = kScMaxStages;
+  while (n > 2 && skipconv_bwd_smem(n, tap_floats, bstats) > 220 * 1024) --n;
+  return n;
 }
 
 // backward workspace: W and (alpha W)^T fragments, alpha / inv_std / zshift, then the CTA partials (16-byte aligned throughout)
@@ -768,6 +1025,11 @@ constexpr size_t kScBwdFixedBytes = 2 * 2 * kScFrags * sizeof(uint4) + 3 * kScC 
 size_t skipconv_bwd_ctas(const c2s_agg_desc* d) {
   return d->B > 0 && d->H > 0 && d->W > 0 ? static_cast<size_t>(d->B) * ((static_cast<size_t>(d->H) * d->W) / kScPB) : 0;
 }
+// batch-statistics forward workspace: W fragments, scale, shift, then the [mean | M2][64][CTAs] partials
+constexpr size_t kScBstatsFixedBytes = 2 * kScFrags * sizeof(uint4) + 2 * kScC * sizeof(float);
+// batch-statistics backward workspace: the backward's fixed part, the two g_y means [2][64], the main kernel's CTA partials
+// (kScPartial floats each, of which the 64 x 64 weight term is used), then the pre-pass partials [2][64][CTAs]
+constexpr size_t kScBstatsBwdFixedBytes = kScBwdFixedBytes + 2 * kScC * sizeof(float);
 
 }  // namespace
 }  // namespace c2s
@@ -813,9 +1075,9 @@ int c2s_agg_skipconv_forward(const c2s_agg_desc* d, const void* x, const float* 
   k.attn = attn, k.pad = pad_mask, k.out = static_cast<__nv_bfloat16*>(out);
   k.wfrag = wfrag, k.scale = scale, k.shift = shift;
   switch (plan.scale_class) {
-    case 2: return launch_skipconv<2>(plan, k, stream, "agg_skipconv<x2>");
-    case 4: return launch_skipconv<4>(plan, k, stream, "agg_skipconv<x4>");
-    default: return launch_skipconv<8>(plan, k, stream, "agg_skipconv<x8>");
+    case 2: return launch_skipconv<2, false>(plan, k, stream, "agg_skipconv<x2>");
+    case 4: return launch_skipconv<4, false>(plan, k, stream, "agg_skipconv<x4>");
+    default: return launch_skipconv<8, false>(plan, k, stream, "agg_skipconv<x8>");
   }
 }
 
@@ -861,22 +1123,154 @@ int c2s_agg_skipconv_backward(const c2s_agg_desc* d, const void* x, const float*
 
   SkipConvBwdArgs k{};
   k.g = plan.g;
-  k.g.n_stages = kScMaxStages;  // fewer if the staged rows make them too large for one CTA (227 KB with the static part)
-  while (k.g.n_stages > 2 && skipconv_bwd_smem(k.g.n_stages, k.g.tap_floats) > 220 * 1024) --k.g.n_stages;
+  k.g.n_stages = skipconv_bwd_stages(k.g.tap_floats, false);
   k.attn = attn, k.pad = pad_mask;
   k.out = static_cast<const __nv_bfloat16*>(out), k.gout = static_cast<const __nv_bfloat16*>(grad_out);
   k.gx = static_cast<__nv_bfloat16*>(io->grad_x), k.gattn = io->grad_attn;
   k.wfrag = wfrag, k.afrag = afrag, k.zshift = zshift, k.partial = want_params ? partial : nullptr;
   switch (plan.scale_class) {
-    case 2: status = launch_skipconv_bwd<2>(plan, k, stream, "agg_skipconv_backward<x2>"); break;
-    case 4: status = launch_skipconv_bwd<4>(plan, k, stream, "agg_skipconv_backward<x4>"); break;
-    default: status = launch_skipconv_bwd<8>(plan, k, stream, "agg_skipconv_backward<x8>"); break;
+    case 2: status = launch_skipconv_bwd<2, false>(plan, k, {}, stream, "agg_skipconv_backward<x2>"); break;
+    case 4: status = launch_skipconv_bwd<4, false>(plan, k, {}, stream, "agg_skipconv_backward<x4>"); break;
+    default: status = launch_skipconv_bwd<8, false>(plan, k, {}, stream, "agg_skipconv_backward<x8>"); break;
   }
   if (status != C2S_OK || !want_params) return status;
   skipconv_bwd_finish_kernel<<<ceil_div(kScPartial, 32), 256, 0, stream>>>(
       partial, static_cast<int>(skipconv_bwd_ctas(d)), alpha, inv_std, io->grad_conv_weight, io->grad_conv_bias,
       io->grad_bn_weight, io->grad_bn_bias);
   C2S_LAUNCH_CHECK("agg_skipconv_backward<reduce>");
+  return C2S_OK;
+}
+
+size_t c2s_agg_skipconv_bstats_workspace_bytes(const c2s_agg_desc* d) {
+  if (d == nullptr) return 0;
+  return c2s::kScBstatsFixedBytes + c2s::skipconv_bwd_ctas(d) * 2 * c2s::kScC * sizeof(float);
+}
+
+int c2s_agg_skipconv_bstats_forward(const c2s_agg_desc* d, const void* x, const float* attn, const uint8_t* pad_mask,
+                                    const c2s_skipconv_params* p, void* z, void* out, float* bn_batch_mean,
+                                    float* bn_batch_var, void* workspace, size_t workspace_bytes, void* stream_ptr) {
+  using namespace c2s;
+  C2S_CHECK_ARG(d != nullptr && p != nullptr, "c2s_agg_skipconv_bstats_forward: desc/params is NULL");
+  C2S_CHECK_ARG(x != nullptr && attn != nullptr && z != nullptr && out != nullptr && bn_batch_mean != nullptr &&
+                    bn_batch_var != nullptr && p->conv_weight != nullptr,
+                "c2s_agg_skipconv_bstats_forward: x/attn/z/out/bn_batch_mean/bn_batch_var/conv_weight is NULL");
+  C2S_CHECK_ARG(d->B > 0 && d->T > 0 && d->H > 0 && d->W > 0, "c2s_agg_skipconv_bstats_forward: non-positive dimension");
+  SkipConvPlan plan;
+  int status = skipconv_plan(d, x, attn, {x, z, out}, /*staged_taps_at_x2=*/false, &plan);
+  if (status == kScNotServed)
+    C2S_UNSUPPORTED("c2s_agg_skipconv_bstats_forward: the fused path serves att_group, bf16, C=64, 16 heads, x2/x4/x8 "
+                    "up-sampling, H*W %% 128 == 0 (got mode %d dtype %d C %d heads %d %dx%d from %dx%d); run c2s_agg_forward "
+                    "and the convolution separately", d->mode, d->dtype, d->C, d->n_heads, d->H, d->W, d->ha, d->wa);
+  if (status != C2S_OK) return status;
+  const size_t need = c2s_agg_skipconv_bstats_workspace_bytes(d);
+  C2S_CHECK_ARG(workspace != nullptr && workspace_bytes >= need && reinterpret_cast<uintptr_t>(workspace) % 16 == 0,
+                "c2s_agg_skipconv_bstats_forward: needs %zu workspace bytes, 16-byte aligned", need);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
+  const int n_ctas = static_cast<int>(skipconv_bwd_ctas(d));
+
+  uint4* wfrag = static_cast<uint4*>(workspace);
+  float* scale = reinterpret_cast<float*>(wfrag + 2 * kScFrags);
+  float* shift = scale + kScC;
+  float* partial = reinterpret_cast<float*>(static_cast<char*>(workspace) + kScBstatsFixedBytes);
+  // blocks 0-1 only: the W fragments (block 2 would read the running statistics)
+  skipconv_prep_kernel<<<2, 256, 0, stream>>>(p->conv_weight, wfrag, nullptr, nullptr, nullptr, nullptr, nullptr, 0.f,
+                                              nullptr, nullptr);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats<prep>");
+  SkipConvArgs k{};
+  k.g = plan.g;
+  k.g.n_stages = 4;
+  k.attn = attn, k.pad = pad_mask, k.out = static_cast<__nv_bfloat16*>(z);
+  k.wfrag = wfrag, k.shift = p->conv_bias, k.partial = partial;
+  switch (plan.scale_class) {
+    case 2: status = launch_skipconv<2, true>(plan, k, stream, "agg_skipconv_bstats<x2>"); break;
+    case 4: status = launch_skipconv<4, true>(plan, k, stream, "agg_skipconv_bstats<x4>"); break;
+    default: status = launch_skipconv<8, true>(plan, k, stream, "agg_skipconv_bstats<x8>"); break;
+  }
+  if (status != C2S_OK) return status;
+  skipconv_bstats_finish_kernel<<<kScC, 256, 0, stream>>>(partial, n_ctas, p->bn_weight, p->bn_bias, p->bn_eps,
+                                                          bn_batch_mean, bn_batch_var, scale, shift);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats<stats>");
+  const int hw_vec = plan.g.hw / kScVec;
+  skipconv_bstats_apply_kernel<<<dim3(d->B * kScC, ceil_div(hw_vec, 256)), 256, 0, stream>>>(
+      static_cast<const __nv_bfloat16*>(z), static_cast<__nv_bfloat16*>(out), scale, shift, hw_vec);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats<apply>");
+  return C2S_OK;
+}
+
+size_t c2s_agg_skipconv_bstats_backward_workspace_bytes(const c2s_agg_desc* d) {
+  if (d == nullptr) return 0;
+  return c2s::kScBstatsBwdFixedBytes + c2s::skipconv_bwd_ctas(d) * (c2s::kScPartial + 2 * c2s::kScC) * sizeof(float);
+}
+
+int c2s_agg_skipconv_bstats_backward(const c2s_agg_desc* d, const void* x, const float* attn, const uint8_t* pad_mask,
+                                     const c2s_skipconv_params* p, const void* z, const float* bn_batch_mean,
+                                     const float* bn_batch_var, const void* out, const void* grad_out,
+                                     const c2s_skipconv_bwd_io* io, void* workspace, size_t workspace_bytes,
+                                     void* stream_ptr) {
+  using namespace c2s;
+  C2S_CHECK_ARG(d != nullptr && p != nullptr && io != nullptr, "c2s_agg_skipconv_bstats_backward: desc/params/io is NULL");
+  C2S_CHECK_ARG(x != nullptr && attn != nullptr && z != nullptr && bn_batch_mean != nullptr && bn_batch_var != nullptr &&
+                    out != nullptr && grad_out != nullptr && p->conv_weight != nullptr,
+                "c2s_agg_skipconv_bstats_backward: x/attn/z/bn_batch_mean/bn_batch_var/out/grad_out/conv_weight is NULL");
+  C2S_CHECK_ARG(d->B > 0 && d->T > 0 && d->H > 0 && d->W > 0, "c2s_agg_skipconv_bstats_backward: non-positive dimension");
+  SkipConvPlan plan;
+  int status = skipconv_plan(d, x, attn, {x, z, out, grad_out, io->grad_x}, /*staged_taps_at_x2=*/true, &plan);
+  C2S_CHECK_ARG(status != kScNotServed,
+                "c2s_agg_skipconv_bstats_backward: the fused backward serves what the fused forward serves: att_group, "
+                "bf16, C=64, 16 heads, x2/x4/x8 up-sampling, H*W %% 128 == 0, 16-byte aligned tensors (got mode %d dtype "
+                "%d C %d heads %d %dx%d from %dx%d)", d->mode, d->dtype, d->C, d->n_heads, d->H, d->W, d->ha, d->wa);
+  if (status != C2S_OK) return status;
+  const bool want_main = io->grad_x != nullptr || io->grad_attn != nullptr || io->grad_conv_weight != nullptr;
+  const bool want_bn = io->grad_bn_weight != nullptr || io->grad_bn_bias != nullptr;
+  if (!want_main && !want_bn && io->grad_conv_bias == nullptr) return C2S_OK;  // nothing asked for
+  const size_t need = c2s_agg_skipconv_bstats_backward_workspace_bytes(d);
+  C2S_CHECK_ARG(workspace != nullptr && workspace_bytes >= need && reinterpret_cast<uintptr_t>(workspace) % 16 == 0,
+                "c2s_agg_skipconv_bstats_backward: needs %zu workspace bytes, 16-byte aligned", need);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_ptr);
+  // batch statistics remove any per-channel constant of z, so the convolution bias has no effect on the output
+  if (io->grad_conv_bias != nullptr) C2S_CUDA(cudaMemsetAsync(io->grad_conv_bias, 0, kScC * sizeof(float), stream));
+  if (!want_main && !want_bn) return C2S_OK;
+  const int n_ctas = static_cast<int>(skipconv_bwd_ctas(d));
+
+  uint4* wfrag = static_cast<uint4*>(workspace);
+  uint4* afrag = wfrag + 2 * kScFrags;
+  float* alpha = reinterpret_cast<float*>(afrag + 2 * kScFrags);
+  float* inv_std = alpha + kScC;
+  float* zshift = inv_std + kScC;
+  float* gmean = zshift + kScC;
+  float* partial = reinterpret_cast<float*>(static_cast<char*>(workspace) + kScBstatsBwdFixedBytes);
+  float* sums = partial + static_cast<size_t>(n_ctas) * kScPartial;
+  // the eval backward's preparation on the batch statistics, without the conv bias: zshift = -mean, alpha = gamma inv_std
+  skipconv_bwd_prep_kernel<<<3, 256, 0, stream>>>(p->conv_weight, nullptr, p->bn_weight, bn_batch_mean, bn_batch_var,
+                                                  p->bn_eps, wfrag, afrag, alpha, inv_std, zshift);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats_backward<prep>");
+  const dim3 grid(plan.g.hw / kScPB, d->B);
+  skipconv_bstats_bwd_sums_kernel<<<grid, kScConsumers, 0, stream>>>(
+      static_cast<const __nv_bfloat16*>(grad_out), static_cast<const __nv_bfloat16*>(out),
+      static_cast<const __nv_bfloat16*>(z), inv_std, zshift, plan.g.hw, sums);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats_backward<sums>");
+  skipconv_bstats_bwd_means_kernel<<<kScC, 256, 0, stream>>>(sums, n_ctas, gmean, io->grad_bn_weight, io->grad_bn_bias);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats_backward<means>");
+  if (!want_main) return C2S_OK;
+
+  SkipConvBwdArgs k{};
+  k.g = plan.g;
+  k.g.n_stages = skipconv_bwd_stages(k.g.tap_floats, true);
+  k.attn = attn, k.pad = pad_mask;
+  k.out = static_cast<const __nv_bfloat16*>(out), k.gout = static_cast<const __nv_bfloat16*>(grad_out);
+  k.gx = static_cast<__nv_bfloat16*>(io->grad_x), k.gattn = io->grad_attn;
+  k.wfrag = wfrag, k.afrag = afrag, k.zshift = zshift, k.partial = io->grad_conv_weight != nullptr ? partial : nullptr;
+  const SkipConvBstatsIn<true> bs{static_cast<const __nv_bfloat16*>(z), inv_std, gmean};
+  switch (plan.scale_class) {
+    case 2: status = launch_skipconv_bwd<2, true>(plan, k, bs, stream, "agg_skipconv_bstats_backward<x2>"); break;
+    case 4: status = launch_skipconv_bwd<4, true>(plan, k, bs, stream, "agg_skipconv_bstats_backward<x4>"); break;
+    default: status = launch_skipconv_bwd<8, true>(plan, k, bs, stream, "agg_skipconv_bstats_backward<x8>"); break;
+  }
+  if (status != C2S_OK || io->grad_conv_weight == nullptr) return status;
+  // the 64 x 64 weight entries only: grad_conv_weight = alpha sum g_z' s^T
+  skipconv_bwd_finish_kernel<<<kScC * kScC / 32, 256, 0, stream>>>(partial, n_ctas, alpha, inv_std, io->grad_conv_weight,
+                                                                   nullptr, nullptr, nullptr);
+  C2S_LAUNCH_CHECK("agg_skipconv_bstats_backward<reduce>");
   return C2S_OK;
 }
 

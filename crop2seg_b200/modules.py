@@ -255,6 +255,18 @@ class _LTAEBase(nn.Module):
                     raise RuntimeError("Class values must be smaller than num_classes.")
 
 
+@torch.no_grad()
+def _update_running_stats(bn, stats, n_rows):
+    """Train-mode bookkeeping of nn.BatchNorm1d / BatchNorm2d from the batch mean and biased variance over ``n_rows``
+    values per channel (momentum or, with momentum=None, the cumulative average; unbiased variance) -- tae.py:445."""
+    mean, var = stats
+    bn.num_batches_tracked += 1
+    momentum = bn.momentum if bn.momentum is not None else 1.0 / float(bn.num_batches_tracked)
+    unbiased = var * (n_rows / max(n_rows - 1, 1))
+    bn.running_mean.mul_(1 - momentum).add_(mean.to(bn.running_mean.dtype), alpha=momentum)
+    bn.running_var.mul_(1 - momentum).add_(unbiased.to(bn.running_var.dtype), alpha=momentum)
+
+
 class LTAE(_LTAEBase):
     """Lightweight Temporal Attention Encoder -- drop-in for ``src.backbones.tae.LTAE`` (tae.py:349)."""
 
@@ -335,19 +347,8 @@ class LTAE(_LTAEBase):
             out, attn, stats = ops.ltae_forward(x, batch_positions, pad_mask, params, spec, need_attn=return_att,
                                                 attn_keep=attn_keep, mlp_keep=mlp_keep, **self._folded_args(params))[:3]
         if stats is not None and self.training and self.mlp[2].track_running_stats:
-            self._update_running_stats(self.mlp[2], stats, b * h * w)
+            _update_running_stats(self.mlp[2], stats, b * h * w)
         return out, (attn if return_att else None)
-
-    @staticmethod
-    @torch.no_grad()
-    def _update_running_stats(bn, stats, n_rows):
-        """nn.BatchNorm1d train-mode bookkeeping (momentum, unbiased variance) -- tae.py:445."""
-        mean, var = stats
-        bn.num_batches_tracked += 1
-        momentum = bn.momentum if bn.momentum is not None else 1.0 / float(bn.num_batches_tracked)
-        unbiased = var * (n_rows / max(n_rows - 1, 1))
-        bn.running_mean.mul_(1 - momentum).add_(mean.to(bn.running_mean.dtype), alpha=momentum)
-        bn.running_var.mul_(1 - momentum).add_(unbiased.to(bn.running_var.dtype), alpha=momentum)
 
 
 class LTAE4WTAE(_LTAEBase):
@@ -392,14 +393,17 @@ class TemporalAggregator(nn.Module):
             return None  # the reference falls through its if/elif chain and returns None
         return ops.temporal_aggregate(x, pad_mask=pad_mask, attn_mask=attn_mask, mode=self.mode)
 
-    def forward_skip_conv(self, x, pad_mask, attn_mask, skip_conv):
+    def forward_skip_conv(self, x, pad_mask, attn_mask, skip_conv, allow_batch_stats=False):
         """``skip_conv(self(x, pad_mask, attn_mask))`` in one kernel, for the decoder's ``UpConvBlock.skip_conv`` =
         ``Sequential(Conv2d(d, d, 1), BatchNorm2d(d), ReLU())`` (conv.py:378-382; SURVEY.md section 8f, rank 1).
 
-        ``skip_conv`` in eval mode (running statistics); ``att_group``, bf16 features with 64 channels.  Differentiable
-        w.r.t. x, attn_mask and the convolution / BatchNorm affine parameters with the BatchNorm frozen (fine-tuning
-        with the decoder's BatchNorm in eval mode); batch statistics are not served.  A maintainer replaces ``self.up_blocks[i](out, skip)`` by the block's own forward with the already-convolved
-        skip (INTEGRATION.md, "Fused skip convolution").
+        ``att_group``, bf16 features with 64 channels.  Differentiable w.r.t. x, attn_mask and the convolution /
+        BatchNorm affine parameters.  By default ``skip_conv`` must be in eval mode (running statistics), so that a model
+        left in ``train()`` never rewrites its running statistics unnoticed.  ``allow_batch_stats=True`` does what
+        ``skip_conv`` itself does in its current mode: batch statistics when ``bn.training or not
+        bn.track_running_stats`` (the running statistics are updated when the BatchNorm is training and tracks them),
+        running statistics otherwise.  A maintainer replaces ``self.up_blocks[i](out, skip)`` by the block's own forward
+        with the already-convolved skip (INTEGRATION.md, "Fused skip convolution").
         """
         if self.mode != "att_group":
             raise NotImplementedError("forward_skip_conv: only the att_group mode has a fused kernel")
@@ -408,7 +412,20 @@ class TemporalAggregator(nn.Module):
             raise TypeError("forward_skip_conv expects Sequential(Conv2d(d, d, 1), BatchNorm2d(d), ReLU())")
         if conv.kernel_size != (1, 1) or conv.stride != (1, 1) or conv.groups != 1:
             raise NotImplementedError("forward_skip_conv: the skip convolution must be a plain 1x1 convolution")
-        if bn.training or bn.running_mean is None:
-            raise RuntimeError("forward_skip_conv is an inference path: put skip_conv in eval mode (running statistics)")
-        return ops.temporal_aggregate_skip_conv(x, pad_mask, attn_mask, conv.weight, conv.bias, bn.weight, bn.bias,
-                                                bn.running_mean, bn.running_var, bn.eps)
+        if not (bn.training or bn.running_mean is None):
+            return ops.temporal_aggregate_skip_conv(x, pad_mask, attn_mask, conv.weight, conv.bias, bn.weight, bn.bias,
+                                                    bn.running_mean, bn.running_var, bn.eps)
+        if not allow_batch_stats:
+            raise RuntimeError("forward_skip_conv is an inference path by default: put skip_conv in eval mode (running "
+                               "statistics), or pass allow_batch_stats=True to normalise with batch statistics")
+        params = (conv.weight, conv.bias, bn.weight, bn.bias)
+        if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (x, attn_mask) + params):
+            from .autograd import AggregateSkipConvBatchStatsFunction
+            out, mean, var = AggregateSkipConvBatchStatsFunction.apply(x, attn_mask, pad_mask, *params, bn.eps)
+        else:
+            out, _, mean, var = ops.temporal_aggregate_skip_conv_bstats_forward(x, pad_mask, attn_mask, *params, bn.eps,
+                                                                                keep_z=False)
+        if bn.training and bn.track_running_stats:
+            b, _, _, h, w = x.shape
+            _update_running_stats(bn, (mean, var), b * h * w)
+        return out

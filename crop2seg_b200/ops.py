@@ -224,6 +224,75 @@ def temporal_aggregate_skip_conv_backward(x: torch.Tensor, pad_mask: Optional[to
     return tuple(res)
 
 
+def temporal_aggregate_skip_conv_bstats_forward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: torch.Tensor,
+                                                conv_weight: torch.Tensor, conv_bias: Optional[torch.Tensor],
+                                                bn_weight: Optional[torch.Tensor], bn_bias: Optional[torch.Tensor],
+                                                bn_eps: float = 1e-5, keep_z: bool = True
+                                                ) -> Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, torch.Tensor]:
+    """``relu(BatchNorm2d_train(Conv2d_1x1(TemporalAggregator('att_group')(x, pad_mask, attn_mask))))`` with the
+    BatchNorm normalising by the batch statistics of z = the bf16 convolution output (``c2s_agg_skipconv_bstats_forward``).
+    Returns ``(out, z | None, batch_mean, batch_var)`` (biased variance, float32 [64]); the running statistics are the
+    caller's.  ``keep_z=False`` writes z into ``out``'s memory and returns None for it.  Same shapes as
+    :func:`temporal_aggregate_skip_conv_forward`."""
+    keep = []
+    x, attn, pad, desc, params = _skipconv_inputs(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                  None, None, bn_eps, keep)
+    b, t, c, h, w = x.shape
+    out = torch.empty((b, c, h, w), dtype=x.dtype, device=x.device)
+    z = torch.empty_like(out) if keep_z else out
+    mean = torch.empty(c, dtype=torch.float32, device=x.device)
+    var = torch.empty_like(mean)
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        ws_bytes = lib.c2s_agg_skipconv_bstats_workspace_bytes(ctypes.byref(desc))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        status = lib.c2s_agg_skipconv_bstats_forward(ctypes.byref(desc), x.data_ptr(), attn.data_ptr(), _ptr(pad),
+                                                     ctypes.byref(params), z.data_ptr(), out.data_ptr(), mean.data_ptr(),
+                                                     var.data_ptr(), ws.data_ptr(), ws_bytes, _stream(x.device))
+    _lib.check(status, "c2s_agg_skipconv_bstats_forward")
+    return out, (z if keep_z else None), mean, var
+
+
+def temporal_aggregate_skip_conv_bstats_backward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: torch.Tensor,
+                                                 conv_weight: torch.Tensor, conv_bias: Optional[torch.Tensor],
+                                                 bn_weight: Optional[torch.Tensor], bn_bias: Optional[torch.Tensor],
+                                                 bn_eps: float, z: torch.Tensor, batch_mean: torch.Tensor,
+                                                 batch_var: torch.Tensor, out: torch.Tensor, grad_out: torch.Tensor,
+                                                 need=(True,) * 6) -> Tuple[Optional[torch.Tensor], ...]:
+    """Backward of :func:`temporal_aggregate_skip_conv_bstats_forward` (``c2s_agg_skipconv_bstats_backward``) from its
+    z, batch statistics and output: ``(grad_x, grad_attn, grad_conv_weight, grad_conv_bias, grad_bn_weight,
+    grad_bn_bias)`` as in :func:`temporal_aggregate_skip_conv_backward`; grad_conv_bias is exactly zero."""
+    keep = []
+    x, attn, pad, desc, params = _skipconv_inputs(x, pad_mask, attn_mask, conv_weight, conv_bias, bn_weight, bn_bias,
+                                                  None, None, bn_eps, keep)
+    b, t, c, h, w = x.shape
+    for name, v in (("z", z), ("out", out), ("grad_out", grad_out)):
+        if tuple(v.shape) != (b, c, h, w):
+            raise RuntimeError(f"crop2seg_b200: {name} {tuple(v.shape)} must be {(b, c, h, w)}")
+    zz, o, gout = (v.to(dtype=x.dtype).contiguous() for v in (z, out, grad_out))
+    mean, var = (v.to(device=x.device, dtype=torch.float32).contiguous() for v in (batch_mean, batch_var))
+    f32 = dict(dtype=torch.float32, device=x.device)
+    want = [bool(n) for n in need]
+    want[3] = want[3] and conv_bias is not None
+    want[4] = want[4] and bn_weight is not None
+    want[5] = want[5] and bn_bias is not None
+    res = [torch.empty_like(x) if want[0] else None, torch.zeros_like(attn) if want[1] else None,
+           torch.empty((c, c), **f32) if want[2] else None] + [torch.empty(c, **f32) if k else None for k in want[3:]]
+    io = _lib.SkipConvBwdIo(**{k: _ptr(r) for k, r in zip(_lib.SKIPCONV_BWD_IO_FIELDS, res)})
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        ws_bytes = lib.c2s_agg_skipconv_bstats_backward_workspace_bytes(ctypes.byref(desc))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        status = lib.c2s_agg_skipconv_bstats_backward(ctypes.byref(desc), x.data_ptr(), attn.data_ptr(), _ptr(pad),
+                                                      ctypes.byref(params), zz.data_ptr(), mean.data_ptr(),
+                                                      var.data_ptr(), o.data_ptr(), gout.data_ptr(), ctypes.byref(io),
+                                                      ws.data_ptr(), ws_bytes, _stream(x.device))
+    _lib.check(status, "c2s_agg_skipconv_bstats_backward")
+    if res[2] is not None:
+        res[2] = res[2].view(conv_weight.shape)
+    return tuple(res)
+
+
 def temporal_aggregate_backward(x: torch.Tensor, pad_mask: Optional[torch.Tensor], attn_mask: Optional[torch.Tensor],
                                 grad_out: torch.Tensor, mode: str, need_x: bool = True, need_attn: bool = True
                                 ) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:

@@ -121,6 +121,26 @@ int c2s_agg_skipconv_backward(const c2s_agg_desc* desc, const void* x, const flo
                               const c2s_skipconv_params* params, const void* out, const void* grad_out,
                               const c2s_skipconv_bwd_io* io, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The same block with its BatchNorm normalising by batch statistics (training mode, or track_running_stats=False):
+ *   z = Conv2d_1x1(aggregate(x, attn, pad))  (bf16, [B,C,H,W]),  out = relu( BatchNorm2d_train(z) )
+ * over N = B*H*W pixels per channel (an all-padded sample counts: its skip map is 0, its z the conv bias).  z crosses HBM
+ * once; the statistics are merged from per-tile (mean, M2) partials in a fixed order (bit-identical from run to run).
+ * bn_batch_mean/var: float32 [C] (biased variance); the caller updates the running statistics (as c2s_ltae_forward).
+ * params->bn_running_mean/var are ignored and may be NULL.  out may be z (when z is not needed afterwards).  Same shapes
+ * as c2s_agg_skipconv_forward; anything else returns C2S_ERR_UNSUPPORTED. */
+size_t c2s_agg_skipconv_bstats_workspace_bytes(const c2s_agg_desc* desc);
+int c2s_agg_skipconv_bstats_forward(const c2s_agg_desc* desc, const void* x, const float* attn, const uint8_t* pad_mask,
+                                    const c2s_skipconv_params* params, void* z, void* out, float* bn_batch_mean,
+                                    float* bn_batch_var, void* workspace, size_t workspace_bytes, void* stream);
+/* Backward of c2s_agg_skipconv_bstats_forward from its z, batch statistics and out (distinct from z).  io as in
+ * c2s_agg_skipconv_backward; grad_conv_bias is written as zeros (batch statistics cancel a per-channel constant of z).
+ * grad_bn_weight / grad_bn_bias / grad_conv_weight are deterministic.  Unsupported shapes return C2S_ERR_BAD_ARGUMENT. */
+size_t c2s_agg_skipconv_bstats_backward_workspace_bytes(const c2s_agg_desc* desc);
+int c2s_agg_skipconv_bstats_backward(const c2s_agg_desc* desc, const void* x, const float* attn, const uint8_t* pad_mask,
+                                     const c2s_skipconv_params* params, const void* z, const float* bn_batch_mean,
+                                     const float* bn_batch_var, const void* out, const void* grad_out,
+                                     const c2s_skipconv_bwd_io* io, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Backward of TemporalAggregator.forward (what autograd derives from temporal_aggregator.py:14-77):
  *   grad_x[b,t,c]        = resize(attn)[c // (C/n_heads), b, t] * (pad ? 0 : 1) * grad_out[b,c]      (x's dtype)
  *   grad_attn[h,b,t,:,:] = resize^T( sum_{c in head h} x[b,t,c] * grad_out[b,c] )                  (float32)
